@@ -24,14 +24,23 @@ t-ramp with every Newton iteration, Hessian assembly, V-cycle PCG solve and line
 path is deterministic, so it is run once, not warmup + steps times).  The reference itself is Julia; there is no Julia here
 (baseline/run_reference.jl is the script for a box that has it).
 N > 1 (torchrun): ONE solve, elements partitioned over the ranks (partition.py), max-over-ranks time ("strong").
+
+`--dump-outputs DIR` writes what the last timed solve returned (z, z_unfinalized and the t-ramp history of SOL_main) as
+float64 DIR/<name>.npy, so that two builds can be compared output for output: the problem is synthetic and deterministic,
+so the same arguments give the same inputs on every run.
+The bench writes nothing into the tree it runs from (which may be read-only): no bytecode, and numba's cache of the host-side
+AMG setup goes to a temporary directory.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -44,6 +53,7 @@ METRIC = "mgb_solve DOF*Newton-steps/s (fem2d_P1 ~1.6M DOF, p=1.5)"
 UNIT = "DOF*Newton-steps/s"
 REF_L = 8          # --impl reference: largest level whose single full-ramp oracle solve takes ~2 minutes
 CPU_L = 7          # cpu_baseline leg of the default run (~30 s)
+DUMP_BYTES = 64 << 20
 
 
 def build_problem(L, p):
@@ -136,6 +146,27 @@ def parity_record(sol, L, p, reduce_sum=None):
     rec["pass"] = bool(rec["rel_vs_fixture"] < 1e-6 and rec["objective_rel_vs_fixture"] < 1e-8 and
                        rec["max_step_count_diff_excl_finalize"] is not None and rec["max_step_count_diff_excl_finalize"] <= 1)
     return rec
+
+
+def dump_outputs(out_dir, sol, budget=DUMP_BYTES):
+    """Write what mgb_solve returned to its caller -- z and SOL_main without its wall-clock fields -- as float64 out_dir/<name>.npy.
+    If the per-node arrays (z, z_unfinalized) do not fit in `budget` bytes, the same fixed sample of their rows (seed 0) is written
+    instead, and the row numbers as node_rows.npy.  Returns the names written."""
+    S = sol["SOL_main"]
+    out = {k: np.asarray(S[k], dtype=np.float64) for k in ("its", "its_finalize", "ts", "kappas", "c_dot_Dz")}
+    nodes = {"z": sol["z"], "z_unfinalized": S["z_unfinalized"]}
+    n = sol["z"].shape[0]
+    row_bytes = sum(8 * a[0].size for a in nodes.values())
+    room = budget - sum(a.nbytes for a in out.values()) - 128 * (len(out) + len(nodes) + 1)     # 128: .npy header
+    if n * row_bytes > room:
+        rows = np.sort(np.random.default_rng(0).choice(n, room // (row_bytes + 8), replace=False))
+        nodes = {k: a[rows] for k, a in nodes.items()}
+        nodes["node_rows"] = rows
+    out.update((k, np.asarray(a, dtype=np.float64)) for k, a in nodes.items())
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    return sorted(out)
 
 
 def oracle_solve(L, p):
@@ -253,11 +284,21 @@ def main():
     ap.add_argument("--fem3d-c", type=int, default=64, help="fem3d sub-record: k=1 hexahedra per edge (64: n = 2 097 152); 0 = skip")
     ap.add_argument("--fem3d-t", type=float, default=0.01, help="initial t of the fem3d sub-record (DESIGN.md: t = 0.1 stalls in the reference algorithm itself on >= 32^3)")
     ap.add_argument("--config", action="append", default=[], help="mgbx_config override key=value (repeatable)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed solve as DIR/<name>.npy (float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and world > 1 and not args.replicas:
+        ap.error("--dump-outputs needs the whole z on one rank: run on one GPU or with --replicas")
+
+    sys.dont_write_bytecode = True
+    if "NUMBA_CACHE_DIR" not in os.environ:
+        os.environ["NUMBA_CACHE_DIR"] = tempfile.mkdtemp(prefix="mgbx-bench-numba-")
+        atexit.register(shutil.rmtree, os.environ["NUMBA_CACHE_DIR"], True)
 
     if args.impl == "reference":
         reference_arm(args, rank, world)
@@ -324,8 +365,7 @@ def main():
         return sol
 
     for _ in range(args.warmup):
-        sol = resident_step()
-    its_total = int(sol["SOL_main"]["its"].sum())
+        resident_step()
 
     sampler = ClockSampler(local_rank)
     sampler.start()
@@ -342,6 +382,9 @@ def main():
     dev_s = e0.elapsed_time(e1) * 1e-3
     launches = h.launch_count() - l0
     sampler.stop_flag = True
+    its_total = int(sol["SOL_main"]["its"].sum())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sol)
     stats = sol["stats"]
     if sharded:
         sol["node_range"] = lprob.node_range
@@ -356,7 +399,7 @@ def main():
         h2d += sum(T.data.nbytes + T.indices.nbytes * 2 + T.indptr.nbytes * 2 for T in M.T)
     h2d += lprob.f.nbytes + lprob.g.nbytes + sum(pc.A.nbytes + pc.b.nbytes for pc in lprob.Q.pieces)
     d2h = 2 * lprob.g.nbytes                              # z and z_unfinalized
-    for k in range(1 + max(1, min(args.steps, 3))):      # one untimed warm-up call (first-use costs of a fresh handle), then the timed ones
+    for k in range(1 + args.steps):      # one untimed warm-up call (first-use costs of a fresh handle), then the timed ones
         barrier()
         t1 = time.time()
         sol_e = solver.mgb_solve(prob, comm=new_comm(), config=dict(device=local_rank, **cfg))
