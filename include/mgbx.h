@@ -43,7 +43,7 @@
 extern "C" {
 #endif
 
-#define MGBX_ABI_VERSION 1
+#define MGBX_ABI_VERSION 2
 #define MGBX_MAX_LEVELS 32
 #define MGBX_MAX_ND 12      /* rows of D seen by one node functor (incl. phase-I extras) */
 #define MGBX_MAX_PIECES 6
@@ -135,29 +135,20 @@ typedef struct {
   int32_t condense;          /* 1 (default): eliminate node-local :full variables exactly before PCG */
   int32_t device;            /* CUDA device ordinal, -1 = current */
   int32_t verbose;
-  int32_t use_graphs;        /* 1 (default): replay each PCG iteration (V-cycle + vector updates) as one CUDA graph */
   int32_t profile;           /* 1: time every kernel launch with CUDA events on the handle's stream (mgbx_kernel_stats) */
-  int32_t persistent;        /* each PCG solve is ONE cooperative persistent kernel (one CTA per SM, grid barriers): 2 (default) the
-                                second-generation kernel (csrc/pcg2.cu: sliced-ELL level matrices, row ownership, tail levels in
-                                CTA 0's shared memory); 1 the first-generation CSR kernel; 0 one kernel per phase (CUDA graph) */
-  int32_t tail_max;          /* V-cycle levels with <= this many unknowns run inside CTA 0 of that kernel (default 1200) */
+  int32_t persistent;        /* must be 2: the only solve kernel, k_pcg2 (csrc/pcg2.cu); kept for callers that read it */
+  int32_t tail_max;          /* V-cycle levels with <= this many unknowns run inside CTA 0 of the solve kernel (default 1200) */
   double pcg_rtol_final;     /* relative residual during the finalize pass (stopping_exact), default 1e-15 (i.e. to stagnation) */
   int32_t fused;             /* 1 (default): fused element kernels (operator blocks staged once in shared memory), with the
                                 specialised kernel for the default (u, s) Euclidean-power family where it applies;
                                 2: generic fused kernel only; 0: separate per-node and per-block kernels (always used
                                 when a block does not fit in shared memory) */
-  int32_t smoother;          /* V-cycle smoother of the persistent kernel: 1 (default) Chebyshev of degree smoother_sweeps
+  int32_t smoother;          /* V-cycle smoother of the solve kernel: 1 (default) Chebyshev of degree smoother_sweeps
                                 with diagonal scaling on [lam/cheb_ratio, lam], lam = Gershgorin bound; 0 l1-Jacobi */
   double cheb_ratio;         /* default 8 (sweep in profiles/r01z_smoother_sweep.jsonl) */
   int32_t precond_fp32;      /* 1: the V-cycle (preconditioner) reads FP32 copies of the level matrices (8 instead of 12 bytes per
                                 non-zero); the PCG operator, vectors and all reductions stay FP64.  0 off, 2 (default) automatic: only when
                                 the level matrices together have >= 10 M non-zeros (they no longer fit the L2: V-cycle HBM-bound) */
-  int32_t pcg_lanes;         /* lanes per matrix row in the persistent kernel's level mat-vecs.  0 (default): per level, the width
-                                in {1, 4, 32} with the shortest dependent-load chain (passes over the rows x loads per pass) when rows average
-                                <= 16 entries, else by average row length;
-                                -2: the same over {1, 2, 4, 8, 16, 32}; -1: by average row length only; 1 / 2 / 4 / 8 / 16 / 32
-                                forces that width on every level.  (Tuning hook: environment variable MGBX_TUNE_LANES =
-                                comma-separated widths per plan level, the last entry being the coarsest level, overrides modes 0 and -2.) */
   int32_t lambda_power;      /* -1 (default): automatic -- 6 when the top matrix averages more than 16 entries per row (3-D meshes), else 0;
                                 > 0: that many power iterations on D^-1 A per level and Newton system (warm-started) replace the
                                 Gershgorin bound of lambda_max in the Chebyshev interval (the bound stays as an upper clamp).  Measured on

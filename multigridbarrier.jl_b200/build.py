@@ -1,7 +1,7 @@
 """In-tree build of libmgbx.so (nvcc, sm_100a only).  The .so is git-ignored but travels to the GPU box.
 
 Two translation units, compiled in parallel and cached as objects under build/: mgbx.cu (handle, host logic, element / setup /
-dense kernels, first-generation solve kernel) and pcg2.cu (the second-generation persistent solve kernel)."""
+dense kernels) and pcg2.cu (the persistent solve kernel)."""
 from __future__ import annotations
 
 import os

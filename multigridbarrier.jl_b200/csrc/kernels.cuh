@@ -6,9 +6,10 @@
 //                     block_ops.jl:118-133 (_block_matvec_kernel!)
 //   k_blockgrad       sum_k D_k' y_k                    src/convex.jl:173-178; block_ops.jl:135-148
 //   k_blockhess       sum_{j,k} D_j' diag(y_jk) D_k     src/convex.jl:185-200; block_ops.jl:58-75 (called nD^2 times there)
-//   (solver_kernels.cuh: k_sell_gather = R'HR into the fixed pattern and the Galerkin products; k_pcg_persistent = the solve)
+//   (solver_kernels.cuh: k_sell_gather = R'HR into the fixed pattern and the Galerkin products)
 //   k_spmv*           R*s, R'*g                          CUSPARSE in the reference (src/convex.jl:156,178)
-//   k_jacobi*, k_pcg* multigrid-preconditioned CG        replaces cuDSS LDL' (ext/.../cudss_solver.jl:264-381)
+//   k_l1diag          smoother diagonals and the Gershgorin bound of every level of the solve kernel
+//   (pcg2.cu: k_pcg2 = the multigrid-preconditioned CG solve, replacing cuDSS LDL' (ext/.../cudss_solver.jl:264-381))
 //   (dense_kernels.cuh: DMMA GEMM and blocked Cholesky of the spectral path)
 // All reductions are fixed-order (block tree + last-block pass): results are run-to-run deterministic.
 #pragma once
@@ -120,53 +121,6 @@ __global__ void __launch_bounds__(256) k_spmv(DevCsr A, const double *__restrict
     for (int o = G / 2; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o, G);
   }
   if (sub == 0) y[row] = alpha * acc + (y0 ? y0[row] : 0.0);
-}
-
-// x_new = x + dinv .* (b - A x)      (one l1-Jacobi sweep; x == nullptr means x = 0)
-template <int G>
-__global__ void __launch_bounds__(256) k_jacobi(DevCsr A, const double *__restrict__ dinv, const double *__restrict__ b,
-                                                 const double *__restrict__ x, double *xnew) {
-  const int64_t gtid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t row = gtid / G;
-  const int sub = (int)(gtid % G);
-  if (row >= A.rows) return;
-  if (x == nullptr) {
-    if (sub == 0) xnew[row] = dinv[row] * b[row];
-    return;
-  }
-  const int64_t bb = A.ptr[row], e = A.ptr[row + 1];
-  double acc = 0.0;
-  for (int64_t k = bb + sub; k < e; k += G) acc += A.val[k] * x[A.idx[k]];
-  if (G > 1) {
-#pragma unroll
-    for (int o = G / 2; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o, G);
-  }
-  if (sub == 0) xnew[row] = x[row] + dinv[row] * (b[row] - acc);
-}
-
-// two l1-Jacobi sweeps from x = 0 in one pass:  x1 = dinv b;  x2 = x1 + dinv (b - A x1)
-template <int G>
-__global__ void __launch_bounds__(256) k_jacobi_first2(DevCsr A, const double *__restrict__ dinv, const double *__restrict__ b,
-                                                        double *xnew) {
-  const int64_t gtid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t row = gtid / G;
-  const int sub = (int)(gtid % G);
-  if (row >= A.rows) return;
-  const int64_t bb = A.ptr[row], e = A.ptr[row + 1];
-  double acc = 0.0;
-  for (int64_t k = bb + sub; k < e; k += G) {
-    const int32_t j = A.idx[k];
-    acc += A.val[k] * (dinv[j] * b[j]);
-  }
-  if (G > 1) {
-#pragma unroll
-    for (int o = G / 2; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o, G);
-  }
-  if (sub == 0) {
-    const double d = dinv[row], bi = b[row];
-    const double x1 = d * bi;
-    xnew[row] = x1 + d * (bi - acc);
-  }
 }
 
 // dinv = 1 / sum_k |a_ik|  (l1-Jacobi), diag = 1 / a_ii, and the Gershgorin bound of lambda_max(D^-1 A),
@@ -546,80 +500,11 @@ __global__ void k_axpby(int64_t m, double a, const double *__restrict__ x, doubl
   if (i < m) out[i] = a * x[i] + (y ? b * y[i] : 0.0);
 }
 
-// PCG: scal = {rz, pAp, rr, rz_new}.
-//  step A: alpha = rz/pAp;  x += alpha p;  r -= alpha Ap;  rr = r.r
-__global__ void __launch_bounds__(kRedThreads) k_pcg_update(int64_t m, double *scal, const double *__restrict__ p, const double *__restrict__ Ap,
-                                                             double *x, double *r, double *partials, unsigned int *ticket) {
-  const double alpha = scal[0] / scal[1];
-  double red[1] = {0.0};
-  const int op[1] = {0};
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += (int64_t)gridDim.x * blockDim.x) {
-    x[i] += alpha * p[i];
-    const double ri = r[i] - alpha * Ap[i];
-    r[i] = ri;
-    red[0] += ri * ri;
-  }
-  grid_reduce<1>(red, op, partials, ticket, scal + 2);
-}
-//  step B: beta = rz_new/rz;  p = z + beta p;  then rz <- rz_new   (done by thread 0 of the LAST block only after all reads:
-//  we avoid the hazard by passing beta through a separate slot written by k_pcg_beta)
-__global__ void k_pcg_init(double *scal) {   // rz = 1 so that the first beta is finite (p starts at 0)
-  scal[0] = 1.0;
-  scal[1] = 1.0;
-  scal[3] = 0.0;
-  scal[4] = 0.0;
-}
-__global__ void k_pcg_beta(double *scal) {   // scal[4] = beta = scal[3]/scal[0]; scal[0] = scal[3]
-  scal[4] = scal[3] / scal[0];
-  scal[0] = scal[3];
-}
-__global__ void k_pcg_dir(int64_t m, const double *scal, const double *__restrict__ z, double *p) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < m) p[i] = z[i] + scal[4] * p[i];
-}
-// out[slot] = a.b
-__global__ void __launch_bounds__(kRedThreads) k_dot(int64_t m, const double *__restrict__ a, const double *__restrict__ b, double *partials,
-                                                      unsigned int *ticket, double *out) {
-  double red[1] = {0.0};
-  const int op[1] = {0};
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += (int64_t)gridDim.x * blockDim.x) red[0] += a[i] * b[i];
-  grid_reduce<1>(red, op, partials, ticket, out);
-}
-
-// ---- power iteration on D^-1 A: a sharper lambda_max for the Chebyshev interval than the Gershgorin bound (cfg.lambda_power) ----
-// start vector: smooth + oscillatory parts, never orthogonal to the top eigenvector in practice
+// start vector of the power iteration on D^-1 A (pcg2_lambda_power: a sharper lambda_max for the Chebyshev interval than the
+// Gershgorin bound): smooth + oscillatory parts, never orthogonal to the top eigenvector in practice
 __global__ void k_pw_init(int64_t m, double *v) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < m) v[i] = 1.0 + 0.5 * cos(0.7 * (double)i) + ((i & 1) ? 0.25 : -0.25);
-}
-
-// w <- idiag .* w (idiag = 1 / a_ii);  out[0] = |w|^2
-__global__ void __launch_bounds__(kRedThreads) k_pw_scale_norm(int64_t m, const double *__restrict__ idiag, double *w, double *partials,
-                                                                unsigned int *ticket, double *out) {
-  double red[1] = {0.0};
-  const int op[1] = {0};
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += (int64_t)gridDim.x * blockDim.x) {
-    const double v = w[i] * idiag[i];
-    w[i] = v;
-    red[0] += v * v;
-  }
-  grid_reduce<1>(red, op, partials, ticket, out);
-}
-
-// v <- w / |w|  (v is left alone when the norm vanished or is not finite)
-__global__ void k_pw_normalize(int64_t m, const double *__restrict__ w, const double *nrm2, double *v) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const double n2 = nrm2[0];
-  if (i < m && n2 > 0.0 && isfinite(n2)) v[i] = w[i] * rsqrt(n2);
-}
-
-// lam <- min(lam, safety * |D^-1 A v|): the Gershgorin bound already in lam stays an upper clamp
-__global__ void k_pw_store(const double *nrm2, double safety, double *lam) {
-  const double n2 = nrm2[0];
-  if (n2 > 0.0 && isfinite(n2)) {
-    const double est = safety * sqrt(n2);
-    if (est < lam[0]) lam[0] = est;
-  }
 }
 
 // per-variable max and max|.| of the state: out[2k] = max, out[2k+1] = absmax  (one launch per variable)

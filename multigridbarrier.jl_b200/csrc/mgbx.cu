@@ -45,10 +45,10 @@ using namespace mgbx;
 static thread_local std::string g_last_error;
 
 // kernel classes for the optional per-class device timing (cfg.profile) and launch statistics
-enum KClass { KC_NODE_F01 = 0, KC_NODE_F2, KC_BLOCKGRAD, KC_BLOCKHESS, KC_GATHER, KC_SPMV, KC_JACOBI, KC_SPGEMM, KC_VEC, KC_COND,
+enum KClass { KC_NODE_F01 = 0, KC_NODE_F2, KC_BLOCKGRAD, KC_BLOCKHESS, KC_GATHER, KC_SPMV, KC_SPGEMM, KC_VEC, KC_COND,
               KC_DENSE, KC_PCG, KC_ELEM_F01, KC_ELEM_F2, KC_DGEMM, KC_ELEMG_F01, KC_ELEMG_F2, KC_COUNT };
-static const char *kKClassNames[KC_COUNT] = {"node_f01", "node_f2", "blockgrad", "blockhess", "csr_gather", "spmv", "jacobi",
-                                             "spgemm", "vector", "condense", "dense", "pcg_persistent", "elem_f01", "elem_f2", "dgemm_dmma", "elem_generic_f01", "elem_generic_f2"};
+static const char *kKClassNames[KC_COUNT] = {"node_f01", "node_f2", "blockgrad", "blockhess", "csr_gather", "spmv", "spgemm",
+                                             "vector", "condense", "dense", "pcg_persistent", "elem_f01", "elem_f2", "dgemm_dmma", "elem_generic_f01", "elem_generic_f2"};
 enum { STAGE_F01 = -1, STAGE_F2 = -2, STAGE_SOLVE = -3 };
 #define LAUNCH(kc, ...)   \
   do {                    \
@@ -384,12 +384,12 @@ struct SysLevel {
   bool has_coarser = false, T_identity = false;
   float *val32 = nullptr;      // FP32 copy of A.val for the preconditioner passes (cfg.precond_fp32)
   double *dinv = nullptr, *diag = nullptr, *lam = nullptr;   // lam: Gershgorin bound of lambda_max(D^-1 A) (device scalar)
-  double *pw = nullptr, *pw_nrm = nullptr;   // power-iteration vector (kept across Newton iterations: warm start) and |D^-1 A v|^2 (cfg.lambda_power)
+  double *pw = nullptr;       // power-iteration vector (kept across Newton iterations: warm start, cfg.lambda_power)
   double *b = nullptr, *x = nullptr, *x2 = nullptr, *r = nullptr;   // V-cycle work
   double *dense = nullptr, *dense_inv = nullptr, *dscale = nullptr;
   int spmv_group = 1;
   std::vector<int64_t> off;  // system offsets of the kept variables (+ end)
-  // sliced-ELL copies for the second-generation persistent solve kernel (pcg2.hpp): pattern built once, A's values refreshed
+  // sliced-ELL copies for the solve kernel (pcg2.hpp): pattern built once, A's values refreshed
   // with every assembly, T / T' filled once
   SellBuild sA, sT, sTt;
   bool sell_A = false, sell_T = false;
@@ -427,15 +427,8 @@ struct System {
   std::vector<KronPair> kp;
   double *Wcat = nullptr;
   // PCG work at the largest size
-  double *pc_r = nullptr, *pc_z = nullptr, *pc_p = nullptr, *pc_Ap = nullptr, *pc_x = nullptr, *pc_b = nullptr;
-  std::map<int, cudaGraphExec_t> graphs;        // captured PCG iteration per top level (non-persistent path)
-  std::map<int, int64_t> graph_launches;
-  // persistent solve kernel: one plan per top level
-  struct PcgDev {
-    PcgPlan host;
-    PcgPlan *dev = nullptr;
-  };
-  std::map<int, PcgDev> pplans;
+  double *pc_r = nullptr, *pc_p = nullptr, *pc_Ap = nullptr, *pc_x = nullptr, *pc_b = nullptr;
+  // solve kernel: one plan per top level
   struct Pcg2Dev {
     Pcg2Plan host;
     Pcg2Plan *dev = nullptr;
@@ -516,8 +509,7 @@ struct mgbx_handle {
   };
   std::vector<Pending> ev_pending;
   cudaEvent_t ev_cur = nullptr;
-  int pcg_grid = 0;
-  int pcg2_grid = 0;         // CTAs of the second-generation persistent kernel (0: not available)
+  int pcg2_grid = 0;         // CTAs of the solve kernel k_pcg2
   double dgemm_flops = 0.0;   // FP64 tensor-core flops issued so far (spectral path)
   double cur_rtol2 = 1e-22;
   int cur_window = 25;       // PCG stagnation window (iterations without a new best residual)
@@ -528,7 +520,7 @@ struct mgbx_handle {
   int rank = 0, nranks = 1;
   void *comm = nullptr;
   int device = -1;           // CUDA device ordinal the handle lives on (made current at every ABI entry point)
-  // phase profile of the second-generation solve kernel (env MGBX_PCG_PROF=1): summed ns and counts per tag (level * 16 + kind)
+  // phase profile of the solve kernel k_pcg2 (env MGBX_PCG_PROF=1): summed ns and counts per tag (level * 16 + kind)
   std::vector<double> prof_ns;
   std::vector<int64_t> prof_cnt;
   std::vector<unsigned long long> prof_host;
@@ -668,64 +660,6 @@ struct Engine {
   }
 
   // ---------------------------------------------------------------- sparse helpers
-  // lam <- min(Gershgorin, 1.2 |D^-1 A v|) after `iters` power iterations on D^-1 A, warm-started from the previous Newton
-  // iteration's vector.  The Gershgorin bound overestimates lambda_max by 1.3-2.5x on 3-D (27-point) Hessians, which
-  // misplaces the Chebyshev interval (DESIGN.md section 9, tools/smoother_lab.py).  Lv.r is free scratch before a solve.
-  void lambda_power(SysLevel &Lv, int iters) {
-    if (!Lv.pw) {
-      Lv.pw = h->pool.alloc<double>(Lv.m);
-      Lv.pw_nrm = h->pool.zeros<double>(1, s);
-      LAUNCH(KC_VEC, k_pw_init<<<nblk(Lv.m), 256, 0, s>>>(Lv.m, Lv.pw));
-    }
-    for (int it = 0; it < iters; ++it) {
-      spmv(Lv.A, Lv.pw, nullptr, 1.0, Lv.r, Lv.spmv_group);
-      LAUNCH(KC_VEC, k_pw_scale_norm<<<red_grid(Lv.m), kRedThreads, 0, s>>>(Lv.m, Lv.diag, Lv.r, h->partials, h->ticket, Lv.pw_nrm));
-      LAUNCH(KC_VEC, k_pw_normalize<<<nblk(Lv.m), 256, 0, s>>>(Lv.m, Lv.r, Lv.pw_nrm, Lv.pw));
-    }
-    LAUNCH(KC_VEC, k_pw_store<<<1, 1, 0, s>>>(Lv.pw_nrm, 1.2, Lv.lam));
-  }
-  // lanes per row of a level matrix inside the persistent kernel (cfg.pcg_lanes); nthr = threads that share the phase,
-  // from_end = distance of the level from the coarsest level of the plan
-  int pcg_lanes(const DevCsr &A, int64_t nthr, int from_end) const {
-    const int mode = h->cfg.pcg_lanes;
-    if (mode == 1 || mode == 2 || mode == 4 || mode == 8 || mode == 16 || mode == 32) return mode;
-    if (mode == -1 || A.rows == 0) return group_for(A);
-    if (const char *env = getenv("MGBX_TUNE_LANES")) {   // tuning hook: comma-separated widths, aligned to the COARSEST plan level
-      std::vector<int> vals;
-      for (const char *c = env; *c;) {
-        vals.push_back(atoi(c));
-        while (*c && *c != ',') ++c;
-        if (*c == ',') ++c;
-      }
-      const int k = (int)vals.size() - 1 - from_end;
-      if (k >= 0) {
-        const int v = vals[k];
-        if (v == 1 || v == 2 || v == 4 || v == 8 || v == 16 || v == 32) return v;
-      }
-    }
-    // dependent loads per thread: every pass over the rows costs the row pointer plus one index -> value chain per
-    // batch of 4 unrolled entries; ties go to the wider (better coalesced) mapping
-    const double avg = (double)A.nnz / (double)A.rows;
-    // long rows (3-D hexahedra, Galerkin levels of 3-D meshes): one lane per row would stride through more matrix
-    // bytes per warp than L1 holds, so the chain model is only trusted up to 16 entries per row (the measured regime)
-    if (mode == 0 && avg > 16.0) return group_for(A);
-    int best = 1;
-    double best_cost = 1e300;
-    const int wide[6] = {1, 2, 4, 8, 16, 32}, narrow[3] = {1, 4, 32};
-    const int *cand = (mode == -2) ? wide : narrow;
-    const int ncand = (mode == -2) ? 6 : 3;
-    for (int c = 0; c < ncand; ++c) {
-      const int G = cand[c];
-      const double passes = std::ceil((double)A.rows * G / (double)nthr);
-      const double iters = std::ceil(avg / G);
-      const double cost = passes * (1.0 + 2.0 * std::ceil(iters / 4.0));
-      if (cost <= best_cost) {
-        best_cost = cost;
-        best = G;
-      }
-    }
-    return best;
-  }
   static int group_for(const DevCsr &A) {
     const double avg = A.rows ? (double)A.nnz / (double)A.rows : 0.0;
     return avg > 48.0 ? 32 : (avg > 6.0 ? 4 : 1);
@@ -738,22 +672,6 @@ struct Engine {
     else if (G == 4) k_spmv<4><<<nblk(A.rows * 4), 256, 0, s>>>(A, x, y0, alpha, y);
     else k_spmv<1><<<nblk(A.rows), 256, 0, s>>>(A, x, y0, alpha, y);
     post_launch(KC_SPMV);
-  }
-  void jacobi(const SysLevel &Lv, const double *b, const double *x, double *xnew) {
-    const int G = Lv.spmv_group;
-    pre_launch(KC_JACOBI);
-    if (G == 32) k_jacobi<32><<<nblk(Lv.m * 32), 256, 0, s>>>(Lv.A, Lv.dinv, b, x, xnew);
-    else if (G == 4) k_jacobi<4><<<nblk(Lv.m * 4), 256, 0, s>>>(Lv.A, Lv.dinv, b, x, xnew);
-    else k_jacobi<1><<<nblk(Lv.m), 256, 0, s>>>(Lv.A, Lv.dinv, b, x, xnew);
-    post_launch(KC_JACOBI);
-  }
-  void jacobi2(const SysLevel &Lv, const double *b, double *xnew) {
-    const int G = Lv.spmv_group;
-    pre_launch(KC_JACOBI);
-    if (G == 32) k_jacobi_first2<32><<<nblk(Lv.m * 32), 256, 0, s>>>(Lv.A, Lv.dinv, b, xnew);
-    else if (G == 4) k_jacobi_first2<4><<<nblk(Lv.m * 4), 256, 0, s>>>(Lv.A, Lv.dinv, b, xnew);
-    else k_jacobi_first2<1><<<nblk(Lv.m), 256, 0, s>>>(Lv.A, Lv.dinv, b, xnew);
-    post_launch(KC_JACOBI);
   }
   void copy(double *dst, const double *src, int64_t m) {
     if (m) CK(cudaMemcpyAsync(dst, src, sizeof(double) * m, cudaMemcpyDeviceToDevice, s));
@@ -1059,7 +977,6 @@ struct Engine {
     if (S.lev.empty() || S.lev[0].A.rows == 0) return 0;
     return ((double)S.lev[0].A.nnz / (double)S.lev[0].A.rows > 16.0) ? 6 : 0;
   }
-  bool gen2_power(const System &S) const { return h->cfg.persistent == 2 && h->pcg2_grid > 0 && (int64_t)S.lev.size() * h->pcg2_grid <= 3 * (int64_t)kPcg2MaxGrid; }
   bool use_direct(const System &S, const SysLevel &Lv) const {
     return S.dense || Lv.m <= h->cfg.dense_direct_max;   // dense (spectral) systems have no hierarchy: always direct
   }
@@ -1070,25 +987,7 @@ struct Engine {
   void setup_hierarchy(Amg &A, System &S, int ktop);
   void dense_factor(System &S, SysLevel &Lv, bool want_inverse);
   void dense_apply(SysLevel &Lv, const double *b, double *x);      // x = A^{-1} b via factor (direct)
-  void vcycle(System &S, int k);
-  void pcg_iteration(System &S, int ktop);
-  System::PcgDev &pcg_plan(System &S, int ktop);
-  Csr32 csr32(const DevCsr &A) {   // 32-bit row pointers for the persistent kernel (pattern is fixed: converted once)
-    if (A.nnz > INT32_MAX || A.rows >= INT32_MAX) throw std::runtime_error("persistent solve kernel: a level matrix exceeds 32-bit indexing");
-    int *p32 = h->pool.alloc<int>((size_t)A.rows + 1);
-    k_ptr32<<<nblk(A.rows + 1), 256, 0, s>>>(A.rows + 1, A.ptr, p32);
-    CK(cudaGetLastError());
-    Csr32 C;
-    C.rows = (int)A.rows;
-    C.nnz = (int)A.nnz;
-    C.ptr = p32;
-    C.idx = A.idx;
-    C.val = A.val;
-    C.valf = nullptr;
-    return C;
-  }
-  int pcg_persistent(System &S, int ktop, const double *b, double *x);
-  // ---- second-generation persistent kernel (pcg2.hpp)
+  // ---- solve kernel (pcg2.hpp)
   std::vector<int> active_levels(const System &S, int ktop) const {
     const int nlev = (int)S.lev.size();
     const int kend = (S.cut >= 0) ? std::max(S.cut, ktop) : nlev - 1;
@@ -1103,7 +1002,6 @@ struct Engine {
   void sell_prepare(System &S, int ktop);
   System::Pcg2Dev &pcg2_plan(System &S, int ktop);
   void pcg2_setup_dist(System::Pcg2Dev &D, int nshard);
-  int pcg_persistent2(System &S, int ktop, const double *b, double *x);
   int pcg(System &S, int ktop, const double *b, double *x);
   int solve_compact(System &S, int ktop, const double *b, double *x);
   int solve(Amg &A, System &S, int J, const double *g, double *dir);
@@ -1398,13 +1296,12 @@ std::unique_ptr<System> build_system(mgbx_handle *h, Amg &A, bool condensed, int
       if (h->cfg.verbose > 0) fprintf(stderr, "[mgbx] build_system(dense, level %d): sum-factorised (Kronecker) assembly %s\n", ltop, S->kron ? "on" : "not applicable");
     }
     S->pc_r = pool.alloc<double>(m);
-    S->pc_z = pool.alloc<double>(m);
     S->pc_p = pool.alloc<double>(m);
     S->pc_p2 = pool.alloc<double>(m);
     S->pc_Ap = pool.alloc<double>(m);
     S->pc_x = pool.alloc<double>(m);
     S->pc_b = pool.alloc<double>(m);
-    S->pcg_partials = pool.zeros<double>(3 * (size_t)std::max(kPcgMaxGrid, kPcg2MaxGrid), s);
+    S->pcg_partials = pool.zeros<double>(3 * (size_t)kPcg2MaxGrid, s);
     S->pcg_out = pool.zeros<double>(8, s);
     S->pcg_bar = pool.zeros<unsigned int>(4, s);
     CK(cudaStreamSynchronize(s));
@@ -1530,13 +1427,12 @@ std::unique_ptr<System> build_system(mgbx_handle *h, Amg &A, bool condensed, int
     }
   const int64_t mx = S->lev[0].m;
   S->pc_r = pool.alloc<double>(mx);
-  S->pc_z = pool.alloc<double>(mx);
   S->pc_p = pool.alloc<double>(mx);
   S->pc_p2 = pool.alloc<double>(mx);
   S->pc_Ap = pool.alloc<double>(mx);
   S->pc_x = pool.alloc<double>(mx);
   S->pc_b = pool.alloc<double>(mx);
-  S->pcg_partials = pool.zeros<double>(3 * (size_t)std::max(kPcgMaxGrid, kPcg2MaxGrid), s);
+  S->pcg_partials = pool.zeros<double>(3 * (size_t)kPcg2MaxGrid, s);
   S->pcg_out = pool.zeros<double>(8, s);
   S->pcg_bar = pool.zeros<unsigned int>(4, s);
   CK(cudaStreamSynchronize(s));
@@ -1745,7 +1641,6 @@ void Engine::setup_hierarchy(Amg &A, System &S, int ktop) {
     SysLevel &Lv = S.lev[k];
     CK(cudaMemsetAsync(Lv.lam, 0, sizeof(double), s));
     LAUNCH(KC_VEC, k_l1diag<<<nblk(Lv.m), 256, 0, s>>>(Lv.A, Lv.dinv, Lv.diag, (unsigned long long *)Lv.lam));
-    if (lambda_power_its(S) > 0 && Lv.m > 1 && !gen2_power(S)) lambda_power(Lv, lambda_power_its(S));
     if (precond_fp32(S)) {
       if (!Lv.val32) Lv.val32 = h->pool.alloc<float>(Lv.A.nnz);
       LAUNCH(KC_VEC, k_f64_to_f32<<<nblk(Lv.A.nnz), 256, 0, s>>>(Lv.A.nnz, Lv.A.val, Lv.val32));
@@ -1757,13 +1652,11 @@ void Engine::setup_hierarchy(Amg &A, System &S, int ktop) {
     if (!Lc.dense_inv) Lc.dense_inv = h->pool.alloc<double>((size_t)m * m);
     LAUNCH(KC_DENSE, k_coarse_inverse<<<1, 1024, coarse_inverse_smem(m), s>>>(Lc.A, Lc.dense_inv));
   }
-  if (h->cfg.persistent == 2 && h->pcg2_grid > 0) {
-    sell_prepare(S, ktop);
-    if (lambda_power_its(S) > 0 && gen2_power(S)) {   // all levels' power iterations in one cooperative launch
-      System::Pcg2Dev &D = pcg2_plan(S, ktop);
-      if ((int64_t)D.host.nlev * h->pcg2_grid > 3 * (int64_t)kPcg2MaxGrid) throw std::runtime_error("internal: too many levels for the power-iteration kernel");
-      LAUNCH(KC_VEC, CK(pcg2_lambda_power(D.dev, h->pcg2_grid, lambda_power_its(S), 1.2, s)));
-    }
+  sell_prepare(S, ktop);
+  if (lambda_power_its(S) > 0) {   // all levels' power iterations in one cooperative launch
+    System::Pcg2Dev &D = pcg2_plan(S, ktop);
+    if ((int64_t)D.host.nlev * h->pcg2_grid > 3 * (int64_t)kPcg2MaxGrid) throw std::runtime_error("internal: too many levels for the power-iteration kernel");
+    LAUNCH(KC_VEC, CK(pcg2_lambda_power(D.dev, h->pcg2_grid, lambda_power_its(S), 1.2, s)));
   }
 }
 
@@ -1798,161 +1691,6 @@ void Engine::dense_factor(System &S, SysLevel &Lv, bool want_inverse) {
 void Engine::dense_apply(SysLevel &Lv, const double *b, double *x) {
   const int m = (int)Lv.m;
   LAUNCH(KC_DENSE, k_chol_solve_blocked<<<1, 1024, sizeof(double) * m, s>>>(Lv.dense, m, Lv.dense_inv, Lv.dscale, b, x));
-}
-
-void Engine::vcycle(System &S, int k) {
-  SysLevel &Lv = S.lev[k];
-  const int nlev = (int)S.lev.size();
-  if (k == S.cut) {
-    // x = A^{-1} b through the explicit inverse (diagonal scaling already folded in by k_coarse_inverse)
-    LAUNCH(KC_DENSE, k_dense_symv<<<nblk(Lv.m * 32), 256, 0, s>>>(Lv.dense_inv, (int)Lv.m, Lv.b, Lv.x));
-    return;
-  }
-  const bool bottom = (k == nlev - 1);
-  if (!bottom && Lv.T_identity) {
-    SysLevel &Lc = S.lev[k + 1];
-    copy(Lc.b, Lv.b, Lv.m);
-    vcycle(S, k + 1);
-    copy(Lv.x, Lc.x, Lv.m);
-    return;
-  }
-  const int nu = bottom ? 30 : std::max(1, h->cfg.smoother_sweeps);
-  // pre-smoothing from x = 0
-  double *xa = Lv.x, *xb = Lv.x2;
-  int done = 1;
-  if (nu >= 2) {
-    jacobi2(Lv, Lv.b, xa);      // two sweeps from x = 0 in one kernel
-    done = 2;
-  } else {
-    jacobi(Lv, Lv.b, nullptr, xa);
-  }
-  for (int it = done; it < nu; ++it) {
-    jacobi(Lv, Lv.b, xa, xb);
-    std::swap(xa, xb);
-  }
-  if (!bottom) {
-    SysLevel &Lc = S.lev[k + 1];
-    spmv(Lv.A, xa, Lv.b, -1.0, Lv.r, Lv.spmv_group);           // r = b - A x
-    spmv(Lv.Tt, Lv.r, nullptr, 1.0, Lc.b);
-    vcycle(S, k + 1);
-    spmv(Lv.T, Lc.x, xa, 1.0, xa);                              // x += T xc (row-local, in place)
-    for (int it = 0; it < nu; ++it) {
-      jacobi(Lv, Lv.b, xa, xb);
-      std::swap(xa, xb);
-    }
-  }
-  if (xa != Lv.x) copy(Lv.x, xa, Lv.m);
-}
-
-// Preconditioned CG on lev[ktop]; returns the iteration count (negative: breakdown)
-// One PCG iteration on fixed buffers (capturable into a CUDA graph):
-//   z = M^{-1} r (V-cycle);  rz_new = r.z;  beta = rz_new/rz;  p = z + beta p;  Ap = A p;  alpha = rz/pAp;
-//   x += alpha p;  r -= alpha Ap;  rr = r.r;  scalars -> pinned host
-void Engine::pcg_iteration(System &S, int ktop) {
-  SysLevel &Lv = S.lev[ktop];
-  const int64_t m = Lv.m;
-  double *r = S.pc_r, *p = S.pc_p, *Ap = S.pc_Ap, *x = S.pc_x;
-  double *scal = h->dscal + 8;   // {rz, pAp, rr, rz_new, beta}
-  const unsigned int rg = red_grid(m);
-  copy(Lv.b, r, m);
-  vcycle(S, ktop);
-  const double *zz = Lv.x;
-  LAUNCH(KC_VEC, k_dot<<<rg, kRedThreads, 0, s>>>(m, r, zz, h->partials, h->ticket, scal + 3));
-  LAUNCH(KC_VEC, k_pcg_beta<<<1, 1, 0, s>>>(scal));
-  LAUNCH(KC_VEC, k_pcg_dir<<<nblk(m), 256, 0, s>>>(m, scal, zz, p));
-  spmv(Lv.A, p, nullptr, 1.0, Ap, Lv.spmv_group);
-  LAUNCH(KC_VEC, k_dot<<<rg, kRedThreads, 0, s>>>(m, p, Ap, h->partials, h->ticket, scal + 1));
-  LAUNCH(KC_VEC, k_pcg_update<<<rg, kRedThreads, 0, s>>>(m, scal, p, Ap, x, r, h->partials, h->ticket));
-  CK(cudaMemcpyAsync(h->hscal + 8, scal, sizeof(double) * 5, cudaMemcpyDeviceToHost, s));
-}
-
-// Preconditioned CG on lev[ktop]; returns the iteration count (negative: breakdown)
-// plan of the persistent solve kernel for the hierarchy below lev[ktop] (built once, lives on the device)
-System::PcgDev &Engine::pcg_plan(System &S, int ktop) {
-  auto it = S.pplans.find(ktop);
-  if (it != S.pplans.end()) return it->second;
-  System::PcgDev &D = S.pplans[ktop];
-  PcgPlan &P = D.host;
-  memset(&P, 0, sizeof(P));
-  const int nlev = (int)S.lev.size();
-  const int kend = (S.cut >= 0) ? std::max(S.cut, ktop) : nlev - 1;
-  std::vector<int> act;
-  for (int k = ktop; k <= kend; ++k) {
-    if (k < kend && S.lev[k].T_identity) continue;   // same matrix as the next level
-    act.push_back(k);
-  }
-  P.nlev = (int)act.size();
-  P.nbig = 0;
-  for (int q = 0; q < P.nlev; ++q)
-    if (S.lev[act[q]].m > h->cfg.tail_max) P.nbig = q + 1;
-  P.nbig = std::max(P.nbig, 1);
-  P.bottom_dense = (S.cut >= 0 && act.back() == S.cut) ? 1 : 0;
-  P.nu = std::max(1, h->cfg.smoother_sweeps);
-  P.nu_bottom = 30;
-  P.smoother = h->cfg.smoother;
-  P.cheb_ratio = h->cfg.cheb_ratio > 1.0 ? h->cfg.cheb_ratio : 8.0;
-  P.maxit = h->cfg.pcg_maxit;
-  P.rtol2 = h->cfg.pcg_rtol * h->cfg.pcg_rtol;
-  for (int q = 0; q < P.nlev; ++q) {
-    SysLevel &Lv = S.lev[act[q]];
-    PLevel &pl = P.lev[q];
-    pl.m = Lv.m;
-    pl.A = csr32(Lv.A);
-    pl.A.valf = precond_fp32(S) ? Lv.val32 : nullptr;
-    pl.dinv = Lv.dinv;
-    pl.diag = Lv.diag;
-    pl.lam = Lv.lam;
-    pl.b = Lv.b;
-    pl.x = Lv.x;
-    pl.x2 = Lv.x2;
-    pl.r = Lv.r;
-    pl.G = pcg_lanes(Lv.A, q < P.nbig ? (int64_t)h->pcg_grid * kPcgThreads : (int64_t)kPcgThreads, P.nlev - 1 - q);
-    if (q + 1 < P.nlev) {
-      pl.T = csr32(Lv.T);
-      pl.Tt = csr32(Lv.Tt);
-      pl.GT = group_for(Lv.T);
-      pl.GTt = group_for(Lv.Tt);
-    }
-  }
-  P.dense_inv = P.bottom_dense ? S.lev[S.cut].dense_inv : nullptr;
-  P.r = S.pc_r;
-  P.p = S.pc_p;
-  P.p2 = S.pc_p2;
-  P.Ap = S.pc_Ap;
-  P.x = S.pc_x;
-  P.b = S.pc_b;
-  P.partials = S.pcg_partials;
-  P.bar = S.pcg_bar;
-  P.out = S.pcg_out;
-  D.dev = h->pool.upload<PcgPlan>(&P, 1, s);
-  CK(cudaStreamSynchronize(s));
-  if (h->cfg.verbose > 0)
-    fprintf(stderr, "[mgbx] persistent PCG plan: %d levels (%d grid-wide, %d in CTA 0), dense bottom %d, grid %d x %d\n", P.nlev, P.nbig,
-            P.nlev - P.nbig, P.bottom_dense, h->pcg_grid, kPcgThreads);
-  return D;
-}
-
-// The whole PCG solve in one cooperative launch; returns the iteration count (negative: breakdown)
-int Engine::pcg_persistent(System &S, int ktop, const double *b, double *x) {
-  SysLevel &Lv = S.lev[ktop];
-  const int64_t m = Lv.m;
-  // the dense bottom inverse must exist before the plan captures its pointer
-  System::PcgDev &D = pcg_plan(S, ktop);
-  if (b != S.pc_b) copy(S.pc_b, b, m);
-  const PcgPlan *dev = D.dev;
-  void *args[] = {(void *)&dev, (void *)&h->cur_rtol2, (void *)&h->cfg.pcg_maxit, (void *)&h->cur_window};
-  pre_launch(KC_PCG);
-  CK(cudaLaunchCooperativeKernel((const void *)k_pcg_persistent, dim3(h->pcg_grid), dim3(kPcgThreads), args, 0, s));
-  post_launch(KC_PCG);
-  CK(cudaMemcpyAsync(h->hscal + 8, S.pcg_out, sizeof(double) * 6, cudaMemcpyDeviceToHost, s));
-  sync();
-  const int it = (int)h->hscal[8];
-  const double status = h->hscal[10];
-  h->last_solve_status = (int)status;
-  h->last_solve_rel = (h->hscal[11] > 0.0) ? std::sqrt(h->hscal[9] / h->hscal[11]) : 0.0;
-  h->last_solve_erel = (h->hscal[12] > 0.0) ? h->hscal[13] / h->hscal[12] : 0.0;
-  if (x != S.pc_x) copy(x, S.pc_x, m);
-  return status < 0 ? -std::max(it, 1) : it;
 }
 
 // sliced-ELL copy of a device CSR pattern (32 rows per slice, slices-per-CTA for the grid the kernel is launched with)
@@ -2067,7 +1805,6 @@ System::Pcg2Dev &Engine::pcg2_plan(System &S, int ktop) {
     pl.r = Lv.r;
     if (!Lv.pw) {   // power-iteration vector (warm-started across Newton iterations)
       Lv.pw = h->pool.alloc<double>(Lv.m);
-      Lv.pw_nrm = h->pool.zeros<double>(1, s);
       LAUNCH(KC_VEC, k_pw_init<<<nblk(Lv.m), 256, 0, s>>>(Lv.m, Lv.pw));
     }
     pl.pw = Lv.pw;
@@ -2114,7 +1851,7 @@ System::Pcg2Dev &Engine::pcg2_plan(System &S, int ktop) {
   D.dev = h->pool.upload<Pcg2Plan>(&P, 1, s);
   CK(cudaStreamSynchronize(s));
   if (h->cfg.verbose > 0)
-    fprintf(stderr, "[mgbx] persistent PCG (gen 2) plan: %d levels (%d grid-wide, %d in CTA 0 from %zu bytes of shared memory), dense bottom %d, grid %d x %d\n",
+    fprintf(stderr, "[mgbx] persistent PCG plan: %d levels (%d grid-wide, %d in CTA 0 from %zu bytes of shared memory), dense bottom %d, grid %d x %d\n",
             P.nlev, P.nbig, P.nlev - P.nbig, D.smem, P.bottom_dense, h->pcg2_grid, kPcg2Threads);
   return D;
 }
@@ -2190,7 +1927,9 @@ void Engine::pcg2_setup_dist(System::Pcg2Dev &D, int nshard) {
     fprintf(stderr, "[mgbx] rank %d: row-sharded solve over %d ranks, %d of %d levels sharded, exchange arena %.1f MB\n", h->rank, nr, nshard, P.nlev, bytes / 1e6);
 }
 
-int Engine::pcg_persistent2(System &S, int ktop, const double *b, double *x) {
+// Preconditioned CG on lev[ktop], the whole solve in one cooperative launch of k_pcg2; returns the iteration count
+// (negative: breakdown)
+int Engine::pcg(System &S, int ktop, const double *b, double *x) {
   SysLevel &Lv = S.lev[ktop];
   const int64_t m = Lv.m;
   System::Pcg2Dev &D = pcg2_plan(S, ktop);
@@ -2224,95 +1963,6 @@ int Engine::pcg_persistent2(System &S, int ktop, const double *b, double *x) {
   if (status == -3.0) throw std::runtime_error("row-sharded solve: a peer rank never arrived at a cross-GPU barrier (ranks out of step?)");
   if (x != D.host.x) copy(x, D.host.x, m);
   return status < 0 ? -std::max(it, 1) : it;
-}
-
-int Engine::pcg(System &S, int ktop, const double *b, double *x) {
-  if (h->cfg.persistent == 2 && h->pcg2_grid > 0) return pcg_persistent2(S, ktop, b, x);
-  if (h->cfg.persistent) return pcg_persistent(S, ktop, b, x);
-  SysLevel &Lv = S.lev[ktop];
-  const int64_t m = Lv.m;
-  double *r = S.pc_r, *p = S.pc_p;
-  double *scal = h->dscal + 8;
-  const unsigned int rg = red_grid(m);
-  zero(S.pc_x, m);
-  zero(p, m);
-  copy(r, b, m);
-  LAUNCH(KC_VEC, k_dot<<<rg, kRedThreads, 0, s>>>(m, r, r, h->partials, h->ticket, scal + 2));
-  LAUNCH(KC_VEC, k_pcg_init<<<1, 1, 0, s>>>(scal));
-  CK(cudaMemcpyAsync(h->hscal + 8, scal, sizeof(double) * 5, cudaMemcpyDeviceToHost, s));
-  sync();
-  const double bb = h->hscal[10];
-  h->last_solve_status = 1;
-  h->last_solve_rel = 0.0;
-  h->last_solve_erel = 0.0;
-  if (!(bb > 0.0) || !std::isfinite(bb)) {
-    zero(x, m);
-    return 0;
-  }
-  double e_tot = 0.0, e_hist[4] = {0.0, 0.0, 0.0, 0.0};
-  const double target = h->cur_rtol2 * bb;
-  // the iteration body is captured once per (system, top level) and replayed as a CUDA graph
-  cudaGraphExec_t gexec = nullptr;
-  const bool use_graph = h->cfg.use_graphs && !h->cfg.profile;
-  if (use_graph) {
-    auto it = S.graphs.find(ktop);
-    if (it == S.graphs.end()) {
-      cudaGraph_t graph = nullptr;
-      CK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-      const int64_t l0 = h->launches;
-      try {
-        pcg_iteration(S, ktop);
-      } catch (...) {
-        cudaStreamEndCapture(s, &graph);
-        if (graph) cudaGraphDestroy(graph);
-        throw;
-      }
-      S.graph_launches[ktop] = h->launches - l0;
-      h->launches = l0;
-      CK(cudaStreamEndCapture(s, &graph));
-      CK(cudaGraphInstantiate(&gexec, graph, 0));
-      cudaGraphDestroy(graph);
-      S.graphs[ktop] = gexec;
-    } else {
-      gexec = it->second;
-    }
-  }
-  int it = 0;
-  double best = bb;
-  int since_best = 0;
-  int status = 1;
-  while (it < h->cfg.pcg_maxit) {
-    if (gexec) {
-      CK(cudaGraphLaunch(gexec, s));
-      h->launches += S.graph_launches[ktop];
-      h->kc_launches[KC_VEC] += 0;
-    } else {
-      pcg_iteration(S, ktop);
-    }
-    ++it;
-    sync();
-    const double rr = h->hscal[10];
-    if (!std::isfinite(rr) || !(h->hscal[9] > 0.0)) {   // breakdown (indefinite or non-finite)
-      status = -1;
-      break;
-    }
-    h->last_solve_rel = std::sqrt(rr / bb);
-    e_hist[it & 3] = e_tot;                                  // value four iterations ago is overwritten next time round
-    e_tot += h->hscal[8] * h->hscal[8] / h->hscal[9];        // alpha (r.z) = (r.z)^2 / p.Ap
-    h->last_solve_erel = e_tot > 0.0 ? (e_tot - e_hist[(it + 1) & 3]) / e_tot : 0.0;
-    if (rr <= target) break;
-    if (rr < best * 0.999) {
-      best = rr;
-      since_best = 0;
-    } else if (++since_best >= h->cur_window) {
-      status = 2;   // stagnation at the attainable accuracy
-      break;
-    }
-  }
-  if (status == 1 && it >= h->cfg.pcg_maxit && h->last_solve_rel * h->last_solve_rel > h->cur_rtol2) status = 3;
-  h->last_solve_status = status;
-  copy(x, S.pc_x, m);
-  return (status < 0 ? -1 : 1) * it;
 }
 
 int Engine::solve_compact(System &S, int ktop, const double *b, double *x) {
@@ -2935,7 +2585,6 @@ void mgbx_default_config(mgbx_config *c) {
   c->device = -1;
   c->verbose = 0;
   c->profile = 0;
-  c->use_graphs = 1;
   c->persistent = 2;
   c->tail_max = 1200;
   c->pcg_rtol_final = 1e-15;
@@ -2943,7 +2592,6 @@ void mgbx_default_config(mgbx_config *c) {
   c->smoother = 1;
   c->cheb_ratio = 8.0;
   c->precond_fp32 = 2;
-  c->pcg_lanes = 0;
   c->lambda_power = -1;
   c->pcg_fail_rtol = 1e-5;
   c->pcg_fail_etol = 1e-8;
@@ -2996,6 +2644,7 @@ int mgbx_create(const mgbx_problem *prob, const mgbx_config *cfg, mgbx_handle **
   if (h->cfg.coarse_max < 0) h->cfg.coarse_max = 0;
   h->cur_rtol2 = h->cfg.pcg_rtol * h->cfg.pcg_rtol;
   int rc = guarded(h, [&]() -> int {
+    if (h->cfg.persistent != 2) throw ArgError("mgbx_config.persistent must be 2 (the only solve kernel)");
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
     if (e != cudaSuccess || ndev == 0)
@@ -3006,18 +2655,14 @@ int mgbx_create(const mgbx_problem *prob, const mgbx_config *cfg, mgbx_handle **
     CK(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
     h->pool.stream = h->stream;
     {
-      int dev = 0, nsm = 0, coop = 0, per_sm = 0;
+      int dev = 0;
       CK(cudaGetDevice(&dev));
       cudaMemPool_t mp = nullptr;
       CK(cudaDeviceGetDefaultMemPool(&mp, dev));
       uint64_t keep = UINT64_MAX;   // freed blocks stay cached in the pool: the next handle reuses them without driver calls
       CK(cudaMemPoolSetAttribute(mp, cudaMemPoolAttrReleaseThreshold, &keep));
-      CK(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev));
-      CK(cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev));
-      CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_pcg_persistent, kPcgThreads, 0));
-      if (!coop || per_sm < 1) throw std::runtime_error("CUDA device cannot run the cooperative persistent solve kernel");
-      h->pcg_grid = std::min(nsm, kPcgMaxGrid);   // one CTA per SM
       h->pcg2_grid = pcg2_grid(dev);
+      if (h->pcg2_grid == 0) throw std::runtime_error("CUDA device cannot run the cooperative solve kernel");
       CK(cudaFuncSetAttribute(k_coarse_inverse, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coarse_inverse_smem(kCoarseMaxDense)));
       CK(cudaFuncSetAttribute(k_dense_solve_small, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dense_solve_small_smem(kCoarseMaxDense)));
       CK(cudaFuncSetAttribute(k_chol_diag_inv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCholDiagSmem));
@@ -3074,10 +2719,6 @@ void mgbx_destroy(mgbx_handle *h) {
   }
   if (h->comm && h->comm == g_comm && g_comm_users > 0) --g_comm_users;
   if (h->stream) cudaStreamSynchronize(h->stream);
-  for (int w = 0; w < 2; ++w)
-    for (System *S : {h->amg[w].sys_cond.get(), h->amg[w].sys_coarse.get(), h->amg[w].sys_hook.get()})
-      if (S)
-        for (auto &kv : S->graphs) cudaGraphExecDestroy(kv.second);
   for (int w = 0; w < 2; ++w)
     for (System *S : {h->amg[w].sys_cond.get(), h->amg[w].sys_coarse.get(), h->amg[w].sys_hook.get()})
       if (S)
@@ -3342,9 +2983,9 @@ int mgbx_solver_info(mgbx_handle *h, int which, mgbx_solver_info_t *out) {
     out->condensed = S->condensed ? 1 : 0;
     out->assembly_terms = S->top.nterms;
     out->hblk_entries = S->hblk_size;
-    auto it2 = S->pplans2.find(0);
-    if (it2 != S->pplans2.end()) {
-      const Pcg2Plan &P = it2->second.host;
+    auto it = S->pplans2.find(0);
+    if (it != S->pplans2.end()) {
+      const Pcg2Plan &P = it->second.host;
       out->nlev = P.nlev;
       out->nbig = P.nbig;
       out->bottom_dense = P.bottom_dense;
@@ -3358,20 +2999,6 @@ int mgbx_solver_info(mgbx_handle *h, int which, mgbx_solver_info_t *out) {
         out->m[q] = P.lev[q].m;
         out->nnz[q] = Lv.A.nnz;
         out->nnzT[q] = (q + 1 < P.nlev) ? Lv.T.nnz : 0;
-      }
-    }
-    auto it = S->pplans.find(0);
-    if (it2 == S->pplans2.end() && it != S->pplans.end()) {
-      const PcgPlan &P = it->second.host;
-      out->nlev = P.nlev;
-      out->nbig = P.nbig;
-      out->bottom_dense = P.bottom_dense;
-      out->grid = h->pcg_grid;
-      out->threads = kPcgThreads;
-      for (int q = 0; q < P.nlev; ++q) {
-        out->m[q] = P.lev[q].m;
-        out->nnz[q] = P.lev[q].A.nnz;
-        out->nnzT[q] = (q + 1 < P.nlev) ? P.lev[q].T.nnz : 0;
       }
     }
     for (auto &Lv : S->lev) out->galerkin_terms += Lv.s1.nterms + Lv.s2.nterms;

@@ -1,4 +1,4 @@
-// pcg2.cu -- second-generation persistent V-cycle-PCG solve kernel (see pcg2.hpp for what it replaces and why).
+// pcg2.cu -- the persistent V-cycle-PCG solve kernel k_pcg2 (see pcg2.hpp for what it replaces and how).
 //
 // One cooperative launch = one Newton system H d = g solved to the requested relative residual:
 //   repeat { z = V-cycle(r);  beta = r.z / r.z_old;  p = z + beta p;  Ap = A p;  alpha = r.z / p.Ap;  x += alpha p;  r -= alpha Ap }

@@ -1,8 +1,9 @@
-// pcg2.hpp -- interface of the second-generation persistent solve kernel (pcg2.cu, its own translation unit).
+// pcg2.hpp -- interface of the persistent solve kernel k_pcg2 (pcg2.cu, its own translation unit).
 //
-// Replaces, like k_pcg_persistent before it, the reference's `solve(Symmetric(H), g)` (src/utils.jl:142-145: CHOLMOD; cuDSS in
-// ext/MultiGridBarrierCUDAExt/cudss_solver.jl:264-381) by ONE cooperative launch that runs the whole V-cycle-preconditioned CG.
-// What changed against the first generation (solver_kernels.cuh):
+// Replaces the reference's `solve(Symmetric(H), g)` (src/utils.jl:142-145: CHOLMOD; cuDSS in
+// ext/MultiGridBarrierCUDAExt/cudss_solver.jl:264-381) by ONE cooperative launch that runs the whole V-cycle-preconditioned CG:
+// every smoother sweep, residual, grid transfer, dot product and the convergence test, phases separated by grid barriers.
+// Design:
 //   * every level matrix (A, T, T') is stored as sliced ELL, 32 rows per slice, column-major inside a slice: a warp owns a slice,
 //     lane = row, so index / value loads are coalesced and a row's loads are independent of each other (no row-pointer ->
 //     entry chain; the only dependent load left is the gather of the vector entry);
@@ -10,7 +11,7 @@
 //     slices round-robin -- the mapping the multi-GPU row partition extends (a rank owns a block of CTAs' blocks);
 //   * the single-CTA tail levels keep their matrices in CTA 0's shared memory (copied once per launch);
 //   * distinct exit states (converged / stagnated / iteration limit / breakdown).
-// Row sums run over a row's entries in column order, as the CSR one-lane-per-row kernel did: results are deterministic.
+// Row sums run over a row's entries in column order: results are deterministic.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>

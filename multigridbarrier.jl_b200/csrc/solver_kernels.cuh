@@ -1,20 +1,14 @@
-// solver_kernels.cuh -- the Newton-system solve as ONE persistent cooperative kernel, the Galerkin
-// gather plans (sliced-ELL) and the coarse dense inverse.
+// solver_kernels.cuh -- the Galerkin gather plans (sliced-ELL), the coarse dense inverse and the small direct solve.
+// The Newton-system solve itself is k_pcg2 (pcg2.hpp / pcg2.cu).
 //
 // What this replaces in the reference (paths under /root/reference):
-//   k_pcg_persistent   solve(Symmetric(H), g)  src/utils.jl:142-145 (CHOLMOD) and the CUDA extension's cuDSS
-//                      analysis/factor/solve (ext/MultiGridBarrierCUDAExt/cudss_solver.jl:264-381): a whole
-//                      V-cycle-preconditioned CG solve -- every smoother sweep, residual, grid transfer, dot
-//                      product and the convergence test -- runs in one launch with one CTA per SM; phases are
-//                      separated by a grid barrier (release/acquire on one counter), levels below `nbig`
-//                      are handled by CTA 0 alone with __syncthreads.  Only {iterations, |r|^2, status}
-//                      return to the host.
-//   k_sell_gather      the numeric Galerkin products A_c = T'(A T) (north-star item 3) and the R'HR scatter
-//                      of src/BlockMatrices.jl:506-555, as fixed-order gathers over a sliced-ELL term list
-//                      (coalesced index/weight streams, deterministic; the reference CUDA ext uses FP64 atomics,
-//                      block_ops.jl:229-249).
-//   k_prod_count/fill  build those term lists on the device (setup, once per system).
-//   k_coarse_inverse   dense Cholesky + explicit inverse of the coarsest level in shared memory (one CTA).
+//   k_sell_gather        the numeric Galerkin products A_c = T'(A T) (north-star item 3) and the R'HR scatter
+//                        of src/BlockMatrices.jl:506-555, as fixed-order gathers over a sliced-ELL term list
+//                        (coalesced index/weight streams, deterministic; the reference CUDA ext uses FP64 atomics,
+//                        block_ops.jl:229-249).
+//   k_prod_plan<0|1>     build those term lists on the device (setup, once per system).
+//   k_coarse_inverse     dense Cholesky + explicit inverse of the coarsest level in shared memory (one CTA).
+//   k_dense_solve_small  solve(Symmetric(H), g) (src/utils.jl:142-145) of a small system in one CTA.
 #pragma once
 #include "kernels.cuh"
 
@@ -48,11 +42,6 @@ __global__ void __launch_bounds__(256) k_sell_gather(SellPlan P, const double *_
 __global__ void k_f64_to_f32(int64_t n, const double *__restrict__ a, float *__restrict__ out) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = (float)a[i];
-}
-
-__global__ void k_ptr32(int64_t n, const int64_t *__restrict__ p64, int *p32) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) p32[i] = (int)p64[i];
 }
 
 // row index of every non-zero of a CSR pattern
@@ -309,523 +298,5 @@ __global__ void __launch_bounds__(1024) k_dense_solve_small(DevCsr A, const doub
   if (tid == 0 && info) info[0] = 1;
 }
 inline size_t dense_solve_small_smem(int m) { return sizeof(double) * ((size_t)m * (m + 1) + 2 * (size_t)m); }
-
-// ------------------------------------------------------------------------------------------------
-// persistent PCG
-// ------------------------------------------------------------------------------------------------
-constexpr int kPcgThreads = 1024;
-constexpr int kPcgMaxGrid = 1024;   // partial slots per reduction
-
-// 32-bit view of a level matrix inside the persistent kernel: halves the index arithmetic, and the explicit
-// __ldg (matrix data: immutable while the kernel runs) / __ldcg (vectors other CTAs wrote in the previous phase: read
-// at L2, never from a stale L1 line) keep the loads on the global path although the pointers come from shared memory.
-struct Csr32 {
-  int rows, nnz;
-  const int *ptr;
-  const int *idx;
-  const double *val;
-  const float *valf;   // optional FP32 copy of the values (preconditioner passes only): 8 instead of 12 bytes per non-zero
-};
-
-struct PLevel {
-  int64_t m;
-  Csr32 A, T, Tt;        // T: this level <- next coarser active level; Tt its transpose (32-bit row pointers)
-  const double *dinv;    // l1-Jacobi: 1 / sum_j |a_ij|
-  const double *diag;    // 1 / a_ii (Chebyshev)
-  const double *lam;     // Gershgorin bound of lambda_max(D^-1 A), refreshed with the matrix values
-  double *b, *x, *x2, *r;
-  int G, GT, GTt;        // lanes per row
-};
-
-struct PcgPlan {
-  int nlev, nbig;        // active levels: [0, nbig) by the whole grid, [nbig, nlev) by CTA 0 alone
-  int bottom_dense;      // the last level is applied through dense_inv
-  int nu, nu_bottom;     // smoother sweeps (pre = post = nu), sweeps on an iterated bottom level
-  int smoother;          // 0: l1-Jacobi, 1: Chebyshev of degree nu on [lam/cheb_ratio, lam] with diagonal scaling
-  double cheb_ratio;
-  int maxit;
-  double rtol2;
-  PLevel lev[MGBX_MAX_LEVELS];
-  const double *dense_inv;
-  double *r, *p, *p2, *Ap, *x;
-  const double *b;
-  double *partials;      // 3 x kPcgMaxGrid
-  unsigned int *bar;
-  double *out;           // [0] iterations, [1] |r|^2, [2] status (1 converged, 2 stagnated above the tolerance, 3 iteration limit, -1 breakdown), [3] |b|^2
-};
-
-__device__ __forceinline__ void grid_barrier(unsigned int *bar) {
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    unsigned int nb = 1;
-    if (blockIdx.x == 0) nb = 0x80000000u - (gridDim.x - 1);
-    unsigned int old, cur;
-    asm volatile("atom.add.release.gpu.u32 %0,[%1],%2;" : "=r"(old) : "l"(bar), "r"(nb) : "memory");
-    int spins = 0;
-    do {
-      asm volatile("ld.acquire.gpu.u32 %0,[%1];" : "=r"(cur) : "l"(bar) : "memory");
-      if (++spins > 64) __nanosleep(40);
-    } while (((old ^ cur) & 0x80000000u) == 0);
-  }
-  __syncthreads();
-}
-
-// scope of a phase: the whole grid (GRID) or one CTA
-template <bool GRID>
-struct Scope {
-  int64_t tid, nthr;
-  unsigned int *bar;
-  __device__ __forceinline__ void sync() const {
-    if (GRID) grid_barrier(bar);
-    else __syncthreads();
-  }
-};
-
-template <int G>
-__device__ __forceinline__ double row_dot(const Csr32 &A, int row, int sub, bool valid, const double *x) {
-  double acc = 0.0;
-  if (valid) {
-    const int b = __ldg(A.ptr + row), e = __ldg(A.ptr + row + 1);
-    if (A.valf) {
-      for (int k = b + sub; k < e; k += G) acc += (double)__ldg(A.valf + k) * __ldcg(x + __ldg(A.idx + k));
-    } else {
-      for (int k = b + sub; k < e; k += G) acc += __ldg(A.val + k) * __ldcg(x + __ldg(A.idx + k));
-    }
-  }
-  if (G > 1) {
-#pragma unroll
-    for (int o = G / 2; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o, G);
-  }
-  return acc;
-}
-
-// y = alpha * A x + (y0 ? y0 : 0)     (y may alias y0; y must not alias x)
-template <int G, class SC>
-__device__ void ph_spmv(const SC &sc, const Csr32 &A, const double *x, const double *y0, double alpha, double *y) {
-  const int step = (int)(sc.nthr / G);
-  const int sub = (int)(sc.tid % G), r0 = (int)(sc.tid / G);
-  for (int base = 0; base < A.rows; base += step) {
-    const int row = base + r0;
-    const bool valid = row < A.rows;
-    const double acc = row_dot<G>(A, row, sub, valid, x);
-    if (valid && sub == 0) y[row] = alpha * acc + (y0 ? __ldcg(y0 + row) : 0.0);
-  }
-}
-
-// two l1-Jacobi sweeps from x = 0:  x1 = dinv b;  x = x1 + dinv (b - A x1)
-template <int G, class SC>
-__device__ void ph_jacobi_first2(const SC &sc, const Csr32 &A, const double *dinv, const double *b, double *xnew) {
-  const int step = (int)(sc.nthr / G);
-  const int sub = (int)(sc.tid % G), r0 = (int)(sc.tid / G);
-  for (int base = 0; base < A.rows; base += step) {
-    const int row = base + r0;
-    const bool valid = row < A.rows;
-    double acc = 0.0;
-    if (valid) {
-      const int bb = __ldg(A.ptr + row), e = __ldg(A.ptr + row + 1);
-      for (int k = bb + sub; k < e; k += G) {
-        const int j = __ldg(A.idx + k);
-        acc += (A.valf ? (double)__ldg(A.valf + k) : __ldg(A.val + k)) * (__ldg(dinv + j) * __ldcg(b + j));
-      }
-    }
-    if (G > 1) {
-#pragma unroll
-      for (int o = G / 2; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o, G);
-    }
-    if (valid && sub == 0) {
-      const double d = __ldg(dinv + row), bi = __ldcg(b + row);
-      const double x1 = d * bi;
-      xnew[row] = x1 + d * (bi - acc);
-    }
-  }
-}
-
-// xnew = x + dinv (b - A x); returns this thread's share of sum_i dotw[i] * xnew[i] (0 if dotw == nullptr)
-template <int G, class SC>
-__device__ double ph_jacobi(const SC &sc, const Csr32 &A, const double *dinv, const double *b, const double *x, double *xnew,
-                            const double *dotw) {
-  const int step = (int)(sc.nthr / G);
-  const int sub = (int)(sc.tid % G), r0 = (int)(sc.tid / G);
-  double part = 0.0;
-  for (int base = 0; base < A.rows; base += step) {
-    const int row = base + r0;
-    const bool valid = row < A.rows;
-    const double acc = row_dot<G>(A, row, sub, valid, x);
-    if (valid && sub == 0) {
-      const double v = __ldcg(x + row) + __ldg(dinv + row) * (__ldcg(b + row) - acc);
-      xnew[row] = v;
-      if (dotw) part += __ldcg(dotw + row) * v;
-    }
-  }
-  return part;
-}
-
-// ---- Chebyshev smoothing (degree nu, diagonal preconditioning) -------------------------------------------
-// 3-term recurrence on [a, b] = [lam/ratio, lam]:  theta = (a+b)/2, delta = (b-a)/2, sigma = theta/delta,
-// rho_0 = 1/sigma, rho_k = 1/(2 sigma - rho_{k-1});  d_0 = D^-1 r_0 / theta,
-// d_k = rho_k rho_{k-1} d_{k-1} + (2 rho_k / delta) D^-1 r_k,  x_{k+1} = x_k + d_k.  The error propagator is a
-// polynomial in D^-1 A, hence A-self-adjoint: the same sweeps before and after the coarse correction keep the
-// V-cycle a symmetric preconditioner.  `idiag` holds 1 / a_ii.
-struct Cheb {
-  double th_inv, sigma, delta;
-  __device__ __forceinline__ Cheb(double lam, double ratio) {
-    const double b = lam, a = lam / ratio;
-    const double theta = 0.5 * (a + b);
-    delta = 0.5 * (b - a);
-    sigma = theta / delta;
-    th_inv = 1.0 / theta;
-  }
-  // coefficients of step k >= 1 given rho_{k-1}; returns rho_k
-  __device__ __forceinline__ double step(double rho_prev, double &c_dd, double &c_dr) const {
-    const double rho = 1.0 / (2.0 * sigma - rho_prev);
-    c_dd = rho * rho_prev;
-    c_dr = 2.0 * rho / delta;
-    return rho;
-  }
-};
-
-// steps 0 and 1 from x = 0 in one pass: d0 = th_inv D^-1 b; r1 = b - A d0; d1 = c_dd d0 + c_dr D^-1 r1; x = d0 + d1
-template <int G, class SC>
-__device__ void ph_cheb_first2(const SC &sc, const Csr32 &A, const double *idiag, const double *b, double *xnew, double *d,
-                               double th_inv, double c_dd, double c_dr) {
-  const int step = (int)(sc.nthr / G);
-  const int sub = (int)(sc.tid % G), r0 = (int)(sc.tid / G);
-  for (int base = 0; base < A.rows; base += step) {
-    const int row = base + r0;
-    const bool valid = row < A.rows;
-    double acc = 0.0;
-    if (valid) {
-      const int bb = __ldg(A.ptr + row), e = __ldg(A.ptr + row + 1);
-      for (int k = bb + sub; k < e; k += G) {
-        const int j = __ldg(A.idx + k);
-        acc += (A.valf ? (double)__ldg(A.valf + k) : __ldg(A.val + k)) * (__ldcg(b + j) * __ldg(idiag + j));
-      }
-    }
-    if (G > 1) {
-#pragma unroll
-      for (int o = G / 2; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o, G);
-    }
-    if (valid && sub == 0) {
-      const double di = __ldg(idiag + row), bi = __ldcg(b + row);
-      const double d0 = th_inv * bi * di;
-      const double d1 = c_dd * d0 + c_dr * (bi - th_inv * acc) * di;
-      xnew[row] = d0 + d1;
-      d[row] = d1;
-    }
-  }
-}
-
-// one step on an existing iterate: r = b - A x; d = (first ? th_inv D^-1 r : c_dd d + c_dr D^-1 r); xnew = x + d
-template <int G, class SC>
-__device__ double ph_cheb_step(const SC &sc, const Csr32 &A, const double *idiag, const double *b, const double *x, double *xnew,
-                               double *d, bool first, double th_inv, double c_dd, double c_dr, const double *dotw) {
-  const int step = (int)(sc.nthr / G);
-  const int sub = (int)(sc.tid % G), r0 = (int)(sc.tid / G);
-  double part = 0.0;
-  for (int base = 0; base < A.rows; base += step) {
-    const int row = base + r0;
-    const bool valid = row < A.rows;
-    const double acc = row_dot<G>(A, row, sub, valid, x);
-    if (valid && sub == 0) {
-      const double rr = (__ldcg(b + row) - acc) * __ldg(idiag + row);
-      const double dn = first ? th_inv * rr : c_dd * d[row] + c_dr * rr;
-      const double v = __ldcg(x + row) + dn;
-      d[row] = dn;
-      xnew[row] = v;
-      if (dotw) part += __ldcg(dotw + row) * v;
-    }
-  }
-  return part;
-}
-
-#define MGBX_G_DISPATCH(G, CALL) \
-  do {                            \
-    if ((G) == 32) { constexpr int GG = 32; CALL; } \
-    else if ((G) == 16) { constexpr int GG = 16; CALL; } \
-    else if ((G) == 8) { constexpr int GG = 8; CALL; } \
-    else if ((G) == 4) { constexpr int GG = 4; CALL; } \
-    else if ((G) == 2) { constexpr int GG = 2; CALL; } \
-    else { constexpr int GG = 1; CALL; } \
-  } while (0)
-
-// x = dense_inv * b, one warp per row
-template <class SC>
-__device__ void ph_dense_apply(const SC &sc, const double *Minv, int m, const double *b, double *x) {
-  const int lane = (int)(sc.tid & 31);
-  const int64_t nw = sc.nthr >> 5;
-  for (int64_t row = sc.tid >> 5; row < m; row += nw) {
-    const double *r = Minv + (size_t)row * m;
-    double s = 0.0;
-    for (int j = lane; j < m; j += 32) s += r[j] * b[j];
-    s = warp_sum(s);
-    if (lane == 0) x[row] = s;
-  }
-}
-
-// block-wide sum, result broadcast to every thread (fixed order)
-__device__ __forceinline__ double block_sum_bcast(double v) {
-  __shared__ double wsum[32];
-  __shared__ double total;
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
-  v = warp_sum(v);
-  __syncthreads();   // protects wsum / total from the previous call
-  if (lane == 0) wsum[wid] = v;
-  __syncthreads();
-  if (wid == 0) {
-    double x = lane < nw ? wsum[lane] : 0.0;
-    x = warp_sum(x);
-    if (lane == 0) total = x;
-  }
-  __syncthreads();
-  return total;
-}
-
-// deposit this CTA's partial, grid barrier, then every CTA sums all partials in the same fixed order
-__device__ __forceinline__ double grid_sum(double part, double *slot, unsigned int *bar) {
-  const double bs = block_sum_bcast(part);
-  if (threadIdx.x == 0) slot[blockIdx.x] = bs;
-  grid_barrier(bar);
-  double v = 0.0;
-  for (unsigned int b = threadIdx.x; b < gridDim.x; b += blockDim.x) v += slot[b];
-  return block_sum_bcast(v);
-}
-
-// V-cycle over the active levels [k0, k1) in scope `sc`; btop: right-hand side of level k0.  After the
-// down-sweep of level k1-1 the coarser levels (if any) are run by CTA 0 alone (GRID scope only).  The
-// result is in lev[k0].x: the ping-pong between x and x2 starts on the buffer that makes the last sweep
-// land in x, so no pointer is ever swapped and every CTA agrees on where results live.
-// dot_top != nullptr: returns this thread's share of sum dot_top[i] * x[i] on level k0, and the barrier after
-// the last sweep is left to the caller's grid_sum.
-template <bool GRID>
-__device__ double vcycle_levels(const PcgPlan &P, const Scope<GRID> &sc, int k0, int k1, const double *btop, const double *dot_top) {
-  double part = 0.0;
-  // ---- down
-  for (int k = k0; k < k1; ++k) {
-    const PLevel &Lv = P.lev[k];
-    const double *bk = (k == k0) ? btop : Lv.b;
-    const bool last = (k == P.nlev - 1);
-    if (last && P.bottom_dense) {
-      ph_dense_apply(sc, P.dense_inv, (int)Lv.m, bk, Lv.x);
-      sc.sync();
-      continue;
-    }
-    const bool cheb = (P.smoother == 1) && !last;   // an iterated bottom level keeps l1-Jacobi
-    const int want = last ? P.nu_bottom : P.nu;
-    const int done = (want >= 2) ? 2 : 1;
-    const int npre = want - done, npost = last ? 0 : P.nu;
-    double *cur = ((npre + npost) & 1) ? Lv.x2 : Lv.x, *oth = ((npre + npost) & 1) ? Lv.x : Lv.x2;
-    if (cheb) {
-      const Cheb C(*Lv.lam, P.cheb_ratio);
-      double rho = 1.0 / C.sigma, c_dd = 0.0, c_dr = 0.0;
-      if (done == 2) {
-        rho = C.step(rho, c_dd, c_dr);
-        MGBX_G_DISPATCH(Lv.G, (ph_cheb_first2<GG>(sc, Lv.A, Lv.diag, bk, cur, Lv.r, C.th_inv, c_dd, c_dr)));
-      } else {
-        for (int64_t i = sc.tid; i < Lv.m; i += sc.nthr) {
-          const double d0 = C.th_inv * bk[i] / Lv.diag[i];
-          cur[i] = d0;
-          Lv.r[i] = d0;
-        }
-      }
-      sc.sync();
-      for (int it = 0; it < npre; ++it) {
-        rho = C.step(rho, c_dd, c_dr);
-        MGBX_G_DISPATCH(Lv.G, (ph_cheb_step<GG>(sc, Lv.A, Lv.diag, bk, cur, oth, Lv.r, false, C.th_inv, c_dd, c_dr, nullptr)));
-        sc.sync();
-        double *t = cur;
-        cur = oth;
-        oth = t;
-      }
-    } else {
-      if (done == 2) {
-        MGBX_G_DISPATCH(Lv.G, (ph_jacobi_first2<GG>(sc, Lv.A, Lv.dinv, bk, cur)));
-      } else {
-        for (int64_t i = sc.tid; i < Lv.m; i += sc.nthr) cur[i] = Lv.dinv[i] * bk[i];
-      }
-      sc.sync();
-      for (int it = 0; it < npre; ++it) {
-        MGBX_G_DISPATCH(Lv.G, (ph_jacobi<GG>(sc, Lv.A, Lv.dinv, bk, cur, oth, nullptr)));
-        sc.sync();
-        double *t = cur;
-        cur = oth;
-        oth = t;
-      }
-    }
-    if (!last) {
-      MGBX_G_DISPATCH(Lv.G, (ph_spmv<GG>(sc, Lv.A, cur, bk, -1.0, Lv.r)));
-      sc.sync();
-      MGBX_G_DISPATCH(Lv.GTt, (ph_spmv<GG>(sc, Lv.Tt, Lv.r, nullptr, 1.0, P.lev[k + 1].b)));
-      sc.sync();
-    }
-  }
-  // ---- coarser levels by CTA 0 alone
-  if (GRID && k1 < P.nlev) {
-    if (blockIdx.x == 0) {
-      Scope<false> cta{(int64_t)threadIdx.x, (int64_t)blockDim.x, nullptr};
-      vcycle_levels<false>(P, cta, k1, P.nlev, P.lev[k1].b, nullptr);
-    }
-    sc.sync();
-  }
-  // ---- up
-  for (int k = k1 - 1; k >= k0; --k) {
-    if (k == P.nlev - 1) continue;   // bottom level: nothing coarser
-    const PLevel &Lv = P.lev[k];
-    const double *bk = (k == k0) ? btop : Lv.b;
-    const int want = P.nu;
-    const int done = (want >= 2) ? 2 : 1;
-    const int npre = want - done, npost = P.nu;
-    // buffer holding the pre-smoothed iterate: start buffer advanced by npre swaps
-    const bool start_x2 = ((npre + npost) & 1) != 0;
-    const bool cur_x2 = start_x2 != ((npre & 1) != 0);
-    double *cur = cur_x2 ? Lv.x2 : Lv.x, *oth = cur_x2 ? Lv.x : Lv.x2;
-    MGBX_G_DISPATCH(Lv.GT, (ph_spmv<GG>(sc, Lv.T, P.lev[k + 1].x, cur, 1.0, cur)));   // x += T xc (row-local)
-    sc.sync();
-    const bool cheb = (P.smoother == 1);
-    const Cheb C(cheb ? *Lv.lam : 1.0, P.cheb_ratio);
-    double rho = 1.0 / C.sigma, c_dd = 0.0, c_dr = 0.0;
-    for (int it = 0; it < npost; ++it) {
-      const bool fin = (it == npost - 1) && (k == k0) && (dot_top != nullptr);
-      double pp = 0.0;
-      if (cheb) {
-        if (it > 0) rho = C.step(rho, c_dd, c_dr);
-        MGBX_G_DISPATCH(Lv.G, (pp = ph_cheb_step<GG>(sc, Lv.A, Lv.diag, bk, cur, oth, Lv.r, it == 0, C.th_inv, c_dd, c_dr,
-                                                     fin ? dot_top : nullptr)));
-      } else {
-        MGBX_G_DISPATCH(Lv.G, (pp = ph_jacobi<GG>(sc, Lv.A, Lv.dinv, bk, cur, oth, fin ? dot_top : nullptr)));
-      }
-      part += pp;
-      if (!fin) sc.sync();
-      double *t = cur;
-      cur = oth;
-      oth = t;
-    }
-  }
-  return part;
-}
-
-__global__ void __launch_bounds__(kPcgThreads, 1) k_pcg_persistent(const PcgPlan *plan_g, double rtol2, int maxit, int stall_window) {
-  __shared__ PcgPlan P;
-  {
-    const uint64_t *src = reinterpret_cast<const uint64_t *>(plan_g);
-    uint64_t *dst = reinterpret_cast<uint64_t *>(&P);
-    for (int i = threadIdx.x; i < (int)(sizeof(PcgPlan) / sizeof(uint64_t)); i += blockDim.x) dst[i] = src[i];
-  }
-  __syncthreads();
-  const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t nthr = (int64_t)gridDim.x * blockDim.x;
-  Scope<true> sc{tid, nthr, P.bar};
-  const int64_t m = P.lev[0].m;
-  double *slot0 = P.partials, *slot1 = P.partials + kPcgMaxGrid, *slot2 = P.partials + 2 * kPcgMaxGrid;
-
-  // the plan in shared memory is read-only from here on; the p / p2 ping-pong lives in registers
-  double *pv = P.p, *pv2 = P.p2;
-  // x = 0, p = 0, r = b, |b|^2
-  double part = 0.0;
-  for (int64_t i = tid; i < m; i += nthr) {
-    const double bi = P.b[i];
-    P.x[i] = 0.0;
-    pv[i] = 0.0;
-    P.r[i] = bi;
-    part += bi * bi;
-  }
-  const double bb = grid_sum(part, slot0, P.bar);
-  int it = 0;
-  double rr = bb, status = 1.0, e_tot = 0.0, e_last4 = 0.0;
-  if (bb > 0.0 && isfinite(bb)) {
-    const double target = rtol2 * bb;
-    double rz_old = 1.0, best = bb;
-    int since_best = 0;
-    // energy bookkeeping: for CG from x = 0, b.x_k = |x_k|_A^2 = sum_j alpha_j (r.z)_j grows monotonically to b.A^-1 b -- the
-    // Newton decrement the caller needs; e_m4 is its value four iterations ago
-    double e_m1 = 0.0, e_m2 = 0.0, e_m3 = 0.0, e_m4 = 0.0;
-    const PLevel &top = P.lev[0];
-    while (it < maxit) {
-      // z = M^{-1} r, with r.z accumulated in the last smoothing sweep of the top level
-      const bool single = (P.nlev == 1);
-      double prz = vcycle_levels<true>(P, sc, 0, P.nbig, P.r, single ? nullptr : P.r);
-      const double *z = P.lev[0].x;
-      if (single) {   // one-level "hierarchy": no up-sweep ran, take the dot here
-        prz = 0.0;
-        for (int64_t i = tid; i < m; i += nthr) prz += P.r[i] * __ldcg(z + i);
-      }
-      const double rz = grid_sum(prz, slot1, P.bar);
-      const double beta = rz / rz_old;
-      rz_old = rz;
-      // p2 = z + beta p;  Ap = A p2 (neighbour values formed on the fly);  p2.Ap
-      double ppap = 0.0;
-      {
-        const int G = top.G;
-        const int64_t step = nthr / G;
-        const int sub = (int)(tid % G);
-        for (int64_t base = 0; base < m; base += step) {
-          const int64_t row = base + tid / G;
-          const bool valid = row < m;
-          double acc = 0.0;
-          if (valid) {
-            const int b0 = __ldg(top.A.ptr + row), e0 = __ldg(top.A.ptr + row + 1);
-            for (int k = b0 + sub; k < e0; k += G) {
-              const int j = __ldg(top.A.idx + k);
-              acc += __ldg(top.A.val + k) * (__ldcg(z + j) + beta * __ldcg(pv + j));
-            }
-          }
-          for (int o = G / 2; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o, G);
-          if (valid && sub == 0) {
-            const double pn = __ldcg(z + row) + beta * __ldcg(pv + row);
-            pv2[row] = pn;
-            P.Ap[row] = acc;
-            ppap += pn * acc;
-          }
-        }
-      }
-      const double pAp = grid_sum(ppap, slot2, P.bar);
-      {
-        double *t = pv;
-        pv = pv2;
-        pv2 = t;
-      }
-      ++it;
-      if (!(pAp > 0.0) || !isfinite(pAp)) {
-        status = -1.0;
-        break;
-      }
-      const double alpha = rz / pAp;
-      e_m4 = e_m3;
-      e_m3 = e_m2;
-      e_m2 = e_m1;
-      e_m1 = e_tot;
-      e_tot += alpha * rz;
-      double prr = 0.0;
-      for (int64_t i = tid; i < m; i += nthr) {
-        P.x[i] += alpha * __ldcg(pv + i);
-        const double ri = P.r[i] - alpha * __ldcg(P.Ap + i);
-        P.r[i] = ri;
-        prr += ri * ri;
-      }
-      rr = grid_sum(prr, slot0, P.bar);
-      if (!isfinite(rr)) {
-        status = -1.0;
-        break;
-      }
-      if (rr <= target) break;
-      if (rr < best * 0.999) {
-        best = rr;
-        since_best = 0;
-      } else if (++since_best >= stall_window) {
-        status = 2.0;   // stagnation at the attainable accuracy (above the requested tolerance)
-        break;
-      }
-    }
-    if (status == 1.0 && rr > target) status = 3.0;   // iteration limit
-    e_last4 = e_tot - e_m4;
-  }
-  if (tid == 0) {
-    P.out[0] = (double)it;
-    P.out[1] = rr;
-    P.out[2] = status;
-    P.out[3] = bb;
-    P.out[4] = e_tot;      // b.x = |x|_A^2 (energy of the computed direction)
-    P.out[5] = e_last4;    // the part of it gained in the last four iterations
-  }
-}
 
 }  // namespace mgbx

@@ -56,10 +56,10 @@ class Problem(C.Structure):
 class Config(C.Structure):
     _fields_ = [("dense_direct_max", C.c_int32), ("coarse_max", C.c_int32), ("pcg_maxit", C.c_int32),
                 ("pcg_rtol", C.c_double), ("smoother_sweeps", C.c_int32), ("condense", C.c_int32),
-                ("device", C.c_int32), ("verbose", C.c_int32), ("use_graphs", C.c_int32), ("profile", C.c_int32),
+                ("device", C.c_int32), ("verbose", C.c_int32), ("profile", C.c_int32),
                 ("persistent", C.c_int32), ("tail_max", C.c_int32), ("pcg_rtol_final", C.c_double),
                 ("fused", C.c_int32), ("smoother", C.c_int32), ("cheb_ratio", C.c_double),
-                ("precond_fp32", C.c_int32), ("pcg_lanes", C.c_int32), ("lambda_power", C.c_int32),
+                ("precond_fp32", C.c_int32), ("lambda_power", C.c_int32),
                 ("pcg_fail_rtol", C.c_double), ("pcg_fail_etol", C.c_double), ("pcg_stall_window", C.c_int32), ("direct_fallback", C.c_int32), ("elem_bulk", C.c_int32), ("shard_solve", C.c_int32),
                 ("shard_min_rows", C.c_int32), ("shard_min_nnz", C.c_int32), ("spectral_kron", C.c_int32), ("uncondensed_pcg", C.c_int32), ("analytic_schur", C.c_int32)]
 

@@ -16,7 +16,9 @@ from mgbx import native
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_matches_header_symbols_and_abi_version():
+    """Every symbol include/mgbx.h declares is exported, and the library reports the header's ABI version (2: mgbx_config
+    without use_graphs and pcg_lanes)."""
     hdr = open(os.path.join(ROOT, "include", "mgbx.h")).read()
     declared = set(re.findall(r"\b(mgbx_[a-z0-9_]+)\s*\(", hdr))
     assert declared, "no prototypes found"
@@ -24,7 +26,8 @@ def test_library_exports_every_declared_symbol():
     for name in sorted(declared):
         assert hasattr(L, name), name
     assert set(native.EXPORTS) == declared
-    assert L.mgbx_abi_version() == 1
+    assert re.search(r"#define MGBX_ABI_VERSION (\d+)", hdr).group(1) == "2"
+    assert L.mgbx_abi_version() == 2
 
 
 def test_struct_sizes_match_header():
@@ -86,6 +89,16 @@ def test_no_gpu_is_a_loud_error():
         native.Handle(prob)
     assert e.value.code == native.ERR_CUDA
     assert "no CPU fallback" in str(e.value)
+
+
+def test_solve_kernel_other_than_2_is_refused():
+    """k_pcg2 is the only solve kernel: any other mgbx_config.persistent is an argument error, checked before the device."""
+    prob = default_problem("fem1d_3nodes", 1.0)
+    for persistent in (0, 1, 3):
+        with pytest.raises(native.MgbxError) as e:
+            native.Handle(prob, persistent=persistent)
+        assert e.value.code == native.ERR_ARG
+        assert "persistent" in str(e.value)
 
 
 def test_bad_arguments_are_reported():

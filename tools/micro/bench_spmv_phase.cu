@@ -1,4 +1,4 @@
-// Microbenchmark of ONE mat-vec phase of the persistent solve kernel (csrc/solver_kernels.cuh: ph_spmv / row_dot),
+// Microbenchmark of ONE mat-vec phase of a persistent solve kernel (the CSR phase of the first solve kernel, since replaced by k_pcg2),
 // run the way the kernel runs it: cooperative launch, one CTA of 1024 threads per SM, the matrix L2-resident, phases
 // separated by the same flip grid barrier, every phase reading the vector the previous phase wrote.
 //

@@ -1,4 +1,4 @@
-"""CPU laboratory for the V-cycle preconditioner of the GPU solve (csrc/solver_kernels.cuh), NumPy/SciPy only.
+"""CPU laboratory for the V-cycle preconditioner of the GPU solve (csrc/pcg2.cu), NumPy/SciPy only.
 
 Runs the CPU oracle on a small 3-D (or 2-D) problem, records the finest-level Newton systems (H, g) along the t-ramp,
 condenses the node-local slack exactly as the library does, and counts PCG iterations to a relative residual of 1e-9

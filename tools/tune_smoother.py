@@ -12,9 +12,6 @@ else:
 base = None
 cfgs = json.load(open(sys.argv[2])) if len(sys.argv) > 2 else [dict(), dict(precond_fp32=1), dict(precond_fp32=1, smoother=0), dict(smoother=0)]
 for cfg in cfgs:
-    cfg = dict(cfg); lanes = cfg.pop("_lanes", None)
-    os.environ.pop("MGBX_TUNE_LANES", None)
-    if lanes: os.environ["MGBX_TUNE_LANES"] = lanes
     try:
         for rep in range(2):
             t0 = time.time(); sol = solver.mgb_solve(prob, config=cfg, **kw); dt = time.time() - t0
@@ -22,5 +19,5 @@ for cfg in cfgs:
         print(json.dumps({"cfg": cfg, "failed": repr(e)[:120]}), flush=True)
         continue
     st = sol["stats"]
-    print(json.dumps({"cfg": cfg, "lanes": lanes, "newton": int(sol["SOL_main"]["its"].sum()), "pcg_iters": st["pcg_iters"], "ms_solve": round(st["ms_solve"]), "ms_f2": round(st["ms_f2"]),
+    print(json.dumps({"cfg": cfg, "newton": int(sol["SOL_main"]["its"].sum()), "pcg_iters": st["pcg_iters"], "ms_solve": round(st["ms_solve"]), "ms_f2": round(st["ms_f2"]),
                       "wall_s": round(dt, 2), "z_sum": float(np.sum(sol["z"]))}), flush=True)
