@@ -1,7 +1,13 @@
 """In-tree build of libmgbx.so (nvcc, sm_100a only).  The .so is git-ignored but travels to the GPU box.
 
-Two translation units, compiled in parallel and cached as objects under build/: mgbx.cu (handle, host logic, element / setup /
-dense kernels) and pcg2.cu (the persistent solve kernel)."""
+One translation unit per responsibility, compiled in parallel and cached as objects under build/; each kernel header is
+compiled by one unit only, so that a host-only edit rebuilds one object:
+  mgbx.cu          the C ABI, handle life cycle and NCCL communicator (no kernels)
+  setup.cu         plans, systems and problem upload             (setup_kernels.cuh)
+  evaluate.cu      f0/f1, Hessian assembly, level chain, vectors   (kernels.cuh, dense_kernels.cuh)
+  linear_solve.cu  preconditioner setup, direct and PCG solves     (solver_kernels.cuh)
+  newton.cu        Newton, mgb_step, matched t (no kernels)
+  pcg2.cu          the persistent solve kernel k_pcg2"""
 from __future__ import annotations
 
 import os
@@ -15,9 +21,17 @@ CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libmgbx.so")
 HDR = os.path.join("..", "..", "include", "mgbx.h")
-ALL_HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith((".cuh", ".hpp", ".h"))) + [HDR]
+# headers every host unit includes (engine.hpp and what it pulls in)
+ENGINE = ["engine.hpp", "host_sparse.hpp", "device_common.cuh", "node_barrier.cuh", "pcg2.hpp", HDR]
 # source -> files whose change forces a recompile of that source
-SOURCES = {"mgbx.cu": ["mgbx.cu"] + ALL_HEADERS, "pcg2.cu": ["pcg2.cu", "pcg2.hpp"]}
+SOURCES = {
+    "mgbx.cu": ["mgbx.cu", "host_amg.hpp"] + ENGINE,
+    "setup.cu": ["setup.cu", "setup_kernels.cuh"] + ENGINE,
+    "evaluate.cu": ["evaluate.cu", "kernels.cuh", "dense_kernels.cuh"] + ENGINE,
+    "linear_solve.cu": ["linear_solve.cu", "solver_kernels.cuh"] + ENGINE,
+    "newton.cu": ["newton.cu"] + ENGINE,
+    "pcg2.cu": ["pcg2.cu", "pcg2.hpp"],
+}
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-DNDEBUG", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC,-O2,-Wall,-Wno-unused-function"]
 

@@ -1,4 +1,4 @@
-// dense_kernels.cuh -- the spectral (dense) assembly path on the FP64 tensor cores.
+// dense_kernels.cuh -- the spectral (dense) assembly path on the FP64 tensor cores (compiled by evaluate.cu only).
 //
 // For spectral1d / spectral2d the "element" is the whole domain: the derivative operators are dense n x n Chebyshev
 // differentiation matrices (src/spectral1d.jl:63-109, src/spectral2d.jl:15-42) and R is a dense basis-evaluation
@@ -10,15 +10,10 @@
 //   (2) Wt[j][r]   = sum_c  Rt_b[j][c] Hd[r][c]          A = Rt_b (m_b x n),  B = Hd
 //   (3) A_top[i][j] = sum_r Rt_a[i][r] Wt[j][r]          A = Rt_a (m_a x n),  B = Wt, C = a block of the m x m system
 #pragma once
-#include "kernels.cuh"
+
+#include "device_common.cuh"
 
 namespace mgbx {
-
-constexpr int kGemmBM = 64, kGemmBN = 64, kGemmBK = 16, kGemmLd = kGemmBK + 4;
-
-__device__ __forceinline__ void dmma_m8n8k4(double &d0, double &d1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};" : "+d"(d0), "+d"(d1) : "d"(a), "d"(b));
-}
 
 // 128 threads = 4 warps in a 2 x 2 arrangement; each warp owns a 32 x 32 sub-tile = 4 x 4 DMMA tiles.
 __global__ void __launch_bounds__(128) k_dgemm_nt(int M, int N, int K, const double *__restrict__ A, int64_t lda, const double *__restrict__ B,
@@ -76,112 +71,6 @@ __global__ void __launch_bounds__(128) k_dgemm_nt(int M, int N, int K, const dou
     }
 }
 
-
-// ------------------------------------------------------------------------------------------------
-// Blocked dense Cholesky (row-major, lower) with panel width 64; the panel solve and the trailing update are
-// DMMA GEMMs (k_dgemm_nt):   L21 = A21 * inv(L11)'   and   A22 -= L21 * L21'.
-// ------------------------------------------------------------------------------------------------
-constexpr int kCholNB = 64;
-constexpr size_t kCholDiagSmem = sizeof(double) * 2 * kCholNB * (kCholNB + 1);
-
-// factor the nb x nb diagonal block at (k0, k0) in shared memory, write L11 back and inv(L11) (row-major, ld 64) to Linv
-__global__ void __launch_bounds__(1024) k_chol_diag_inv(double *A, int m, int k0, double *Linv) {
-  extern __shared__ double chol_sm[];   // 2 x 64 x 65 doubles (dynamic: above the 48 KB static limit)
-  double (*L)[kCholNB + 1] = reinterpret_cast<double (*)[kCholNB + 1]>(chol_sm);
-  double (*Li)[kCholNB + 1] = reinterpret_cast<double (*)[kCholNB + 1]>(chol_sm + kCholNB * (kCholNB + 1));
-  const int nb = min(kCholNB, m - k0);
-  const int tid = threadIdx.x, nt = blockDim.x;
-  for (int t = tid; t < kCholNB * kCholNB; t += nt) {
-    const int i = t / kCholNB, j = t % kCholNB;
-    L[i][j] = (i < nb && j <= i) ? A[(size_t)(k0 + i) * m + k0 + j] : 0.0;
-    Li[i][j] = 0.0;
-  }
-  __syncthreads();
-  for (int j = 0; j < nb; ++j) {
-    if (tid == 0) L[j][j] = sqrt(L[j][j]);
-    __syncthreads();
-    const double pv = L[j][j];
-    for (int i = j + 1 + tid; i < nb; i += nt) L[i][j] /= pv;
-    __syncthreads();
-    const int rem = nb - j - 1;
-    for (int t = tid; t < rem * rem; t += nt) {
-      const int i = j + 1 + t / rem, k = j + 1 + t % rem;
-      if (k <= i) L[i][k] -= L[i][j] * L[k][j];
-    }
-    __syncthreads();
-  }
-  // inverse of the triangular block, one warp per column
-  const int lane = tid & 31, wid = tid >> 5, nw = nt >> 5;
-  for (int c = wid; c < nb; c += nw) {
-    if (lane == 0) Li[c][c] = 1.0 / L[c][c];
-    __syncwarp();
-    for (int i = c + 1; i < nb; ++i) {
-      double sacc = 0.0;
-      for (int k = c + lane; k < i; k += 32) sacc += L[i][k] * Li[k][c];
-      sacc = warp_sum(sacc);
-      if (lane == 0) Li[i][c] = -sacc / L[i][i];
-      __syncwarp();
-    }
-  }
-  __syncthreads();
-  for (int t = tid; t < kCholNB * kCholNB; t += nt) {
-    const int i = t / kCholNB, j = t % kCholNB;
-    if (i < nb && j <= i) A[(size_t)(k0 + i) * m + k0 + j] = L[i][j];
-    Linv[t] = (i < nb && j < nb) ? Li[i][j] : 0.0;
-  }
-}
-
-// x = (L L')^{-1} (d .* b) .* d for ONE right-hand side with the blocked factor and the panel inverses (Linv: panels x 64 x 64).
-// One CTA walks the panels (the dependency is sequential anyway): y_blk = inv(L11) b_blk, then b_rest -= L21 y_blk; and back.
-__global__ void __launch_bounds__(1024) k_chol_solve_blocked(const double *__restrict__ A, int m, const double *__restrict__ Linv,
-                                                              const double *__restrict__ d, const double *__restrict__ b, double *x) {
-  extern __shared__ double v[];   // m
-  __shared__ double blk[kCholNB];
-  const int tid = threadIdx.x, nt = blockDim.x;
-  for (int i = tid; i < m; i += nt) v[i] = b[i] * d[i];
-  __syncthreads();
-  const int npan = (m + kCholNB - 1) / kCholNB;
-  for (int pnl = 0; pnl < npan; ++pnl) {
-    const int k0 = pnl * kCholNB, nb = min(kCholNB, m - k0);
-    const double *Li = Linv + (size_t)pnl * kCholNB * kCholNB;
-    if (tid < nb) {
-      double sacc = 0.0;
-      for (int j = 0; j <= tid; ++j) sacc += Li[tid * kCholNB + j] * v[k0 + j];
-      blk[tid] = sacc;
-    }
-    __syncthreads();
-    if (tid < nb) v[k0 + tid] = blk[tid];
-    for (int i = k0 + nb + tid; i < m; i += nt) {
-      const double *row = A + (size_t)i * m + k0;
-      double sacc = 0.0;
-      for (int j = 0; j < nb; ++j) sacc += row[j] * blk[j];
-      v[i] -= sacc;
-    }
-    __syncthreads();
-  }
-  for (int pnl = npan - 1; pnl >= 0; --pnl) {
-    const int k0 = pnl * kCholNB, nb = min(kCholNB, m - k0);
-    const double *Li = Linv + (size_t)pnl * kCholNB * kCholNB;
-    // y_blk[j] -= sum_{i >= k0+nb} L[i][k0+j] x[i]   (column sums: warp per j, lanes over rows)
-    const int lane = tid & 31, wid = tid >> 5, nw = nt >> 5;
-    for (int j = wid; j < nb; j += nw) {
-      double sacc = 0.0;
-      for (int i = k0 + nb + lane; i < m; i += 32) sacc += A[(size_t)i * m + k0 + j] * v[i];
-      sacc = warp_sum(sacc);
-      if (lane == 0) blk[j] = v[k0 + j] - sacc;
-    }
-    __syncthreads();
-    // x_blk = inv(L11)' y_blk
-    if (tid < nb) {
-      double sacc = 0.0;
-      for (int i = tid; i < nb; ++i) sacc += Li[i * kCholNB + tid] * blk[i];
-      v[k0 + tid] = sacc;
-    }
-    __syncthreads();
-  }
-  for (int i = tid; i < m; i += nt) x[i] = v[i] * d[i];
-}
-
 // Hd[r][c] += (ident_j ? delta : D_j[.][r]) ... the three cheap cases of D_j' diag(h) D_k with an identity operand:
 //   mode 0: both identities          Hd[r][r] += h[r]
 //   mode 1: D_j = I, D_k = Dk        Hd[r][c] += h[r] * Dk[r][c]        (Dk column-major: Dk[c*n + r])
@@ -198,35 +87,6 @@ __global__ void __launch_bounds__(256) k_dense_hess_ident(int n, int mode, const
   else Hd[t] += D[(int64_t)r * n + c] * h[c];
 }
 
-// Rt[j][i] = R[i][cols j] for the row block [r0, r0+n) and column block [c0, c0+mv) of a CSR matrix (dense transposed copy)
-__global__ void k_csr_block_to_dense_t(DevCsr R, int64_t r0, int n, int64_t c0, int mv, double *Rt) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  for (int64_t k = R.ptr[r0 + i]; k < R.ptr[r0 + i + 1]; ++k) {
-    const int64_t c = R.idx[k] - c0;
-    if (c >= 0 && c < mv) Rt[c * (int64_t)n + i] = R.val[k];
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Sum-factorised (Kronecker) assembly for tensor-product spectral discretisations (spectral2d).
-// There :dx = kron(DX, I), :dy = kron(I, DX), :id = kron(I, I) (src/spectral2d.jl:28-35) and every prolongation is
-// R = kron(R1, R1) (src/spectral2d.jl:22-25), so each D_j R_v = kron(P_j, Q_j) with n1 x c factors, and the block (a, b) of
-// R'HR = sum_{j in a, k in b} (P_j (x) Q_j)' diag(h_jk) (P_k (x) Q_k)   has the entries
-//     [(i, i'), (l, l')] = sum_e P_j[e, i] P_k[e, l] * ( sum_f Q_j[f, i'] h_jk[e, f] Q_k[f, l'] ).
-// Inner sum: k_kron_w (n1 small products per node row e);  outer sum over (pair, e): ONE DMMA GEMM per block with the
-// constant operand AA[(i, l)][c n1 + e] = P_j[e, i] P_k[e, l] (built once) -- 2 c1a c1b c2a c2b (pairs n1) flops instead of
-// the 2 n^3 per pair of the unstructured product (n = n1^2): 31 GFLOP instead of 1.6 TFLOP per assembly at n1 = 64.
-// ------------------------------------------------------------------------------------------------
-struct KronCombo {
-  const double *Qj, *Qk;   // n1 x c2a / n1 x c2b, row-major
-  const double *h;         // node samples h_jk (n = n1 * n1), node q = e * n1 + f
-};
-constexpr int kKronMaxCombos = 16;
-struct KronWArgs {
-  int n1, c2a, c2b, ncombo, K;   // K = ncombo * n1
-  KronCombo c[kKronMaxCombos];
-};
 // W[(i' c2b + l') K + c n1 + e] = sum_f Qj[f, i'] h[e n1 + f] Qk[f, l']     grid: (ncombo * n1) blocks
 __global__ void __launch_bounds__(256) k_kron_w(KronWArgs P, double *__restrict__ W) {
   extern __shared__ double kw_sm[];   // h row (n1), Qj scaled by h (n1 x c2a), Qk (n1 x c2b)
@@ -246,6 +106,7 @@ __global__ void __launch_bounds__(256) k_kron_w(KronWArgs P, double *__restrict_
     W[(size_t)o * P.K + (size_t)c * P.n1 + e] = acc;
   }
 }
+
 // Atop[(offa + i c2a + i') m + offb + l c2b + l'] = C[(i c1b + l) N + i' c2b + l'],  N = c2a c2b
 __global__ void __launch_bounds__(256) k_kron_scatter(int c1a, int c2a, int c1b, int c2b, const double *__restrict__ C, double *Atop, int64_t m,
                                                       int64_t offa, int64_t offb) {

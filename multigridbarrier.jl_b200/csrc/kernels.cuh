@@ -1,4 +1,4 @@
-// kernels.cuh -- sm_100a device kernels of the barrier-Newton hot path.
+// kernels.cuh -- sm_100a device kernels of barrier evaluation and Hessian assembly (compiled by evaluate.cu only).
 //
 // What each kernel replaces in the reference (paths under /root/reference):
 //   k_node            apply_D + map_rows_gpu(F0/F1/F2) + the (1/n)·y + w.*c combination
@@ -6,101 +6,22 @@
 //                     block_ops.jl:118-133 (_block_matvec_kernel!)
 //   k_blockgrad       sum_k D_k' y_k                    src/convex.jl:173-178; block_ops.jl:135-148
 //   k_blockhess       sum_{j,k} D_j' diag(y_jk) D_k     src/convex.jl:185-200; block_ops.jl:58-75 (called nD^2 times there)
-//   (solver_kernels.cuh: k_sell_gather = R'HR into the fixed pattern and the Galerkin products)
+//   k_sell_gather     R'HR into the fixed pattern and the numeric Galerkin products A_c = T'(A T) (north-star item 3),
+//                     src/BlockMatrices.jl:506-555, as fixed-order gathers over a sliced-ELL term list (coalesced
+//                     index/weight streams, deterministic; the reference CUDA ext uses FP64 atomics, block_ops.jl:229-249)
 //   k_spmv*           R*s, R'*g                          CUSPARSE in the reference (src/convex.jl:156,178)
-//   k_l1diag          smoother diagonals and the Gershgorin bound of every level of the solve kernel
+//   (solver_kernels.cuh: k_l1diag = smoother diagonals and the Gershgorin bound of every level of the solve kernel)
 //   (pcg2.cu: k_pcg2 = the multigrid-preconditioned CG solve, replacing cuDSS LDL' (ext/.../cudss_solver.jl:264-381))
-//   (dense_kernels.cuh: DMMA GEMM and blocked Cholesky of the spectral path)
+//   (dense_kernels.cuh: DMMA GEMM of the spectral path; solver_kernels.cuh: its blocked Cholesky)
 // All reductions are fixed-order (block tree + last-block pass): results are run-to-run deterministic.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include "node_barrier.cuh"
+
+#include "device_common.cuh"
 
 namespace mgbx {
-
-#define MGBX_MAX_OPS 8
-constexpr int kRedBlocks = 592;   // 148 SMs x 4
-constexpr int kRedThreads = 256;
-
-struct DevCsr {
-  int64_t rows = 0, cols = 0, nnz = 0;
-  int64_t *ptr = nullptr;
-  int32_t *idx = nullptr;
-  double *val = nullptr;
-};
-
-// ------------------------------------------------------------------------------------------------
-// reductions
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-  return v;
-}
-__device__ __forceinline__ double warp_max(double v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_down_sync(0xffffffffu, v, o));
-  return v;
-}
-
-// Block-reduce NV values (op[k] == 0: sum, 1: max); result valid in thread 0.
-template <int NV>
-__device__ __forceinline__ void block_reduce(double (&v)[NV], const int (&op)[NV]) {
-  __shared__ double sm[NV][32];
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = (blockDim.x + 31) >> 5;
-#pragma unroll
-  for (int k = 0; k < NV; ++k) {
-    v[k] = op[k] ? warp_max(v[k]) : warp_sum(v[k]);
-    if (lane == 0) sm[k][wid] = v[k];
-  }
-  __syncthreads();
-  if (wid == 0) {
-#pragma unroll
-    for (int k = 0; k < NV; ++k) {
-      double x = lane < nw ? sm[k][lane] : (op[k] ? -INFINITY : 0.0);
-      v[k] = op[k] ? warp_max(x) : warp_sum(x);
-    }
-  }
-  __syncthreads();
-}
-
-// Grid-wide fixed-order reduction: every block deposits its partials, the last block to arrive
-// (atomic ticket) combines them in block order and writes out[0..NV).
-template <int NV>
-__device__ __forceinline__ void grid_reduce(double (&v)[NV], const int (&op)[NV], double *partials,
-                                            unsigned int *ticket, double *out) {
-  block_reduce<NV>(v, op);
-  __shared__ bool last;
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int k = 0; k < NV; ++k) partials[(size_t)k * gridDim.x + blockIdx.x] = v[k];
-    __threadfence();
-    const unsigned int t = atomicAdd(ticket, 1u);
-    last = (t == gridDim.x - 1);
-  }
-  __syncthreads();
-  if (last) {
-    __threadfence();
-    double a[NV];
-#pragma unroll
-    for (int k = 0; k < NV; ++k) {
-      double acc = op[k] ? -INFINITY : 0.0;
-      for (unsigned int b = threadIdx.x; b < gridDim.x; b += blockDim.x) {
-        const double x = ((volatile double *)partials)[(size_t)k * gridDim.x + b];
-        acc = op[k] ? fmax(acc, x) : acc + x;
-      }
-      a[k] = acc;
-    }
-    block_reduce<NV>(a, op);
-    if (threadIdx.x == 0) {
-#pragma unroll
-      for (int k = 0; k < NV; ++k) out[k] = a[k];
-      *ticket = 0;
-    }
-  }
-}
 
 // ------------------------------------------------------------------------------------------------
 // sparse matrix-vector products.  G threads cooperate on one row (G = 1, 4, 32).
@@ -121,111 +42,6 @@ __global__ void __launch_bounds__(256) k_spmv(DevCsr A, const double *__restrict
     for (int o = G / 2; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o, G);
   }
   if (sub == 0) y[row] = alpha * acc + (y0 ? y0[row] : 0.0);
-}
-
-// dinv = 1 / sum_k |a_ik|  (l1-Jacobi), diag = 1 / a_ii, and the Gershgorin bound of lambda_max(D^-1 A),
-// max_i sum_k |a_ik| / a_ii, folded with atomicMax on the bit pattern (non-negative doubles order like integers;
-// max is order-independent, so the result is deterministic).  *lam_bits must be zeroed before the launch.
-__global__ void __launch_bounds__(256) k_l1diag(DevCsr A, double *dinv, double *diag, unsigned long long *lam_bits) {
-  const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  double ratio = 0.0;
-  if (row < A.rows) {
-    double s = 0.0, d = 0.0;
-    for (int64_t k = A.ptr[row]; k < A.ptr[row + 1]; ++k) {
-      s += fabs(A.val[k]);
-      if (A.idx[k] == row) d = A.val[k];
-    }
-    dinv[row] = s > 0.0 ? 1.0 / s : 0.0;
-    if (diag) diag[row] = d > 0.0 ? 1.0 / d : 0.0;   // inverse diagonal (Chebyshev scaling)
-    if (d > 0.0 && isfinite(s)) ratio = s / d;
-  }
-  if (lam_bits) {
-    ratio = warp_max(ratio);
-    if ((threadIdx.x & 31) == 0 && ratio > 0.0) atomicMax(lam_bits, (unsigned long long)__double_as_longlong(ratio));
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// per-node barrier kernel
-// ------------------------------------------------------------------------------------------------
-enum { NODE_F01 = 0, NODE_F2 = 1, NODE_SLACK = 2 };
-
-struct NodeParams {
-  int64_t n;
-  int p, nu, nD;
-  int D_var[MGBX_MAX_ND], D_op[MGBX_MAX_ND];
-  const double *ops[MGBX_MAX_OPS];   // each N x (p x p), offset e*p*p + col*p + row
-  const double *zf;                  // nu*n broken state  z0 + R s
-  const double *w, *f, *bw;          // weights, cost grid n x nD, barrier weights or nullptr
-  double t, inv_n;
-  ConvexDev cd;
-  // F01 outputs
-  double *G;                         // n x nD: bw*F1 + w*t*f
-  double *partials;                  // 4 x gridDim
-  unsigned int *ticket;
-  double *red_out;                   // [0] sum bw*F0 (or sum F0), [1] sum w*(c.Dz), [2] #non-finite F0, [3] max slack
-  // F2 outputs (condensed when nE > 0)
-  int nK, nE;
-  int Krow[MGBX_MAX_ND];             // D rows of the kept variables
-  int Erow[MGBX_MAX_ND];             // per D row: index of its eliminated variable, or -1
-  double *Hn;                        // n x nK(nK+1)/2, packed (a<=b): a*nK - a(a-1)/2 + (b-a)
-  double *hEEinv;                    // n x nE(nE+1)/2
-  double *hKE;                       // n x (nK*nE): entry (a, ev) at column a*nE + ev
-  unsigned schur_pieces, schur_elim; // pieces condensed analytically by node_eval / the eliminated variables they cover (bit masks)
-  // SLACK output
-  double *slack;                     // n
-};
-
-// the analytic condensation only applies when something is eliminated
-__device__ __forceinline__ unsigned nE_mask_guard(const NodeParams &P) { return P.nE > 0 ? P.schur_pieces : 0u; }
-
-__device__ __forceinline__ void node_Dz(const NodeParams &P, int64_t i, double *y) {
-  const int64_t e = i / P.p;
-  const int r = (int)(i - e * P.p);
-  for (int j = 0; j < P.nD; ++j) {
-    const int v = P.D_var[j], o = P.D_op[j];
-    const double *zv = P.zf + (int64_t)v * P.n;
-    if (o < 0) {
-      y[j] = zv[i];
-    } else {
-      const double *blk = P.ops[o] + e * (int64_t)(P.p * P.p) + r;
-      const double *ze = zv + e * P.p;
-      double acc = 0.0;
-      for (int c = 0; c < P.p; ++c) acc += blk[(int64_t)c * P.p] * ze[c];
-      y[j] = acc;
-    }
-  }
-}
-
-// small symmetric positive definite inverse (nE <= 4) by Cholesky; packed lower-by-rows in/out is
-// avoided: we work on a full nE x nE array.
-__device__ __forceinline__ void spd_inverse(double *M, int m) {
-  // in-place Cholesky M = L L'
-  double L[16];
-  for (int i = 0; i < m; ++i)
-    for (int j = 0; j <= i; ++j) {
-      double s = M[i * m + j];
-      for (int k = 0; k < j; ++k) s -= L[i * m + k] * L[j * m + k];
-      L[i * m + j] = (i == j) ? sqrt(s) : s / L[j * m + j];
-    }
-  // Linv
-  double Li[16];
-  for (int i = 0; i < m; ++i)
-    for (int j = 0; j < m; ++j) Li[i * m + j] = 0.0;
-  for (int j = 0; j < m; ++j) {
-    Li[j * m + j] = 1.0 / L[j * m + j];
-    for (int i = j + 1; i < m; ++i) {
-      double s = 0.0;
-      for (int k = j; k < i; ++k) s -= L[i * m + k] * Li[k * m + j];
-      Li[i * m + j] = s / L[i * m + i];
-    }
-  }
-  for (int i = 0; i < m; ++i)
-    for (int j = 0; j < m; ++j) {
-      double s = 0.0;
-      for (int k = (i > j ? i : j); k < m; ++k) s += Li[k * m + i] * Li[k * m + j];
-      M[i * m + j] = s;
-    }
 }
 
 // NDT >= nD bounds the per-thread arrays (y, F1, F2 = NDT^2 doubles) so that they stay in registers / L1
@@ -315,18 +131,6 @@ __global__ void __launch_bounds__(kRedThreads) k_node(NodeParams P) {
   if (MODE != NODE_F2) grid_reduce<4>(red, op, P.partials, P.ticket, P.red_out);
 }
 
-// ------------------------------------------------------------------------------------------------
-// element-block kernels
-// ------------------------------------------------------------------------------------------------
-struct ElemParams {
-  int64_t n, N;
-  int p, nD;
-  int D_var[MGBX_MAX_ND], D_op[MGBX_MAX_ND];
-  const double *ops[MGBX_MAX_OPS];
-  int nK;                    // rows used (Hessian: kept rows; gradient: all rows)
-  int Krow[MGBX_MAX_ND];
-};
-
 // gb[v*n + e*p + c] = sum_{j in rows(v), j in Krow} sum_q D_j[q][c] * G[j*n + e*p + q]
 // one thread per (variable slot, broken node)
 __global__ void __launch_bounds__(256) k_blockgrad(ElemParams P, const double *__restrict__ G, double *gb, int nu) {
@@ -352,12 +156,6 @@ __global__ void __launch_bounds__(256) k_blockgrad(ElemParams P, const double *_
   gb[tid] = acc;
 }
 
-// Hblk[((pair*N + e)*p + r)*p + c] = sum_{j in rows(a), k in rows(b)} sum_q D_j[q][r] h_jk[q] D_k[q][c]
-// with h packed over the kept rows.  One thread per (pair, e, r, c).
-struct PairList {
-  int npairs;
-  int va[16], vb[16];
-};
 __global__ void __launch_bounds__(256) k_blockhess(ElemParams P, PairList PL, const double *__restrict__ Hn, double *Hblk) {
   const int pp = P.p * P.p;
   const int64_t total = (int64_t)PL.npairs * P.N * pp;
@@ -400,70 +198,6 @@ __global__ void __launch_bounds__(256) k_blockhess(ElemParams P, PairList PL, co
 }
 
 // ------------------------------------------------------------------------------------------------
-// condensation helpers (node-local elimination of the :full variables)
-// ------------------------------------------------------------------------------------------------
-struct CondParams {
-  int64_t n;
-  int nD, nK, nE;
-  int Krow[MGBX_MAX_ND];
-  int64_t Eoff[4];            // first index of eliminated variable ev in the level-L vector
-  const double *hEEinv, *hKE;
-};
-
-// Gt[Krow[a]*n + i] = - sum_ev hKE[a][ev] * (hEEinv * gE)[ev],  gE[ev] = g[Eoff[ev] + i]; other rows of Gt are not touched
-__global__ void __launch_bounds__(256) k_condense_rhs(CondParams P, const double *__restrict__ g, double *Gt) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= P.n) return;
-  double gE[4], tE[4], Hi[16];
-  const int nE = P.nE;
-  for (int ev = 0; ev < nE; ++ev) gE[ev] = g[P.Eoff[ev] + i];
-  int q = 0;
-  for (int a = 0; a < nE; ++a)
-    for (int b = a; b < nE; ++b, ++q) {
-      const double v = P.hEEinv[i + (int64_t)q * P.n];
-      Hi[a * nE + b] = v;
-      Hi[b * nE + a] = v;
-    }
-  for (int ev = 0; ev < nE; ++ev) {
-    double s = 0.0;
-    for (int ew = 0; ew < nE; ++ew) s += Hi[ev * nE + ew] * gE[ew];
-    tE[ev] = s;
-  }
-  for (int a = 0; a < P.nK; ++a) {
-    double s = 0.0;
-    for (int ev = 0; ev < nE; ++ev) s += P.hKE[i + (int64_t)(a * nE + ev) * P.n] * tE[ev];
-    Gt[i + (int64_t)P.Krow[a] * P.n] = -s;
-  }
-}
-
-// xE = hEEinv (gE - hEK * DnK):  x[Eoff[ev] + i]; DnK = rows Krow of D applied to the broken vector nb
-__global__ void __launch_bounds__(256) k_backsubst(CondParams P, NodeParams NP, const double *__restrict__ g, double *x) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= P.n) return;
-  double y[MGBX_MAX_ND];
-  node_Dz(NP, i, y);   // NP.zf = broken image of the kept part of the direction
-  const int nE = P.nE;
-  double rE[4], Hi[16];
-  for (int ev = 0; ev < nE; ++ev) {
-    double s = g[P.Eoff[ev] + i];
-    for (int a = 0; a < P.nK; ++a) s -= P.hKE[i + (int64_t)(a * nE + ev) * P.n] * y[P.Krow[a]];
-    rE[ev] = s;
-  }
-  int q = 0;
-  for (int a = 0; a < nE; ++a)
-    for (int b = a; b < nE; ++b, ++q) {
-      const double v = P.hEEinv[i + (int64_t)q * P.n];
-      Hi[a * nE + b] = v;
-      Hi[b * nE + a] = v;
-    }
-  for (int ev = 0; ev < nE; ++ev) {
-    double s = 0.0;
-    for (int ew = 0; ew < nE; ++ew) s += Hi[ev * nE + ew] * rE[ew];
-    x[P.Eoff[ev] + i] = s;
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
 // vector kernels (all scalars stay on the device)
 // ------------------------------------------------------------------------------------------------
 // out[0] = a.b, out[1] = a.a, out[2] = #non-finite entries of a
@@ -500,13 +234,6 @@ __global__ void k_axpby(int64_t m, double a, const double *__restrict__ x, doubl
   if (i < m) out[i] = a * x[i] + (y ? b * y[i] : 0.0);
 }
 
-// start vector of the power iteration on D^-1 A (pcg2_lambda_power: a sharper lambda_max for the Chebyshev interval than the
-// Gershgorin bound): smooth + oscillatory parts, never orthogonal to the top eigenvector in practice
-__global__ void k_pw_init(int64_t m, double *v) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < m) v[i] = 1.0 + 0.5 * cos(0.7 * (double)i) + ((i & 1) ? 0.25 : -0.25);
-}
-
 // per-variable max and max|.| of the state: out[2k] = max, out[2k+1] = absmax  (one launch per variable)
 __global__ void __launch_bounds__(kRedThreads) k_maxabs(int64_t m, const double *__restrict__ a, double *partials, unsigned int *ticket,
                                                          double *out) {
@@ -525,55 +252,6 @@ __global__ void __launch_bounds__(kRedThreads) k_maxabs(int64_t m, const double 
 __global__ void k_phase1_slack(int64_t n, const double *slack, double *out) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = 2.0 * fmax(slack[i], 1.0);
-}
-
-// ------------------------------------------------------------------------------------------------
-// dense helpers (the blocked DMMA Cholesky lives in dense_kernels.cuh)
-// ------------------------------------------------------------------------------------------------
-// Ad = 0 then Ad[i][j] = a_ij * d_i * d_j  with d = 1/sqrt(a_ii)
-__global__ void k_dense_scale_diag(DevCsr A, double *d) {
-  const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (row >= A.rows) return;
-  double dg = 0.0;
-  for (int64_t k = A.ptr[row]; k < A.ptr[row + 1]; ++k)
-    if (A.idx[k] == row) dg = A.val[k];
-  d[row] = dg > 0.0 ? 1.0 / sqrt(dg) : 1.0;
-}
-__global__ void k_csr_to_dense(DevCsr A, const double *d, double *Ad) {
-  const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (row >= A.rows) return;
-  const double di = d[row];
-  for (int64_t k = A.ptr[row]; k < A.ptr[row + 1]; ++k) Ad[row * A.rows + A.idx[k]] = A.val[k] * di * d[A.idx[k]];
-}
-
-// y = M x for a dense symmetric m x m matrix stored as m columns (coarse inverse); one warp per row
-__global__ void __launch_bounds__(256) k_dense_symv(const double *__restrict__ M, int m, const double *__restrict__ x, double *y) {
-  const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int lane = threadIdx.x & 31;
-  if (row >= m) return;
-  const double *r = M + (size_t)row * m;
-  double s = 0.0;
-  for (int j = lane; j < m; j += 32) s += r[j] * x[j];
-  s = warp_sum(s);
-  if (lane == 0) y[row] = s;
-}
-
-
-// ------------------------------------------------------------------------------------------------
-// multi-GPU (element partition): a level vector is a list of segments, one per state variable; `shared`
-// segments are replicated on every rank, `local` segments hold the rank's own node-local unknowns.  Reductions
-// over such vectors are split: the shared part is summed redundantly (identically) on every rank, the local
-// part is a partial sum completed by an all-reduce.
-// ------------------------------------------------------------------------------------------------
-struct SegList {
-  int n;
-  int64_t off[MGBX_MAX_ND + 1];   // segment q = [off[q], off[q+1])
-  int local[MGBX_MAX_ND];
-};
-__device__ __forceinline__ int seg_is_local(const SegList &S, int64_t i) {
-  int q = 0;
-  while (q + 1 < S.n && i >= S.off[q + 1]) ++q;
-  return S.local[q];
 }
 
 // out[0..2] = {a.b, a.a, #non-finite entries of a} over the LOCAL segments, out[3..5] the same over the SHARED ones
@@ -604,33 +282,6 @@ __global__ void __launch_bounds__(kRedThreads) k_trial_seg(SegList S, int64_t m,
     red[seg_is_local(S, i) ? 1 : 0] += df * df;
   }
   grid_reduce<2>(red, op, partials, ticket, out);
-}
-
-// ------------------------------------------------------------------------------------------------
-// Fused element kernels (north-star items 1 + 2): one pass per barrier evaluation.
-//   k_elem<NODE_F01>  apply_D -> F0/F1 -> (1/n) F1 + w.*c -> sum_k D_k' y_k      (k_node<F01> + k_blockgrad in one kernel)
-//   k_elem<NODE_F2>   apply_D -> F2 -> node-local Schur condensation -> sum_jk D_j' diag(h_jk) D_k   (k_node<F2> + k_blockhess)
-// A block owns `epb` whole elements per tile (one thread per broken node) and walks tiles grid-stride.  The
-// operator blocks of the tile are staged ONCE in shared memory (padded against bank conflicts) and serve both
-// the forward application D z and the adjoint / triple product; the per-node samples (G or the packed Hessian)
-// are exchanged through shared memory and never touch HBM.  Replaces, per evaluation, nD block matvecs +
-// map_rows + nD adjoint matvecs (src/convex.jl:155-179) resp. nD^2 block_fused_triple! calls each allocating
-// p x p x N (src/convex.jl:185-200, src/BlockMatrices.jl:170-212).
-// ------------------------------------------------------------------------------------------------
-struct ElemFused {
-  NodeParams np;
-  PairList pl;
-  double *Hblk;     // F2: pairs x N x p x p
-  double *gb;       // F01: nu x n
-  int64_t N;
-  int epb;          // elements per tile
-  int p1, ES;       // padded column stride and element stride of the staged operator blocks (doubles)
-  int nex;          // exchange rows
-  int nops;
-};
-
-inline size_t elem_fused_smem(int nops, int epb, int ES, int nu, int nex, int p) {
-  return sizeof(double) * ((size_t)nops * epb * ES + (size_t)(nu + nex) * epb * p);
 }
 
 template <int MODE, int NDT>
@@ -811,96 +462,6 @@ __global__ void __launch_bounds__(256) k_elem(ElemFused Q) {
   }
   if (MODE == NODE_F01) grid_reduce<4>(red, op4, P.partials, P.ticket, P.red_out);
 }
-
-}  // namespace mgbx
-
-namespace mgbx {
-
-// ------------------------------------------------------------------------------------------------
-// k_elem_plap<MODE, DIM>: the fused element kernel specialised for the reference's default problem family
-// (src/mgb.jl:587-613,711-727): state (u, s), D = [u:id; u:d_1..d_DIM; s:id], one Euclidean-power cone on rows
-// 1..DIM+1 with identity A, zero b and uniform p, mu; s condensed node-locally.  Same shared-memory staging and
-// the same outputs (gb; hEEinv, hKE, Hblk) as the generic k_elem, but every loop over D rows / pieces / index maps
-// is resolved at compile time: the generic kernel is instruction-bound (~1700 warp instructions per warp of nodes,
-// 90% of them index bookkeeping), this one is bound by the operator-block stream.
-// ------------------------------------------------------------------------------------------------
-struct FastDiv {
-  unsigned int mul, d;   // q = umulhi(t, mul) for 0 <= t < 2^16, 1 <= d < 2^16
-};
-inline FastDiv make_fastdiv(unsigned int d) {
-  FastDiv f;
-  f.d = d;
-  f.mul = (unsigned int)((0x100000000ull + d - 1) / d);
-  return f;
-}
-__device__ __forceinline__ unsigned int fdiv(unsigned int t, const FastDiv &f) { return f.d == 1 ? t : __umulhi(t, f.mul); }
-
-struct PlapParams {
-  int64_t n, N;
-  int p, epb, p1, ES;
-  int bulk;                    // 0: per-double cp.async staging; 1: one bulk copy per operator slab (p1 == p, ES == p*p);
-                               // 2: one bulk copy per block column (p even, p1 and ES even).  Ragged tiles use the per-double path.
-  FastDiv dp, dpp;
-  const double *ops[3];
-  const double *zu, *zs;       // broken state of u and s (n each)
-  const double *w, *f, *bw;    // f: n x (DIM+2)
-  double t, inv_n, pexp, mu;
-  // F01
-  double *gbu, *gbs;
-  double *partials;
-  unsigned int *ticket;
-  double *red_out;
-  // F2
-  double *hEEinv, *hKE, *Hblk;
-};
-
-// shared memory: two input buffers (operator blocks + the tile's node inputs, filled by cp.async one tile ahead) + exchange rows
-inline size_t elem_plap_smem(int dim, int epb, int ES, int p, bool condensed = true) {
-  const size_t tm = (size_t)epb * p;
-  const size_t buf = (size_t)dim * epb * ES + (size_t)(4 + dim + 2) * tm;
-  const int nh = (dim * (dim + 1)) / 2;
-  const int nex = condensed ? (nh > dim ? nh : dim) : nh + dim + 1;
-  return sizeof(double) * (2 * buf + (size_t)nex * tm);
-}
-
-__device__ __forceinline__ void cp_async8(void *smem, const void *gmem) {
-  const unsigned int sa = (unsigned int)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(sa), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
-
-// ---- bulk asynchronous copies (cp.async.bulk, the 1-D form of TMA: SASS UBLKCP) completing on an mbarrier -------------------
-__device__ __forceinline__ void mbar_init(unsigned long long *bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((unsigned int)__cvta_generic_to_shared(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long *bar, unsigned int bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"((unsigned int)__cvta_generic_to_shared(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long *bar, unsigned int parity) {
-  const unsigned int a = (unsigned int)__cvta_generic_to_shared(bar);
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_%=:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra DONE_%=;\n"
-      "bra WAIT_%=;\n"
-      "DONE_%=:\n"
-      "}\n" ::"r"(a),
-      "r"(parity)
-      : "memory");
-}
-// bytes: multiple of 16; smem and gmem 16-byte aligned
-__device__ __forceinline__ void bulk_g2s(void *smem, const void *gmem, unsigned int bytes, unsigned long long *bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"((unsigned int)__cvta_generic_to_shared(smem)),
-               "l"(gmem), "r"(bytes), "r"((unsigned int)__cvta_generic_to_shared(bar))
-               : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // Tiles are software-pipelined: while tile k is evaluated, the operator blocks and node inputs of tile k+1 stream into the
 // other shared-memory buffer with cp.async (LDGSTS), so the evaluation never waits on HBM latency after the first tile.
@@ -1175,6 +736,20 @@ __global__ void __launch_bounds__(256, 3) k_elem_plap(PlapParams P) {
     b ^= 1;
   }
   if (MODE == NODE_F01) grid_reduce<4>(red, op4, P.partials, P.ticket, P.red_out);
+}
+
+__global__ void __launch_bounds__(256) k_sell_gather(SellPlan P, const double *__restrict__ in, double *__restrict__ out) {
+  const int64_t nz = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (nz >= P.nout) return;
+  const int64_t off = P.sptr[nz >> 5] + (nz & 31);
+  const int c = P.cnt[nz];
+  double acc = 0.0;
+  if (P.w) {
+    for (int k = 0; k < c; ++k) acc += P.w[off + 32 * (int64_t)k] * in[P.src[off + 32 * (int64_t)k]];
+  } else {
+    for (int k = 0; k < c; ++k) acc += in[P.src[off + 32 * (int64_t)k]];
+  }
+  out[nz] = acc;
 }
 
 }  // namespace mgbx

@@ -5,11 +5,13 @@
 //                        symbolic half of the Galerkin products A T and T'(A T)
 //   k_top_plan           term list of the element-block -> CSR gather (the scatter_idx of
 //                        src/BlockMatrices.jl:448-491, inverted into a fixed-order gather)
-// CUB (radix sort / scan / unique) is used for the sort; everything else is hand-written.
+//   k_prod_plan<0|1>     term lists of the Galerkin gathers (k_sell_gather)
+//   k_csr_block_to_dense_t  dense prolongation blocks of the spectral path
+// CUB (radix sort / scan / unique) is used for the sort; everything else is hand-written.  Compiled by setup.cu only.
 #pragma once
 #include <cub/cub.cuh>
 
-#include "solver_kernels.cuh"
+#include "device_common.cuh"
 
 namespace mgbx {
 
@@ -55,24 +57,6 @@ __global__ void k_sym_finish(const unsigned long long *__restrict__ uniq, int64_
   }
 }
 
-// Element-block -> CSR gather plan.  One thread per non-zero (i, j) of the top pattern: the pair of state
-// variables is fixed by the variable blocks i and j live in; the elements incident to i come from the
-// transposed element incidence; inside an element the rows r (resp. c) whose R row carries column i (resp. j)
-// are found by binary search.  Terms are emitted in the order (element, r, c): fixed, so the gather is
-// deterministic.  FILL == 0 counts (cnt, slice widths), FILL == 1 writes src / w.
-struct TopPlanParams {
-  DevCsr R;                    // level->broken prolongation of the system's top level (rows nu*n)
-  DevCsr EincT;                // system unknown -> incident elements (sorted)
-  DevCsr pat;                  // top pattern
-  const int32_t *rowof;        // row of every non-zero of pat
-  int64_t n, N;
-  int p, nkept, unit;
-  int kept[MGBX_MAX_ND];       // state variable of kept slot q
-  int64_t off[MGBX_MAX_ND + 1];    // system offsets of the kept slots
-  int64_t rcol0[MGBX_MAX_ND];      // first R column of the kept slot's variable
-  int pair_of[MGBX_MAX_ND * MGBX_MAX_ND];   // [qa * nkept + qb] -> pair index or -1
-};
-
 template <int FILL>
 __global__ void __launch_bounds__(256) k_top_plan(TopPlanParams Q, SellPlan P, int32_t *width) {
   const int64_t nz = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -112,6 +96,55 @@ __global__ void __launch_bounds__(256) k_top_plan(TopPlanParams Q, SellPlan P, i
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) wmax = max(wmax, __shfl_xor_sync(0xffffffffu, wmax, o));
     if ((threadIdx.x & 31) == 0 && nz < Q.pat.nnz) width[nz >> 5] = wmax;
+  }
+}
+
+// row index of every non-zero of a CSR pattern
+__global__ void k_csr_rows(DevCsr A, int32_t *rowof) {
+  const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (row >= A.rows) return;
+  for (int64_t k = A.ptr[row]; k < A.ptr[row + 1]; ++k) rowof[k] = (int32_t)row;
+}
+
+// Term list of C = Lm * Rm into the fixed pattern C.  variable_left: the values of Lm change between
+// uses (source = nz of Lm, weight = value of Rm), otherwise the values of Rm change.  One thread per
+// non-zero of C walks row i of Lm and looks column c up in the rows of Rm: no atomics, fixed order.
+// FILL == 0: cnt[nz] and per-slice width;  FILL == 1: write src / w.
+template <int FILL>
+__global__ void __launch_bounds__(256) k_prod_plan(DevCsr Lm, DevCsr Rm, DevCsr C, const int32_t *__restrict__ rowof, int variable_left,
+                                                    SellPlan P, int32_t *width) {
+  const int64_t nz = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  int count = 0;
+  if (nz < C.nnz) {
+    const int64_t i = rowof[nz];
+    const int32_t c = C.idx[nz];
+    const int64_t off = FILL ? P.sptr[nz >> 5] + (nz & 31) : 0;
+    for (int64_t a = Lm.ptr[i]; a < Lm.ptr[i + 1]; ++a) {
+      const int64_t b = csr_find(Rm, Lm.idx[a], c);
+      if (b < 0) continue;
+      if (FILL) {
+        P.src[off + 32 * (int64_t)count] = (int32_t)(variable_left ? a : b);
+        P.w[off + 32 * (int64_t)count] = variable_left ? Rm.val[b] : Lm.val[a];
+      }
+      ++count;
+    }
+    if (!FILL) P.cnt[nz] = count;
+  }
+  if (!FILL) {
+    int wmax = count;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) wmax = max(wmax, __shfl_xor_sync(0xffffffffu, wmax, o));
+    if ((threadIdx.x & 31) == 0 && nz < C.nnz) width[nz >> 5] = wmax;
+  }
+}
+
+// Rt[j][i] = R[i][cols j] for the row block [r0, r0+n) and column block [c0, c0+mv) of a CSR matrix (dense transposed copy)
+__global__ void k_csr_block_to_dense_t(DevCsr R, int64_t r0, int n, int64_t c0, int mv, double *Rt) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  for (int64_t k = R.ptr[r0 + i]; k < R.ptr[r0 + i + 1]; ++k) {
+    const int64_t c = R.idx[k] - c0;
+    if (c >= 0 && c < mv) Rt[c * (int64_t)n + i] = R.val[k];
   }
 }
 

@@ -1,107 +1,137 @@
-// solver_kernels.cuh -- the Galerkin gather plans (sliced-ELL), the coarse dense inverse and the small direct solve.
+// solver_kernels.cuh -- kernels of the linear solve around k_pcg2 (compiled by linear_solve.cu only): smoother
+// diagonals, FP32 copies and the power-iteration start of the preconditioner levels, the node-local condensation of the
+// right-hand side and its back-substitution, the coarse dense inverse, and the direct solves.
 // The Newton-system solve itself is k_pcg2 (pcg2.hpp / pcg2.cu).
 //
 // What this replaces in the reference (paths under /root/reference):
-//   k_sell_gather        the numeric Galerkin products A_c = T'(A T) (north-star item 3) and the R'HR scatter
-//                        of src/BlockMatrices.jl:506-555, as fixed-order gathers over a sliced-ELL term list
-//                        (coalesced index/weight streams, deterministic; the reference CUDA ext uses FP64 atomics,
-//                        block_ops.jl:229-249).
-//   k_prod_plan<0|1>     build those term lists on the device (setup, once per system).
 //   k_coarse_inverse     dense Cholesky + explicit inverse of the coarsest level in shared memory (one CTA).
 //   k_dense_solve_small  solve(Symmetric(H), g) (src/utils.jl:142-145) of a small system in one CTA.
+//   k_chol_*             the same for up to 8192 unknowns: blocked Cholesky (panel width 64, the panel solve and the
+//                        trailing update are k_dgemm_nt DMMA GEMMs) and the triangular solves.
 #pragma once
-#include "kernels.cuh"
+
+#include "device_common.cuh"
 
 namespace mgbx {
 
-// ------------------------------------------------------------------------------------------------
-// sliced-ELL gather:  out[nz] = sum_{k < cnt[nz]} w[off + 32k] * in[src[off + 32k]],  off = sptr[nz/32] + nz%32
-// ------------------------------------------------------------------------------------------------
-struct SellPlan {
-  int64_t nout = 0, nslices = 0, nterms = 0;   // nterms: real (unpadded) terms
-  int64_t *sptr = nullptr;                      // nslices + 1 entry offsets
-  int32_t *cnt = nullptr;                       // nout
-  int32_t *src = nullptr;                       // padded entries
-  double *w = nullptr;                          // padded entries, or nullptr (all weights 1)
-};
-
-__global__ void __launch_bounds__(256) k_sell_gather(SellPlan P, const double *__restrict__ in, double *__restrict__ out) {
-  const int64_t nz = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (nz >= P.nout) return;
-  const int64_t off = P.sptr[nz >> 5] + (nz & 31);
-  const int c = P.cnt[nz];
-  double acc = 0.0;
-  if (P.w) {
-    for (int k = 0; k < c; ++k) acc += P.w[off + 32 * (int64_t)k] * in[P.src[off + 32 * (int64_t)k]];
-  } else {
-    for (int k = 0; k < c; ++k) acc += in[P.src[off + 32 * (int64_t)k]];
+// Gt[Krow[a]*n + i] = - sum_ev hKE[a][ev] * (hEEinv * gE)[ev],  gE[ev] = g[Eoff[ev] + i]; other rows of Gt are not touched
+__global__ void __launch_bounds__(256) k_condense_rhs(CondParams P, const double *__restrict__ g, double *Gt) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.n) return;
+  double gE[4], tE[4], Hi[16];
+  const int nE = P.nE;
+  for (int ev = 0; ev < nE; ++ev) gE[ev] = g[P.Eoff[ev] + i];
+  int q = 0;
+  for (int a = 0; a < nE; ++a)
+    for (int b = a; b < nE; ++b, ++q) {
+      const double v = P.hEEinv[i + (int64_t)q * P.n];
+      Hi[a * nE + b] = v;
+      Hi[b * nE + a] = v;
+    }
+  for (int ev = 0; ev < nE; ++ev) {
+    double s = 0.0;
+    for (int ew = 0; ew < nE; ++ew) s += Hi[ev * nE + ew] * gE[ew];
+    tE[ev] = s;
   }
-  out[nz] = acc;
+  for (int a = 0; a < P.nK; ++a) {
+    double s = 0.0;
+    for (int ev = 0; ev < nE; ++ev) s += P.hKE[i + (int64_t)(a * nE + ev) * P.n] * tE[ev];
+    Gt[i + (int64_t)P.Krow[a] * P.n] = -s;
+  }
+}
+
+// xE = hEEinv (gE - hEK * DnK):  x[Eoff[ev] + i]; DnK = rows Krow of D applied to the broken vector nb
+__global__ void __launch_bounds__(256) k_backsubst(CondParams P, NodeParams NP, const double *__restrict__ g, double *x) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P.n) return;
+  double y[MGBX_MAX_ND];
+  node_Dz(NP, i, y);   // NP.zf = broken image of the kept part of the direction
+  const int nE = P.nE;
+  double rE[4], Hi[16];
+  for (int ev = 0; ev < nE; ++ev) {
+    double s = g[P.Eoff[ev] + i];
+    for (int a = 0; a < P.nK; ++a) s -= P.hKE[i + (int64_t)(a * nE + ev) * P.n] * y[P.Krow[a]];
+    rE[ev] = s;
+  }
+  int q = 0;
+  for (int a = 0; a < nE; ++a)
+    for (int b = a; b < nE; ++b, ++q) {
+      const double v = P.hEEinv[i + (int64_t)q * P.n];
+      Hi[a * nE + b] = v;
+      Hi[b * nE + a] = v;
+    }
+  for (int ev = 0; ev < nE; ++ev) {
+    double s = 0.0;
+    for (int ew = 0; ew < nE; ++ew) s += Hi[ev * nE + ew] * rE[ew];
+    x[P.Eoff[ev] + i] = s;
+  }
+}
+
+// start vector of the power iteration on D^-1 A (pcg2_lambda_power: a sharper lambda_max for the Chebyshev interval than the
+// Gershgorin bound): smooth + oscillatory parts, never orthogonal to the top eigenvector in practice
+__global__ void k_pw_init(int64_t m, double *v) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < m) v[i] = 1.0 + 0.5 * cos(0.7 * (double)i) + ((i & 1) ? 0.25 : -0.25);
+}
+
+// dinv = 1 / sum_k |a_ik|  (l1-Jacobi), diag = 1 / a_ii, and the Gershgorin bound of lambda_max(D^-1 A),
+// max_i sum_k |a_ik| / a_ii, folded with atomicMax on the bit pattern (non-negative doubles order like integers;
+// max is order-independent, so the result is deterministic).  *lam_bits must be zeroed before the launch.
+__global__ void __launch_bounds__(256) k_l1diag(DevCsr A, double *dinv, double *diag, unsigned long long *lam_bits) {
+  const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  double ratio = 0.0;
+  if (row < A.rows) {
+    double s = 0.0, d = 0.0;
+    for (int64_t k = A.ptr[row]; k < A.ptr[row + 1]; ++k) {
+      s += fabs(A.val[k]);
+      if (A.idx[k] == row) d = A.val[k];
+    }
+    dinv[row] = s > 0.0 ? 1.0 / s : 0.0;
+    if (diag) diag[row] = d > 0.0 ? 1.0 / d : 0.0;   // inverse diagonal (Chebyshev scaling)
+    if (d > 0.0 && isfinite(s)) ratio = s / d;
+  }
+  if (lam_bits) {
+    ratio = warp_max(ratio);
+    if ((threadIdx.x & 31) == 0 && ratio > 0.0) atomicMax(lam_bits, (unsigned long long)__double_as_longlong(ratio));
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// dense helpers (the blocked DMMA Cholesky lives in dense_kernels.cuh)
+// ------------------------------------------------------------------------------------------------
+// Ad = 0 then Ad[i][j] = a_ij * d_i * d_j  with d = 1/sqrt(a_ii)
+__global__ void k_dense_scale_diag(DevCsr A, double *d) {
+  const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (row >= A.rows) return;
+  double dg = 0.0;
+  for (int64_t k = A.ptr[row]; k < A.ptr[row + 1]; ++k)
+    if (A.idx[k] == row) dg = A.val[k];
+  d[row] = dg > 0.0 ? 1.0 / sqrt(dg) : 1.0;
+}
+
+__global__ void k_csr_to_dense(DevCsr A, const double *d, double *Ad) {
+  const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (row >= A.rows) return;
+  const double di = d[row];
+  for (int64_t k = A.ptr[row]; k < A.ptr[row + 1]; ++k) Ad[row * A.rows + A.idx[k]] = A.val[k] * di * d[A.idx[k]];
+}
+
+// y = M x for a dense symmetric m x m matrix stored as m columns (coarse inverse); one warp per row
+__global__ void __launch_bounds__(256) k_dense_symv(const double *__restrict__ M, int m, const double *__restrict__ x, double *y) {
+  const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (row >= m) return;
+  const double *r = M + (size_t)row * m;
+  double s = 0.0;
+  for (int j = lane; j < m; j += 32) s += r[j] * x[j];
+  s = warp_sum(s);
+  if (lane == 0) y[row] = s;
 }
 
 __global__ void k_f64_to_f32(int64_t n, const double *__restrict__ a, float *__restrict__ out) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = (float)a[i];
 }
-
-// row index of every non-zero of a CSR pattern
-__global__ void k_csr_rows(DevCsr A, int32_t *rowof) {
-  const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (row >= A.rows) return;
-  for (int64_t k = A.ptr[row]; k < A.ptr[row + 1]; ++k) rowof[k] = (int32_t)row;
-}
-
-__device__ __forceinline__ int64_t csr_find(const DevCsr &A, int64_t row, int32_t col) {
-  int64_t lo = A.ptr[row], hi = A.ptr[row + 1];
-  while (lo < hi) {
-    const int64_t mid = (lo + hi) >> 1;
-    const int32_t c = A.idx[mid];
-    if (c < col) lo = mid + 1;
-    else if (c > col) hi = mid;
-    else return mid;
-  }
-  return -1;
-}
-
-// Term list of C = Lm * Rm into the fixed pattern C.  variable_left: the values of Lm change between
-// uses (source = nz of Lm, weight = value of Rm), otherwise the values of Rm change.  One thread per
-// non-zero of C walks row i of Lm and looks column c up in the rows of Rm: no atomics, fixed order.
-// FILL == 0: cnt[nz] and per-slice width;  FILL == 1: write src / w.
-template <int FILL>
-__global__ void __launch_bounds__(256) k_prod_plan(DevCsr Lm, DevCsr Rm, DevCsr C, const int32_t *__restrict__ rowof, int variable_left,
-                                                    SellPlan P, int32_t *width) {
-  const int64_t nz = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  int count = 0;
-  if (nz < C.nnz) {
-    const int64_t i = rowof[nz];
-    const int32_t c = C.idx[nz];
-    const int64_t off = FILL ? P.sptr[nz >> 5] + (nz & 31) : 0;
-    for (int64_t a = Lm.ptr[i]; a < Lm.ptr[i + 1]; ++a) {
-      const int64_t b = csr_find(Rm, Lm.idx[a], c);
-      if (b < 0) continue;
-      if (FILL) {
-        P.src[off + 32 * (int64_t)count] = (int32_t)(variable_left ? a : b);
-        P.w[off + 32 * (int64_t)count] = variable_left ? Rm.val[b] : Lm.val[a];
-      }
-      ++count;
-    }
-    if (!FILL) P.cnt[nz] = count;
-  }
-  if (!FILL) {
-    int wmax = count;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) wmax = max(wmax, __shfl_xor_sync(0xffffffffu, wmax, o));
-    if ((threadIdx.x & 31) == 0 && nz < C.nnz) width[nz >> 5] = wmax;
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// coarse dense inverse: Minv = (D A D)^{-1} with D = diag(a_ii)^{-1/2} folded back in, so that
-// x = Minv_out * b solves A x = b.  One CTA, everything in shared memory, m <= kCoarseMaxDense.
-//   shared layout: S[m][m+1] (scaled matrix -> Cholesky factor L), Li[m(m+1)/2] (packed inverse of L), d[m]
-// ------------------------------------------------------------------------------------------------
-constexpr int kCoarseMaxDense = 128;
-inline size_t coarse_inverse_smem(int m) { return sizeof(double) * ((size_t)m * (m + 1) + (size_t)m * (m + 1) / 2 + m); }
 
 __global__ void __launch_bounds__(1024) k_coarse_inverse(DevCsr A, double *Minv) {
   extern __shared__ double sm[];
@@ -162,7 +192,6 @@ __global__ void __launch_bounds__(1024) k_coarse_inverse(DevCsr A, double *Minv)
     Minv[t] = s * d[i] * d[j];
   }
 }
-
 
 // ------------------------------------------------------------------------------------------------
 // Robust direct solve of a small system (m <= kCoarseMaxDense) in one CTA:  x = A^{-1} b.
@@ -297,6 +326,103 @@ __global__ void __launch_bounds__(1024) k_dense_solve_small(DevCsr A, const doub
   for (int i = tid; i < m; i += nt) x[i] = rhs[i];
   if (tid == 0 && info) info[0] = 1;
 }
-inline size_t dense_solve_small_smem(int m) { return sizeof(double) * ((size_t)m * (m + 1) + 2 * (size_t)m); }
+
+// factor the nb x nb diagonal block at (k0, k0) in shared memory, write L11 back and inv(L11) (row-major, ld 64) to Linv
+__global__ void __launch_bounds__(1024) k_chol_diag_inv(double *A, int m, int k0, double *Linv) {
+  extern __shared__ double chol_sm[];   // 2 x 64 x 65 doubles (dynamic: above the 48 KB static limit)
+  double (*L)[kCholNB + 1] = reinterpret_cast<double (*)[kCholNB + 1]>(chol_sm);
+  double (*Li)[kCholNB + 1] = reinterpret_cast<double (*)[kCholNB + 1]>(chol_sm + kCholNB * (kCholNB + 1));
+  const int nb = min(kCholNB, m - k0);
+  const int tid = threadIdx.x, nt = blockDim.x;
+  for (int t = tid; t < kCholNB * kCholNB; t += nt) {
+    const int i = t / kCholNB, j = t % kCholNB;
+    L[i][j] = (i < nb && j <= i) ? A[(size_t)(k0 + i) * m + k0 + j] : 0.0;
+    Li[i][j] = 0.0;
+  }
+  __syncthreads();
+  for (int j = 0; j < nb; ++j) {
+    if (tid == 0) L[j][j] = sqrt(L[j][j]);
+    __syncthreads();
+    const double pv = L[j][j];
+    for (int i = j + 1 + tid; i < nb; i += nt) L[i][j] /= pv;
+    __syncthreads();
+    const int rem = nb - j - 1;
+    for (int t = tid; t < rem * rem; t += nt) {
+      const int i = j + 1 + t / rem, k = j + 1 + t % rem;
+      if (k <= i) L[i][k] -= L[i][j] * L[k][j];
+    }
+    __syncthreads();
+  }
+  // inverse of the triangular block, one warp per column
+  const int lane = tid & 31, wid = tid >> 5, nw = nt >> 5;
+  for (int c = wid; c < nb; c += nw) {
+    if (lane == 0) Li[c][c] = 1.0 / L[c][c];
+    __syncwarp();
+    for (int i = c + 1; i < nb; ++i) {
+      double sacc = 0.0;
+      for (int k = c + lane; k < i; k += 32) sacc += L[i][k] * Li[k][c];
+      sacc = warp_sum(sacc);
+      if (lane == 0) Li[i][c] = -sacc / L[i][i];
+      __syncwarp();
+    }
+  }
+  __syncthreads();
+  for (int t = tid; t < kCholNB * kCholNB; t += nt) {
+    const int i = t / kCholNB, j = t % kCholNB;
+    if (i < nb && j <= i) A[(size_t)(k0 + i) * m + k0 + j] = L[i][j];
+    Linv[t] = (i < nb && j < nb) ? Li[i][j] : 0.0;
+  }
+}
+
+// x = (L L')^{-1} (d .* b) .* d for ONE right-hand side with the blocked factor and the panel inverses (Linv: panels x 64 x 64).
+// One CTA walks the panels (the dependency is sequential anyway): y_blk = inv(L11) b_blk, then b_rest -= L21 y_blk; and back.
+__global__ void __launch_bounds__(1024) k_chol_solve_blocked(const double *__restrict__ A, int m, const double *__restrict__ Linv,
+                                                              const double *__restrict__ d, const double *__restrict__ b, double *x) {
+  extern __shared__ double v[];   // m
+  __shared__ double blk[kCholNB];
+  const int tid = threadIdx.x, nt = blockDim.x;
+  for (int i = tid; i < m; i += nt) v[i] = b[i] * d[i];
+  __syncthreads();
+  const int npan = (m + kCholNB - 1) / kCholNB;
+  for (int pnl = 0; pnl < npan; ++pnl) {
+    const int k0 = pnl * kCholNB, nb = min(kCholNB, m - k0);
+    const double *Li = Linv + (size_t)pnl * kCholNB * kCholNB;
+    if (tid < nb) {
+      double sacc = 0.0;
+      for (int j = 0; j <= tid; ++j) sacc += Li[tid * kCholNB + j] * v[k0 + j];
+      blk[tid] = sacc;
+    }
+    __syncthreads();
+    if (tid < nb) v[k0 + tid] = blk[tid];
+    for (int i = k0 + nb + tid; i < m; i += nt) {
+      const double *row = A + (size_t)i * m + k0;
+      double sacc = 0.0;
+      for (int j = 0; j < nb; ++j) sacc += row[j] * blk[j];
+      v[i] -= sacc;
+    }
+    __syncthreads();
+  }
+  for (int pnl = npan - 1; pnl >= 0; --pnl) {
+    const int k0 = pnl * kCholNB, nb = min(kCholNB, m - k0);
+    const double *Li = Linv + (size_t)pnl * kCholNB * kCholNB;
+    // y_blk[j] -= sum_{i >= k0+nb} L[i][k0+j] x[i]   (column sums: warp per j, lanes over rows)
+    const int lane = tid & 31, wid = tid >> 5, nw = nt >> 5;
+    for (int j = wid; j < nb; j += nw) {
+      double sacc = 0.0;
+      for (int i = k0 + nb + lane; i < m; i += 32) sacc += A[(size_t)i * m + k0 + j] * v[i];
+      sacc = warp_sum(sacc);
+      if (lane == 0) blk[j] = v[k0 + j] - sacc;
+    }
+    __syncthreads();
+    // x_blk = inv(L11)' y_blk
+    if (tid < nb) {
+      double sacc = 0.0;
+      for (int i = tid; i < nb; ++i) sacc += Li[i * kCholNB + tid] * blk[i];
+      v[k0 + tid] = sacc;
+    }
+    __syncthreads();
+  }
+  for (int i = tid; i < m; i += nt) x[i] = v[i] * d[i];
+}
 
 }  // namespace mgbx

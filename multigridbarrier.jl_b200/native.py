@@ -547,7 +547,7 @@ def ruge_stuben(K, max_coarse=2, max_levels=10, theta=0.25):
 
 def kron_factor(M, r1, r2, c1, c2):
     """Host-only: (A, B) with M == kron(A, B) (A r1 x c1, B r2 x c2) or None -- the structure test behind the sum-factorised spectral
-    assembly (csrc/mgbx.cu kron_factor)."""
+    assembly (csrc/engine.hpp kron_factor)."""
     M = np.ascontiguousarray(M, dtype=np.float64)
     assert M.shape == (r1 * r2, c1 * c2)
     A, B = np.zeros((r1, c1)), np.zeros((r2, c2))
