@@ -247,6 +247,45 @@ struct EvalOut {
   bool finite;
   double nonfinite_nodes, lin;
 };
+// f0 / f1 at a trial point, with |xn - x|^2 exactly as evaluated in floating point (zero: the step no longer moves x)
+struct TrialOut : EvalOut {
+  double step2;
+};
+struct Dot2 {
+  double ab, aa, nonfinite;   // a.b, a.a, #non-finite entries of a
+};
+struct MaxAbs {
+  double max, absmax, nonfinite;
+};
+// PCG stopping parameters: |r|^2 <= rtol2 |b|^2, or stagnation for `window` iterations without a new best residual
+struct SolveTol {
+  double rtol2;
+  int window;
+};
+
+// Slots of the handle's device scalars dscal[kScalSlots] and of their pinned host mirror hscal.  The reduction kernels
+// write fixed regions of dscal; evaluate.cu copies them to hscal and returns the values.  Successive calls reuse regions:
+// each result is read before the next launch that writes its region.
+// single GPU (fetched as the leading kScalSingle slots):
+constexpr int kScalEval = 0;     // [0, 4) red_out of the f0 / f1 node and element kernels (and of k_node<NODE_SLACK> on every
+                                 // path): sum bw F0 (or sum F0), sum w c.Dz, #non-finite F0, max slack (computed, never read)
+constexpr int kScalMaxAbs = 0;   // [0, 3) k_maxabs: max, max|.|, #non-finite; reuses the evaluation slots, on every path
+constexpr int kScalDot = 4;      // [4, 7) k_dot2: a.b, a.a, #non-finite(a)
+constexpr int kScalTrial = 7;    // [7] k_trial: |xn - x|^2, read by the evaluation that follows the trial
+constexpr int kScalSingle = 8;
+// hscal only: readback of the solve kernel's result record (kPcg2Out*, pcg2.hpp)
+constexpr int kScalPcgOut = 8;   // [8, 14)
+// multi-GPU (the whole array is fetched); eval_f01 sums [kScalTrialSeg + 1, kScalDotSeg + 3) over the ranks in one all-reduce
+constexpr int kScalTrialSeg = 38;   // [38] shared / [39] local part of |xn - x|^2 (k_trial_seg), zeroed by each evaluation
+constexpr int kScalEvalDist = 40;   // [40, 44) red_out; the max slack is summed over the ranks here, not max-reduced
+constexpr int kScalDotSeg = 44;     // [44, 50) k_dot2_seg: local part {a.b, a.a, #non-finite}, then shared part
+constexpr int kScalDotSeg2 = 50;    // [50, 56) eval_f01's second k_dot2_seg, after the shared gradient entries were summed
+constexpr int kScalSlots = 64;
+static_assert(kScalEval + 4 <= kScalDot && kScalDot + 3 <= kScalTrial && kScalTrial + 1 <= kScalSingle &&
+                  kScalSingle <= kScalPcgOut && kScalPcgOut + kPcg2OutCount <= kScalTrialSeg &&
+                  kScalTrialSeg + 2 == kScalEvalDist && kScalEvalDist + 4 == kScalDotSeg &&   // contiguous for the all-reduce
+                  kScalDotSeg + 6 <= kScalDotSeg2 && kScalDotSeg2 + 6 <= kScalSlots,
+              "scalar slot regions overlap, break the all-reduced range or exceed dscal");
 
 }  // namespace mgbx
 
@@ -260,7 +299,7 @@ struct mgbx_handle {
   // reduction scratch
   double *partials = nullptr;
   unsigned int *ticket = nullptr;
-  double *dscal = nullptr;   // device scalars
+  double *dscal = nullptr;   // device scalars, kScalSlots (layout above)
   double *hscal = nullptr;   // pinned host mirror
   // stats of the current step
   mgbx_step_result *res = nullptr;
@@ -277,8 +316,7 @@ struct mgbx_handle {
   cudaEvent_t ev_cur = nullptr;
   int pcg2_grid = 0;         // CTAs of the solve kernel k_pcg2
   double dgemm_flops = 0.0;   // FP64 tensor-core flops issued so far (spectral path)
-  double cur_rtol2 = 1e-22;
-  int cur_window = 25;       // PCG stagnation window (iterations without a new best residual)
+  mgbx::SolveTol last_tol{};   // the last Newton run's tolerance (mgbx_create's before any), inherited by matched t and mgbx_solve_newton_system
   // multi-GPU
   int rank = 0, nranks = 1;
   void *comm = nullptr;
@@ -296,6 +334,7 @@ struct SolveResult {
   int status = 1;      // 1 converged / direct, 2 stagnated above the tolerance, 3 iteration limit, -1 breakdown
   double rel = 0.0;    // final relative residual |r| / |b| (0 for a direct solve)
   double erel = 0.0;   // share of the direction's energy b.x = |x|_A^2 gained in the last four PCG iterations
+  Dot2 dg{};           // (dir, g) of Engine::solve: the Newton decrement g.dir, |dir|^2 and dir's non-finite entries
 };
 
 struct Engine {
@@ -391,9 +430,9 @@ struct Engine {
   void axpby(int64_t m, double a, const double *x, double b, const double *y, double *out);
   void prolong_to_fine(Amg &A, int J, const double *x, const double *zbase, double *zf);
   void restrict_from_fine(Amg &A, int J, const double *gb, double *gJ);
-  void dot2_fetch(Amg &A, int J, const double *a, const double *b);
-  void maxabs_fetch(int64_t n, const double *v);
-  void trial(Amg &A, int J, double sigma);
+  Dot2 dot2(Amg &A, int J, const double *a, const double *b);
+  MaxAbs maxabs(int64_t n, const double *v);
+  TrialOut eval_trial(Amg &A, int J, double t, double sigma);
   void phase1_slack(Amg &A, Amg &F);
   void blockgrad(Amg &A, const ElemParams &E);
   NodeParams node_params(Amg &A, double t);
@@ -401,7 +440,8 @@ struct Engine {
   bool elem_fused_setup(Amg &A, const NodeParams &NP, int nex, ElemFused &Q, size_t &smem, unsigned int &grid);
   int plap_dim(const Amg &A) const;
   bool plap_setup(Amg &A, int dim, double t, bool use_bw, PlapParams &Q, size_t &smem, unsigned int &grid, bool cond = true);
-  EvalOut eval_f01(Amg &A, int J, double t, const double *zbase, const double *x, double *gout, bool use_bw = true);
+  EvalOut eval_f01(Amg &A, int J, double t, const double *zbase, const double *x, double *gout, bool use_bw = true,
+                   double *step2 = nullptr);
 
   // ---------------------------------------------------------------- system assembly (evaluate.cu; system_for: setup.cu)
   System &system_for(Amg &A, int J);
@@ -425,9 +465,9 @@ struct Engine {
   void sell_prepare(System &S, int ktop);
   System::Pcg2Dev &pcg2_plan(System &S, int ktop);
   void pcg2_setup_dist(System::Pcg2Dev &D, int nshard);
-  SolveResult pcg(System &S, int ktop, const double *b, double *x);
-  SolveResult solve_compact(System &S, int ktop, const double *b, double *x);
-  SolveResult solve(Amg &A, System &S, int J, const double *g, double *dir);
+  SolveResult pcg(System &S, int ktop, const double *b, double *x, const SolveTol &tol);
+  SolveResult solve_compact(System &S, int ktop, const double *b, double *x, const SolveTol &tol);
+  SolveResult solve(Amg &A, System &S, int J, const double *g, double *dir, const SolveTol &tol);
 
   // ---------------------------------------------------------------- Newton (newton.cu)
   struct NewtonOut {

@@ -58,6 +58,12 @@ void launch_plap(int dim, bool cond, const PlapParams &Q, unsigned int grid, siz
   }
 }
 
+// the result of k_dot2 from its slots, and of k_dot2_seg: the local part (summed over the ranks) plus the shared part
+Dot2 dot2_slots(const double *d) { return {d[0], d[1], d[2]}; }
+Dot2 dot2_seg_slots(const double *local, const double *shared) {
+  return {local[0] + shared[0], local[1] + shared[1], local[2] + shared[2]};
+}
+
 }  // namespace
 
 void kron_w_init(size_t smem) { CK(cudaFuncSetAttribute(k_kron_w, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); }
@@ -128,32 +134,37 @@ void Engine::allreduce_shared(Amg &A, int J, double *v, double *extra, int64_t n
   if (extra) allreduce(extra, nextra);
   NCK(nccl_api().GroupEnd());
 }
-// hscal[4..6] = {a.b, a.a, #non-finite(a)} over a level-J vector (all ranks obtain the same values)
-void Engine::dot2_fetch(Amg &A, int J, const double *a, const double *b) {
+// {a.b, a.a, #non-finite(a)} over a level-J vector (all ranks obtain the same values)
+Dot2 Engine::dot2(Amg &A, int J, const double *a, const double *b) {
   const int64_t m = A.m[J];
   if (!dist()) {
-    LAUNCH(KC_VEC, k_dot2<<<red_grid(m), kRedThreads, 0, s>>>(m, a, b, h->partials, h->ticket, h->dscal + 4));
-    fetch(8);
-    return;
+    LAUNCH(KC_VEC, k_dot2<<<red_grid(m), kRedThreads, 0, s>>>(m, a, b, h->partials, h->ticket, h->dscal + kScalDot));
+    fetch(kScalSingle);
+    return dot2_slots(h->hscal + kScalDot);
   }
-  LAUNCH(KC_VEC, k_dot2_seg<<<red_grid(m), kRedThreads, 0, s>>>(seglist(A, J), m, a, b, h->partials, h->ticket, h->dscal + 44));
-  allreduce(h->dscal + 44, 3);
-  fetch(64);
-  for (int k = 0; k < 3; ++k) h->hscal[4 + k] = h->hscal[44 + k] + h->hscal[47 + k];
+  LAUNCH(KC_VEC, k_dot2_seg<<<red_grid(m), kRedThreads, 0, s>>>(seglist(A, J), m, a, b, h->partials, h->ticket, h->dscal + kScalDotSeg));
+  allreduce(h->dscal + kScalDotSeg, 3);   // the local part; the shared part is already the same on every rank
+  fetch(kScalSlots);
+  return dot2_seg_slots(h->hscal + kScalDotSeg, h->hscal + kScalDotSeg + 3);
 }
 
-// hscal[0..2] = {max, max|.|, #non-finite} of a node vector (over all ranks)
-void Engine::maxabs_fetch(int64_t n, const double *v) {
-  LAUNCH(KC_VEC, k_maxabs<<<red_grid(n), kRedThreads, 0, s>>>(n, v, h->partials, h->ticket, h->dscal));
-  if (dist()) allreduce(h->dscal, 3, kNcclMax);
-  fetch(3);
+// {max, max|.|, #non-finite} of a node vector (over all ranks)
+MaxAbs Engine::maxabs(int64_t n, const double *v) {
+  LAUNCH(KC_VEC, k_maxabs<<<red_grid(n), kRedThreads, 0, s>>>(n, v, h->partials, h->ticket, h->dscal + kScalMaxAbs));
+  if (dist()) allreduce(h->dscal + kScalMaxAbs, 3, kNcclMax);
+  fetch(kScalMaxAbs + 3);
+  const double *d = h->hscal + kScalMaxAbs;
+  return {d[0], d[1], d[2]};
 }
 
-// A.xn = A.x - sigma A.dir at level J, with the step norm(s) for the stall test left in dscal
-void Engine::trial(Amg &A, int J, double sigma) {
+// f0 / f1 at the level-J trial point A.xn = A.x - sigma A.dir (gradient into A.gn)
+TrialOut Engine::eval_trial(Amg &A, int J, double t, double sigma) {
   const int64_t m = A.m[J];
-  if (!dist()) LAUNCH(KC_VEC, k_trial<<<red_grid(m), kRedThreads, 0, s>>>(m, A.x, A.dir, sigma, A.xn, h->partials, h->ticket, h->dscal + 7));
-  else LAUNCH(KC_VEC, k_trial_seg<<<red_grid(m), kRedThreads, 0, s>>>(seglist(A, J), m, A.x, A.dir, sigma, A.xn, h->partials, h->ticket, h->dscal + 38));
+  if (!dist()) LAUNCH(KC_VEC, k_trial<<<red_grid(m), kRedThreads, 0, s>>>(m, A.x, A.dir, sigma, A.xn, h->partials, h->ticket, h->dscal + kScalTrial));
+  else LAUNCH(KC_VEC, k_trial_seg<<<red_grid(m), kRedThreads, 0, s>>>(seglist(A, J), m, A.x, A.dir, sigma, A.xn, h->partials, h->ticket, h->dscal + kScalTrialSeg));
+  double step2 = 0.0;
+  const EvalOut e = eval_f01(A, J, t, A.z, A.xn, A.gn, true, &step2);
+  return {e, step2};
 }
 
 // phase-I start of the feasibility AMG F: [z0, slack] with slack_i = 2*max(slack_fn(D z0), 1) (src/mgb.jl:437-445);
@@ -193,7 +204,7 @@ NodeParams Engine::node_params(Amg &A, double t) {
   P.G = A.G;
   P.partials = h->partials;
   P.ticket = h->ticket;
-  P.red_out = h->dscal;
+  P.red_out = h->dscal + kScalEval;
   P.slack = A.slack;
   return P;
 }
@@ -298,7 +309,7 @@ bool Engine::plap_setup(Amg &A, int dim, double t, bool use_bw, PlapParams &Q, s
   Q.mu = A.cd.pc[0].mu_uniform;
   Q.partials = h->partials;
   Q.ticket = h->ticket;
-  Q.red_out = dist() ? h->dscal + 40 : h->dscal;
+  Q.red_out = h->dscal + (dist() ? kScalEvalDist : kScalEval);
   if (Q.bulk) {   // bulk copies need 16-byte aligned sources: every base pointer, and the column stride n of f / the state blocks
     auto al16 = [](const void *q) { return q == nullptr || ((uintptr_t)q & 15) == 0; };
     bool ok = al16(Q.zu) && al16(Q.zs) && al16(Q.w) && al16(Q.bw) && al16(Q.f) && (A.n % 2 == 0);
@@ -317,12 +328,13 @@ bool Engine::plap_setup(Amg &A, int dim, double t, bool use_bw, PlapParams &Q, s
 }
 // ---------------------------------------------------------------- f0 + f1 at level J
 // zbase: broken state the level correction is added to; x: level-J coefficients; gout: level-J gradient
-EvalOut Engine::eval_f01(Amg &A, int J, double t, const double *zbase, const double *x, double *gout, bool use_bw) {
+// step2: |xn - x|^2 of the trial launch that produced x (eval_trial)
+EvalOut Engine::eval_f01(Amg &A, int J, double t, const double *zbase, const double *x, double *gout, bool use_bw, double *step2) {
   cudaEvent_t st = stage_begin();
   prolong_to_fine(A, J, x, zbase, A.zf);
   NodeParams P = node_params(A, t);
   if (!use_bw) P.bw = nullptr;
-  if (dist()) P.red_out = h->dscal + 40;
+  if (dist()) P.red_out = h->dscal + kScalEvalDist;
   ElemFused Q;
   PlapParams PQ;
   size_t smem = 0;
@@ -340,32 +352,38 @@ EvalOut Engine::eval_f01(Amg &A, int J, double t, const double *zbase, const dou
     blockgrad(A, elem_params(A));
   }
   restrict_from_fine(A, J, A.gb, gout);
+  const double *red;   // red_out: {sum bw F0 (or sum F0), sum w c.Dz, #non-finite F0, max slack}
+  Dot2 gg;             // {0, |gout|^2, #non-finite(gout)}
   if (!dist()) {
-    LAUNCH(KC_VEC, k_dot2<<<red_grid(A.m[J]), kRedThreads, 0, s>>>(A.m[J], gout, nullptr, h->partials, h->ticket, h->dscal + 4));
+    LAUNCH(KC_VEC, k_dot2<<<red_grid(A.m[J]), kRedThreads, 0, s>>>(A.m[J], gout, nullptr, h->partials, h->ticket, h->dscal + kScalDot));
     stage_end(STAGE_F01, st);
-    fetch(8);
+    fetch(kScalSingle);
+    red = h->hscal + kScalEval;
+    gg = dot2_slots(h->hscal + kScalDot);
+    if (step2) *step2 = h->hscal[kScalTrial];
   } else {
     // partial sums over this rank's elements -> all ranks: the shared part of R'g, the objective scalars, and the
     // local-part norms (one grouped all-reduce); the shared-part norm is then formed identically on every rank
     const SegList SG = seglist(A, J);
-    LAUNCH(KC_VEC, k_dot2_seg<<<red_grid(A.m[J]), kRedThreads, 0, s>>>(SG, A.m[J], gout, nullptr, h->partials, h->ticket, h->dscal + 44));
-    allreduce_shared(A, J, gout, h->dscal + 39, 8);   // [39] trial norm (local part), [40..43] node sums, [44..46] local dot
-    LAUNCH(KC_VEC, k_dot2_seg<<<red_grid(A.m[J]), kRedThreads, 0, s>>>(SG, A.m[J], gout, nullptr, h->partials, h->ticket, h->dscal + 50));
+    LAUNCH(KC_VEC, k_dot2_seg<<<red_grid(A.m[J]), kRedThreads, 0, s>>>(SG, A.m[J], gout, nullptr, h->partials, h->ticket, h->dscal + kScalDotSeg));
+    // the local trial norm, the node sums and the local dot
+    allreduce_shared(A, J, gout, h->dscal + kScalTrialSeg + 1, kScalDotSeg + 3 - (kScalTrialSeg + 1));
+    LAUNCH(KC_VEC, k_dot2_seg<<<red_grid(A.m[J]), kRedThreads, 0, s>>>(SG, A.m[J], gout, nullptr, h->partials, h->ticket, h->dscal + kScalDotSeg2));
     stage_end(STAGE_F01, st);
-    fetch(64);
-    for (int k = 0; k < 4; ++k) h->hscal[k] = h->hscal[40 + k];
-    for (int k = 0; k < 3; ++k) h->hscal[4 + k] = h->hscal[44 + k] + h->hscal[53 + k];
-    h->hscal[7] = h->hscal[38] + h->hscal[39];
-    CK(cudaMemsetAsync(h->dscal + 38, 0, 2 * sizeof(double), s));   // the trial norms are consumed
+    fetch(kScalSlots);
+    red = h->hscal + kScalEvalDist;
+    gg = dot2_seg_slots(h->hscal + kScalDotSeg, h->hscal + kScalDotSeg2 + 3);
+    if (step2) *step2 = h->hscal[kScalTrialSeg] + h->hscal[kScalTrialSeg + 1];
+    CK(cudaMemsetAsync(h->dscal + kScalTrialSeg, 0, 2 * sizeof(double), s));   // the trial norms are consumed
   }
   if (h->res) h->res->f01_evals++;
   EvalOut o;
-  const double bar = (use_bw && A.bw) ? h->hscal[0] : h->hscal[0] * (1.0 / (double)A.n_global);
-  o.lin = h->hscal[1];
-  o.y = bar + h->hscal[1];
-  o.nonfinite_nodes = h->hscal[2];
-  o.gnorm = std::sqrt(h->hscal[5]);
-  o.finite = std::isfinite(o.y) && (h->hscal[6] == 0.0) && std::isfinite(h->hscal[5]);
+  const double bar = (use_bw && A.bw) ? red[0] : red[0] * (1.0 / (double)A.n_global);
+  o.lin = red[1];
+  o.y = bar + red[1];
+  o.nonfinite_nodes = red[2];
+  o.gnorm = std::sqrt(gg.aa);
+  o.finite = std::isfinite(o.y) && (gg.nonfinite == 0.0) && std::isfinite(gg.aa);
   return o;
 }
 // Which Euclidean-power pieces can be condensed analytically (node_barrier.cuh piece_eval): identity A, not under the phase-I

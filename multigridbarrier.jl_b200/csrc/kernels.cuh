@@ -200,7 +200,7 @@ __global__ void __launch_bounds__(256) k_blockhess(ElemParams P, PairList PL, co
 // ------------------------------------------------------------------------------------------------
 // vector kernels (all scalars stay on the device)
 // ------------------------------------------------------------------------------------------------
-// out[0] = a.b, out[1] = a.a, out[2] = #non-finite entries of a
+// out = {a.b, a.a, #non-finite entries of a}
 __global__ void __launch_bounds__(kRedThreads) k_dot2(int64_t m, const double *__restrict__ a, const double *__restrict__ b,
                                                        double *partials, unsigned int *ticket, double *out) {
   double red[3] = {0.0, 0.0, 0.0};
@@ -214,7 +214,7 @@ __global__ void __launch_bounds__(kRedThreads) k_dot2(int64_t m, const double *_
   grid_reduce<3>(red, op, partials, ticket, out);
 }
 
-// xn = x - s*d;  out[0] = |xn - x|^2 (exactly as evaluated in floating point: stall detection, src/newton.jl:141)
+// xn = x - s*d;  out = {|xn - x|^2} (exactly as evaluated in floating point: stall detection, src/newton.jl:141)
 __global__ void __launch_bounds__(kRedThreads) k_trial(int64_t m, const double *__restrict__ x, const double *__restrict__ d, double s,
                                                         double *xn, double *partials, unsigned int *ticket, double *out) {
   double red[1] = {0.0};
@@ -254,7 +254,7 @@ __global__ void k_phase1_slack(int64_t n, const double *slack, double *out) {
   if (i < n) out[i] = 2.0 * fmax(slack[i], 1.0);
 }
 
-// out[0..2] = {a.b, a.a, #non-finite entries of a} over the LOCAL segments, out[3..5] the same over the SHARED ones
+// out = {a.b, a.a, #non-finite entries of a} over the LOCAL segments, then the same three over the SHARED ones
 __global__ void __launch_bounds__(kRedThreads) k_dot2_seg(SegList S, int64_t m, const double *__restrict__ a, const double *__restrict__ b,
                                                            double *partials, unsigned int *ticket, double *out) {
   double red[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
@@ -269,7 +269,7 @@ __global__ void __launch_bounds__(kRedThreads) k_dot2_seg(SegList S, int64_t m, 
   grid_reduce<6>(red, op, partials, ticket, out);
 }
 
-// xn = x - s*d;  out[0] = |xn - x|^2 over the SHARED segments, out[1] over the LOCAL ones
+// xn = x - s*d;  out = {|xn - x|^2 over the SHARED segments, the same over the LOCAL ones}
 __global__ void __launch_bounds__(kRedThreads) k_trial_seg(SegList S, int64_t m, const double *__restrict__ x, const double *__restrict__ d,
                                                             double s, double *xn, double *partials, unsigned int *ticket, double *out) {
   double red[2] = {0.0, 0.0};

@@ -360,13 +360,13 @@ void Engine::pcg2_setup_dist(System::Pcg2Dev &D, int nshard) {
 }
 
 // Preconditioned CG on lev[ktop], the whole solve in one cooperative launch of k_pcg2
-SolveResult Engine::pcg(System &S, int ktop, const double *b, double *x) {
+SolveResult Engine::pcg(System &S, int ktop, const double *b, double *x, const SolveTol &tol) {
   SysLevel &Lv = S.lev[ktop];
   const int64_t m = Lv.m;
   System::Pcg2Dev &D = pcg2_plan(S, ktop);
   if (b != S.pc_b) copy(S.pc_b, b, m);
   pre_launch(KC_PCG);
-  CK(pcg2_launch(D.dev, h->pcg2_grid, D.smem, h->cur_rtol2, h->cfg.pcg_maxit, h->cur_window, D.host.dist.nshard > 0, s));
+  CK(pcg2_launch(D.dev, h->pcg2_grid, D.smem, tol.rtol2, h->cfg.pcg_maxit, tol.window, D.host.dist.nshard > 0, s));
   post_launch(KC_PCG);
   if (D.host.prof) {   // debugging aid: accumulate the per-phase durations of this launch
     h->prof_host.resize(1 + 2 * (size_t)kPcg2ProfCap);
@@ -384,23 +384,22 @@ SolveResult Engine::pcg(System &S, int ktop, const double *b, double *x) {
       h->prof_cnt[tag]++;
     }
   }
-  // k_pcg2's out: [0] iterations, [1] |r|^2, [2] exit status, [3] |b|^2, [4] b.x, [5] b.x gained in the last four iterations
-  CK(cudaMemcpyAsync(h->hscal + 8, S.pcg_out, sizeof(double) * 6, cudaMemcpyDeviceToHost, s));
+  CK(cudaMemcpyAsync(h->hscal + kScalPcgOut, S.pcg_out, sizeof(double) * kPcg2OutCount, cudaMemcpyDeviceToHost, s));
   sync();
-  const double *o = h->hscal + 8;
-  const int it = (int)o[0];
-  const double status = o[2];
+  const double *o = h->hscal + kScalPcgOut;
+  const int it = (int)o[kPcg2OutIters];
+  const double status = o[kPcg2OutStatus];
   if (status == -3.0) throw std::runtime_error("row-sharded solve: a peer rank never arrived at a cross-GPU barrier (ranks out of step?)");
   if (x != D.host.x) copy(x, D.host.x, m);
   SolveResult r;
   r.iters = status < 0 ? -std::max(it, 1) : it;
   r.status = (int)status;
-  r.rel = (o[3] > 0.0) ? std::sqrt(o[1] / o[3]) : 0.0;
-  r.erel = (o[4] > 0.0) ? o[5] / o[4] : 0.0;
+  r.rel = (o[kPcg2OutBB] > 0.0) ? std::sqrt(o[kPcg2OutRR] / o[kPcg2OutBB]) : 0.0;
+  r.erel = (o[kPcg2OutEnergy] > 0.0) ? o[kPcg2OutEnergyLast4] / o[kPcg2OutEnergy] : 0.0;
   return r;
 }
 
-SolveResult Engine::solve_compact(System &S, int ktop, const double *b, double *x) {
+SolveResult Engine::solve_compact(System &S, int ktop, const double *b, double *x, const SolveTol &tol) {
   SysLevel &Lv = S.lev[ktop];
   if (use_direct(S, Lv)) {
     direct_solve(Lv, b, x);
@@ -413,7 +412,7 @@ SolveResult Engine::solve_compact(System &S, int ktop, const double *b, double *
     throw UnsupportedError("Newton system with a slack variable that cannot be eliminated node-locally (e.g. a slack in :broken_P1) and " +
                            std::to_string((long long)Lv.m) + " unknowns: above the dense direct solver's size (8192) only the V-cycle PCG is available, "
                            "which is not reliable for these systems (set cfg.uncondensed_pcg = 1 to try anyway)");
-  SolveResult r = pcg(S, ktop, b, x);
+  SolveResult r = pcg(S, ktop, b, x, tol);
   // PCG first, direct second: a solve that broke down or stayed inexact is redone by the dense Cholesky when the system is
   // small enough to hold as a dense matrix (the un-condensable families, the last steps of a parabolic ramp)
   const bool bad = r.status < 0 || (r.rel > h->cfg.pcg_fail_rtol && r.erel > h->cfg.pcg_fail_etol);
@@ -432,13 +431,13 @@ SolveResult Engine::solve_compact(System &S, int ktop, const double *b, double *
 
 // dir = H_J^{-1} g  (full level-J vectors).  With a condensed system the node-local variables are
 // eliminated exactly first and recovered by back-substitution.
-SolveResult Engine::solve(Amg &A, System &S, int J, const double *g, double *dir) {
+SolveResult Engine::solve(Amg &A, System &S, int J, const double *g, double *dir, const SolveTol &tol) {
   cudaEvent_t st = stage_begin();
   const int ktop = S.ltop - J;
   SysLevel &Lv = S.lev[ktop];
   SolveResult r;
   if (S.nE == 0) {
-    r = solve_compact(S, ktop, g, dir);
+    r = solve_compact(S, ktop, g, dir, tol);
   } else {
     // (only at the fine level)  rhs_K = g_K + R_K' sum_j D_j' gt_j
     CondParams C;
@@ -465,7 +464,7 @@ SolveResult Engine::solve(Amg &A, System &S, int J, const double *g, double *dir
     }
     for (size_t q = 0; q < S.kept.size(); ++q)
       copy(S.pc_b + Lv.off[q], A.tmp + A.voff[A.L - 1][S.kept[q]], Lv.off[q + 1] - Lv.off[q]);
-    r = solve_compact(S, ktop, S.pc_b, S.pc_x);
+    r = solve_compact(S, ktop, S.pc_b, S.pc_x, tol);
     zero(dir, A.m[A.L - 1]);
     for (size_t q = 0; q < S.kept.size(); ++q)
       copy(dir + A.voff[A.L - 1][S.kept[q]], S.pc_x + Lv.off[q], Lv.off[q + 1] - Lv.off[q]);
@@ -476,8 +475,7 @@ SolveResult Engine::solve(Amg &A, System &S, int J, const double *g, double *dir
     LAUNCH(KC_COND, k_backsubst<<<nblk(A.n), 256, 0, s>>>(C, NP, g, dir));
   }
   stage_end(STAGE_SOLVE, st);
-  // inc = g . dir, finiteness of dir
-  dot2_fetch(A, J, dir, g);
+  r.dg = dot2(A, J, dir, g);
   if (h->res) {
     h->res->linear_solves++;
     h->res->pcg_iters += r.iters > 0 ? r.iters : -r.iters;

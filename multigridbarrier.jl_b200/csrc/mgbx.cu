@@ -165,7 +165,7 @@ int mgbx_create(const mgbx_problem *prob, const mgbx_config *cfg, mgbx_handle **
   if (h->cfg.dense_direct_max > kDenseMaxUnknowns) h->cfg.dense_direct_max = kDenseMaxUnknowns;
   if (h->cfg.coarse_max > kCoarseMaxDense) h->cfg.coarse_max = kCoarseMaxDense;
   if (h->cfg.coarse_max < 0) h->cfg.coarse_max = 0;
-  h->cur_rtol2 = h->cfg.pcg_rtol * h->cfg.pcg_rtol;
+  h->last_tol = {h->cfg.pcg_rtol * h->cfg.pcg_rtol, 25};   // until the first Newton run: a window of 25, not cfg.pcg_stall_window
   int rc = guarded(h, [&]() -> int {
     if (h->cfg.persistent != 2) throw ArgError("mgbx_config.persistent must be 2 (the only solve kernel)");
     int ndev = 0;
@@ -190,8 +190,8 @@ int mgbx_create(const mgbx_problem *prob, const mgbx_config *cfg, mgbx_handle **
     }
     h->partials = h->pool.zeros<double>((size_t)kRedBlocks * 8, h->stream);
     h->ticket = h->pool.zeros<unsigned int>(4, h->stream);
-    h->dscal = h->pool.zeros<double>(64, h->stream);
-    CK(cudaMallocHost((void **)&h->hscal, sizeof(double) * 64));
+    h->dscal = h->pool.zeros<double>(kScalSlots, h->stream);
+    CK(cudaMallocHost((void **)&h->hscal, sizeof(double) * kScalSlots));
     const mgbx_amg &a0 = prob->amg[0];
     create_amg(h, a0, h->amg[0]);
     Amg &A = h->amg[0];
@@ -334,10 +334,10 @@ int mgbx_scalars(mgbx_handle *h, int which, mgbx_scalars_out *out) {
     out->c_dot_Dz = e.lin;
     out->all_finite = 1;
     for (int v = 0; v < A.nu; ++v) {
-      E.maxabs_fetch(A.n, A.z + (int64_t)v * A.n);
-      out->var_max[v] = h->hscal[0];
-      out->var_absmax[v] = h->hscal[1];
-      if (h->hscal[2] != 0.0) out->all_finite = 0;
+      const MaxAbs r = E.maxabs(A.n, A.z + (int64_t)v * A.n);
+      out->var_max[v] = r.max;
+      out->var_absmax[v] = r.absmax;
+      if (r.nonfinite != 0.0) out->all_finite = 0;
     }
     return MGBX_OK;
   });
@@ -353,10 +353,7 @@ int mgbx_phase1_init(mgbx_handle *h, int32_t *needs_phase1, double *b, double *z
     EvalOut e = E.eval_f01(A, A.L - 1, 0.0, A.z, A.x, A.gn, /*use_bw=*/false);
     *needs_phase1 = (e.nonfinite_nodes > 0.0 || !std::isfinite(e.y)) ? 1 : 0;
     double zmax = 0.0;
-    for (int v = 0; v < A.nu; ++v) {
-      E.maxabs_fetch(A.n, A.z + (int64_t)v * A.n);
-      zmax = std::max(zmax, h->hscal[1]);
-    }
+    for (int v = 0; v < A.nu; ++v) zmax = std::max(zmax, E.maxabs(A.n, A.z + (int64_t)v * A.n).absmax);
     *zabsmax = zmax;
     *b = 0.0;
     if (*needs_phase1) {
@@ -364,8 +361,7 @@ int mgbx_phase1_init(mgbx_handle *h, int32_t *needs_phase1, double *b, double *z
       Amg &F = h->amg[1];
       // b = 2*max(1, max slack)   (src/mgb.jl:437-445)
       E.phase1_slack(A, F);
-      E.maxabs_fetch(A.n, F.zinit + (int64_t)A.nu * A.n);
-      *b = 2.0 * std::max(1.0, h->hscal[0]);
+      *b = 2.0 * std::max(1.0, E.maxabs(A.n, F.zinit + (int64_t)A.nu * A.n).max);
     }
     return MGBX_OK;
   });
@@ -546,7 +542,7 @@ int mgbx_barrier_eval(mgbx_handle *h, int which, int level, double t, const doub
     Engine E(h);
     CK(cudaMemcpyAsync(A.xn, s, sizeof(double) * A.m[level], cudaMemcpyHostToDevice, h->stream));
     EvalOut e = E.eval_f01(A, level, t, A.z, A.xn, A.gn);
-    if (order == 0) out[0] = e.y;
+    if (order == 0) *out = e.y;
     else {
       CK(cudaMemcpyAsync(out, A.gn, sizeof(double) * A.m[level], cudaMemcpyDeviceToHost, h->stream));
       CK(cudaStreamSynchronize(h->stream));
@@ -608,7 +604,7 @@ int mgbx_solve_newton_system(mgbx_handle *h, int which, int level, double t, con
     CK(cudaMemcpyAsync(A.xn, s, sizeof(double) * m, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(A.gn, rhs, sizeof(double) * m, cudaMemcpyHostToDevice, h->stream));
     E.assemble(A, S, level, t, A.z, A.xn);
-    const SolveResult r = E.solve(A, S, level, A.gn, A.dir);
+    const SolveResult r = E.solve(A, S, level, A.gn, A.dir, h->last_tol);
     if (pcg_iters) *pcg_iters = r.iters;
     CK(cudaMemcpyAsync(x, A.dir, sizeof(double) * m, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));

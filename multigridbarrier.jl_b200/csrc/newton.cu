@@ -29,8 +29,8 @@ Engine::NewtonOut Engine::newton(Amg &A, int J, double t, int maxit, int stop_ki
   // the finalize pass stops on floating-point stagnation (stopping_exact): give it directions converged to the
   // attainable accuracy so that it stagnates where a direct solve would
   const double rt = (stop_kind == 0) ? std::min(h->cfg.pcg_rtol, h->cfg.pcg_rtol_final) : h->cfg.pcg_rtol;
-  h->cur_rtol2 = rt * rt;
-  h->cur_window = (stop_kind == 0) ? 6 : std::max(1, h->cfg.pcg_stall_window);   // finalize: iterate to the attainable accuracy, detected quickly
+  const SolveTol tol{rt * rt, (stop_kind == 0) ? 6 : std::max(1, h->cfg.pcg_stall_window)};   // finalize: iterate to the attainable accuracy, detected quickly
+  h->last_tol = tol;
   zero(A.x, m);
   EvalOut e0 = eval_f01(A, J, t, A.z, A.x, A.g);
   if (!e0.finite) {
@@ -48,10 +48,10 @@ Engine::NewtonOut Engine::newton(Amg &A, int J, double t, int maxit, int stop_ki
   while (k < maxit && !converged) {
     ++k;
     assemble(A, S, J, t, A.z, A.x);
-    const SolveResult sr = solve(A, S, J, A.g, A.dir);
+    const SolveResult sr = solve(A, S, J, A.g, A.dir, tol);
     const int pit = sr.iters;
-    const double inc = h->hscal[4];
-    const bool dir_finite = (h->hscal[6] == 0.0) && std::isfinite(h->hscal[5]) && std::isfinite(inc);
+    const double inc = sr.dg.ab;
+    const bool dir_finite = (sr.dg.nonfinite == 0.0) && std::isfinite(sr.dg.aa) && std::isfinite(inc);
     out.inc = inc;
     if (h->cfg.verbose > 1)
       fprintf(stderr, "[mgbx] newton J=%d m=%lld k=%d y=%.17g |g|=%.6g lam2=%.6g pcg=%d status=%d rel=%.3g erel=%.3g t=%g\n", J, (long long)m, k, y, gnorm, inc, pit,
@@ -86,7 +86,7 @@ Engine::NewtonOut Engine::newton(Amg &A, int J, double t, int maxit, int stop_ki
     if (!dir_finite) {
       if (h->cfg.verbose > 0)
         fprintf(stderr, "[mgbx] newton J=%d m=%lld k=%d: non-finite direction (g.d=%g |d|^2=%g non-finite entries=%g, pcg=%d, |r|/|b|=%g)\n", J,
-                (long long)m, k, inc, h->hscal[5], h->hscal[6], pit, sr.rel);
+                (long long)m, k, inc, sr.dg.aa, sr.dg.nonfinite, pit, sr.rel);
       out.status = MGBX_NON_FINITE;
       break;
     }
@@ -101,15 +101,14 @@ Engine::NewtonOut Engine::newton(Amg &A, int J, double t, int maxit, int stop_ki
     while (o.line_search == 1 && sstep > 0.0) {
       bool ok = true;
       auto phi = [&](double sigma) -> double {
-        trial(A, J, sigma);
-        EvalOut e = eval_f01(A, J, t, A.z, A.xn, A.gn);
+        const TrialOut e = eval_trial(A, J, t, sigma);
         if (!std::isfinite(e.y)) {   // "line search: non-finite barrier value"
           ok = false;
           return NAN;
         }
-        dot2_fetch(A, J, A.gn, A.dir);
-        if (!std::isfinite(h->hscal[4])) ok = false;   // @assert isfinite(fc)
-        return h->hscal[4];
+        const double fc = dot2(A, J, A.gn, A.dir).ab;
+        if (!std::isfinite(fc)) ok = false;   // @assert isfinite(fc)
+        return fc;
       };
       double a = 0.0, b = sstep, fa = inc, fb = phi(b), sstar = b;
       if (ok) {
@@ -139,8 +138,7 @@ Engine::NewtonOut Engine::newton(Amg &A, int J, double t, int maxit, int stop_ki
         }
       }
       if (ok) {
-        trial(A, J, sstar);
-        EvalOut et = eval_f01(A, J, t, A.z, A.xn, A.gn);
+        const TrialOut et = eval_trial(A, J, t, sstar);
         if (et.finite) {
           std::swap(A.xn, A.xbest);
           std::swap(A.gn, A.gbest);
@@ -154,9 +152,8 @@ Engine::NewtonOut Engine::newton(Amg &A, int J, double t, int maxit, int stop_ki
     }
     // backtracking line search (newton.jl:139-154 with the trial loop of :35-50)
     while (o.line_search == 0 && sstep > 0.0) {
-      trial(A, J, sstep);
-      EvalOut et = eval_f01(A, J, t, A.z, A.xn, A.gn);
-      const bool stalled = (h->hscal[7] == 0.0);
+      const TrialOut et = eval_trial(A, J, t, sstep);
+      const bool stalled = (et.step2 == 0.0);
       if (et.finite) {
         std::swap(A.xn, A.xbest);
         std::swap(A.gn, A.gbest);
@@ -247,14 +244,10 @@ int Engine::matched_t(double t_default, double *t_out, double *tstar_out) {
   (void)e1;
   axpby(m, 1.0, A.gn, -1.0, A.g, A.gn);   // gn = gc
   assemble(A, S, J, 1.0, A.z, A.x);
-  solve(A, S, J, A.g, A.dir);      // nphi
-  solve(A, S, J, A.gn, A.xn);      // nc
-  const double d = h->hscal[4];    // gc . nc
-  (void)m;
-  dot2_fetch(A, J, A.xn, A.g);
-  const double b1 = h->hscal[4];
-  dot2_fetch(A, J, A.dir, A.gn);
-  const double b = b1 + h->hscal[4];
+  solve(A, S, J, A.g, A.dir, h->last_tol);                       // nphi
+  const double d = solve(A, S, J, A.gn, A.xn, h->last_tol).dg.ab;   // gc . nc
+  const double b1 = dot2(A, J, A.xn, A.g).ab;
+  const double b = b1 + dot2(A, J, A.dir, A.gn).ab;
   *tstar_out = NAN;
   *t_out = t_default;
   if (!(d > 0.0)) return MGBX_OK;

@@ -791,12 +791,12 @@ __global__ void __launch_bounds__(kPcg2Threads, 1) k_pcg2(const Pcg2Plan *plan_g
     if (s_xrt.aborted) status = -3.0;   // a peer never arrived at a cross-GPU barrier
   }
   if (tid == 0) {
-    P.out[0] = (double)it;
-    P.out[1] = rr;
-    P.out[2] = status;
-    P.out[3] = bb;
-    P.out[4] = e_tot;      // b.x = |x|_A^2 (energy of the computed direction)
-    P.out[5] = e_last4;    // the part of it gained in the last four iterations
+    P.out[kPcg2OutIters] = (double)it;
+    P.out[kPcg2OutRR] = rr;
+    P.out[kPcg2OutStatus] = status;
+    P.out[kPcg2OutBB] = bb;
+    P.out[kPcg2OutEnergy] = e_tot;
+    P.out[kPcg2OutEnergyLast4] = e_last4;
   }
 }
 

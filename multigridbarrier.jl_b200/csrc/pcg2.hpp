@@ -88,9 +88,19 @@ struct Pcg2Plan {
   unsigned int *bar = nullptr;
   Pcg2Dist dist;
   unsigned long long *prof = nullptr;   // optional phase profile: [0] count, then (tag, globaltimer ns) pairs; tag = level * 16 + kind
-  double *out = nullptr;       // [0] iterations, [1] |r|^2, [2] status (1 converged, 2 stagnated above the tolerance, 3 iteration limit, -1 breakdown,
-                               // -3 a peer never arrived at a cross-GPU barrier), [3] |b|^2,
-                               // [4] b.x = |x|_A^2, [5] the part of [4] gained in the last four iterations
+  double *out = nullptr;       // result record, kPcg2OutCount slots (below)
+};
+
+// slots of Pcg2Plan::out, written by k_pcg2 once per launch
+enum {
+  kPcg2OutIters = 0,   // iterations
+  kPcg2OutRR,          // |r|^2
+  kPcg2OutStatus,      // 1 converged, 2 stagnated above the tolerance, 3 iteration limit, -1 breakdown,
+                       // -3 a peer never arrived at a cross-GPU barrier
+  kPcg2OutBB,          // |b|^2
+  kPcg2OutEnergy,      // b.x = |x|_A^2
+  kPcg2OutEnergyLast4, // the part of kPcg2OutEnergy gained in the last four iterations
+  kPcg2OutCount
 };
 
 // shared memory the tail needs: indices + FP32 values of A, T, Tt of the levels >= nbig, their diagonals and work vectors
