@@ -372,6 +372,7 @@ __device__ __forceinline__ void dmma_m8n8k4(double &d0, double &d1, double a, do
 // blocked dense Cholesky (solver_kernels.cuh): panel width and the diagonal-block kernel's shared memory
 constexpr int kCholNB = 64;
 constexpr size_t kCholDiagSmem = sizeof(double) * 2 * kCholNB * (kCholNB + 1);
+constexpr int kDenseMaxUnknowns = 8192;   // blocked Cholesky: the triangular solve keeps the right-hand side in shared memory (64 KB)
 
 // ------------------------------------------------------------------------------------------------
 // Sum-factorised (Kronecker) assembly for tensor-product spectral discretisations (spectral2d).

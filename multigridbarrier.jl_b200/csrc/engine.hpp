@@ -486,7 +486,6 @@ void solve_kernels_init();
 void kron_w_init(size_t smem);
 
 inline bool dense_mode(const Amg &A) { return A.N == 1 && A.p > 64; }
-constexpr int kDenseMaxUnknowns = 8192;   // blocked Cholesky: the triangular solve keeps the right-hand side in shared memory (64 KB)
 
 // M = kron(A, B) with A r1 x c1 and B r2 x c2 (row-major outputs)?  M(r, c) is any accessor.  The factors are fixed up to a
 // scalar by taking B as the block through the entry of largest magnitude; the product is verified entry by entry.

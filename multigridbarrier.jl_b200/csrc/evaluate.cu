@@ -508,6 +508,9 @@ void Engine::assemble_unfused(Amg &A, System &S, int J, double t, const double *
 void Engine::dgemm_nt(int M, int N, int K, const double *Am, int64_t lda, const double *Bm, int64_t ldb, const double *sc, double *C, int64_t ldc,
                       bool acc, double alpha) {
   if (M <= 0 || N <= 0) return;
+  // in place (C = A, e.g. L21 = A21 inv(L11)' in dense_factor) is correct only while one CTA owns whole rows of C: it reads
+  // all K columns of its rows of A before it writes any of them, and no other CTA reads those rows
+  if (C == Am && (N > kGemmBN || ldc != lda)) throw std::runtime_error("internal: in-place dgemm_nt needs N <= 64 and ldc == lda");
   dim3 grid((N + kGemmBN - 1) / kGemmBN, (M + kGemmBM - 1) / kGemmBM);
   LAUNCH(KC_DGEMM, k_dgemm_nt<<<grid, 128, 0, s>>>(M, N, K, Am, lda, Bm, ldb, sc, C, ldc, acc ? 1 : 0, alpha));
   h->dgemm_flops += 2.0 * M * (double)N * K;

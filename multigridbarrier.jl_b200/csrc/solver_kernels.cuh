@@ -153,15 +153,20 @@ __global__ void __launch_bounds__(1024) k_coarse_inverse(DevCsr A, double *Minv)
   for (int row = tid; row < m; row += nt)
     for (int64_t k = A.ptr[row]; k < A.ptr[row + 1]; ++k) S[row * ld + A.idx[k]] = A.val[k] * d[row] * d[A.idx[k]];
   __syncthreads();
-  // right-looking Cholesky on the lower triangle
+  // right-looking Cholesky on the lower triangle.  A non-positive pivot means numerical indefiniteness: keep the
+  // preconditioner finite and SPD (any SPD approximation is a valid preconditioner) by decoupling unknown j -- unit pivot,
+  // zero column below it, so no trailing update.  (A tiny pivot instead divides the column by it, grows the trailing
+  // matrix by its inverse square, and overflows after a few such pivots.)  Positive pivots are used as they are.
+  __shared__ int drop;
   for (int j = 0; j < m; ++j) {
-    if (tid == 0) {   // a non-positive pivot means numerical indefiniteness: keep the preconditioner finite (any SPD
-      const double v = S[j * ld + j];   // approximation is a valid preconditioner); positive pivots are used as they are
-      S[j * ld + j] = sqrt((v > 0.0 && isfinite(v)) ? v : 1e-16);
+    if (tid == 0) {
+      const double v = S[j * ld + j];
+      drop = !(v > 0.0 && isfinite(v));
+      S[j * ld + j] = drop ? 1.0 : sqrt(v);
     }
     __syncthreads();
     const double piv = S[j * ld + j];
-    for (int i = j + 1 + tid; i < m; i += nt) S[i * ld + j] /= piv;
+    for (int i = j + 1 + tid; i < m; i += nt) S[i * ld + j] = drop ? 0.0 : S[i * ld + j] / piv;
     __syncthreads();
     const int rem = m - j - 1;
     for (int t = tid; t < rem * rem; t += nt) {
