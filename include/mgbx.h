@@ -181,9 +181,11 @@ typedef struct {
   int32_t spectral_kron;     /* 1 (default): dense (spectral) discretisations whose operators and prolongations are Kronecker products
                                 (spectral2d: :dx = kron(DX, I), R = kron(R1, R1), src/spectral2d.jl:22-35) assemble R'HR sum-factorised
                                 (one small DMMA GEMM per block of variables instead of full n x n x n products); 0: unstructured GEMMs */
-  int32_t uncondensed_pcg;   /* 0 (default): a fine-level Newton system that keeps a slack variable which cannot be eliminated node-locally
-                                (a slack in :broken_P1, test/test_pure_p2.jl) and has more unknowns than the dense direct solver takes
-                                (8192) is refused with MGBX_ERR_UNSUPPORTED; 1: run the V-cycle PCG on it anyway (slow to fail) */
+  int32_t uncondensed_pcg;   /* 0 (default): a fine-level Newton system that keeps a slack variable which can be eliminated neither
+                                node-locally nor element-locally, or whose slack was eliminated element-locally (a slack in :broken_P1,
+                                test/test_pure_p2.jl: exact, element by element, when cfg.condense = 1 on one GPU), and that has more
+                                unknowns than the dense direct solver takes (8192, counted after the elimination) is refused with
+                                MGBX_ERR_UNSUPPORTED; 1: run the V-cycle PCG on it anyway (slow to fail late in the t-ramp) */
   int32_t analytic_schur;    /* 1 (default): the node-local Schur complement of a slack that enters ONE Euclidean-power cone is formed in
                                 closed form, (2/rho) I + (4/rho^2)(B/(A+B)) q q' with H_ss = A + B, instead of H_qq - H_qs H_sq / H_ss:
                                 the subtraction cancels to O(1/t) relative and leaves no correct digit along q at t ~ 1e8 (the reduced

@@ -22,7 +22,7 @@ OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libmgbx.so")
 HDR = os.path.join("..", "..", "include", "mgbx.h")
 # headers every host unit includes (engine.hpp and what it pulls in)
-ENGINE = ["engine.hpp", "host_sparse.hpp", "device_common.cuh", "node_barrier.cuh", "pcg2.hpp", HDR]
+ENGINE = ["engine.hpp", "host_sparse.hpp", "device_common.cuh", "elem_schur.cuh", "node_barrier.cuh", "pcg2.hpp", HDR]
 # source -> files whose change forces a recompile of that source
 SOURCES = {
     "mgbx.cu": ["mgbx.cu", "host_amg.hpp"] + ENGINE,

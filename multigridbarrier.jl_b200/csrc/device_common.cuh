@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "elem_schur.cuh"
 #include "node_barrier.cuh"
 
 namespace mgbx {
@@ -202,6 +203,14 @@ struct CondParams {
   int Krow[MGBX_MAX_ND];
   int64_t Eoff[4];            // first index of eliminated variable ev in the level-L vector
   const double *hEEinv, *hKE;
+};
+
+// an element-local eliminated variable (elem_schur.cuh): nc coefficients per element, the only eliminated variable
+struct ElemLocal {
+  int nc;
+  const int64_t *c0;          // per element: index of its first coefficient within the variable's block
+  const double *P;            // per element: the p x nc block of R_fine (row-major)
+  double *R;                  // per element: packed factor R of W = A^{1/2} P (elem_rsize(nc)), written by each assembly
 };
 
 // ------------------------------------------------------------------------------------------------

@@ -190,9 +190,12 @@ struct System {
     int hidx[kKronMaxCombos];              // packed-symmetric index of the node sample h_jk
   };
   bool kron = false;
-  // fine-level system with a slack-like variable (only :id rows) that could NOT be eliminated node-locally (e.g. a slack in
-  // :broken_P1): its 1/slack^2 entries stay in the matrix, which the V-cycle PCG cannot solve reliably late in the t-ramp
+  // fine-level system with a slack-like variable (only :id rows) that could be eliminated neither node-locally nor element-locally:
+  // its 1/slack^2 entries stay in the matrix, which the V-cycle PCG cannot solve reliably late in the t-ramp
   bool uncondensed_slack = false;
+  // the eliminated variable is element-local (elem_schur.cuh, e.g. a slack in :broken_P1): elim == {that variable}, nE == 1
+  bool elem_local = false;
+  ElemLocal el{};
   std::vector<KronPair> kp;
   double *Wcat = nullptr;
   // PCG work at the largest size (sparse systems only)

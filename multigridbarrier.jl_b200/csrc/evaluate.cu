@@ -465,6 +465,12 @@ void Engine::assemble(Amg &A, System &S, int J, double t, const double *zbase, c
     for (int j = 0; j < S.nK; ++j) E.Krow[j] = S.Krow[j];
     LAUNCH(KC_BLOCKHESS, k_blockhess<<<nblk(S.hblk_size), 256, 0, s>>>(E, S.pl, A.Hn, S.Hblk));
   }
+  if (S.elem_local) {   // the element-local part of the slack's Schur complement, on top of the node-local one
+    ElemParams E = elem_params(A);
+    E.nK = S.nK;
+    for (int j = 0; j < S.nK; ++j) E.Krow[j] = S.Krow[j];
+    LAUNCH(KC_COND, k_elem_local_schur<<<nblk(A.N, 128), 128, 0, s>>>(E, S.pl, S.el, A.hEEinv, A.hKE, S.Hblk));
+  }
   SysLevel &top = S.lev[0];
   LAUNCH(KC_GATHER, k_sell_gather<<<nblk(top.A.nnz), 256, 0, s>>>(S.top, S.Hblk, top.A.val));
   if (dist()) allreduce(top.A.val, top.A.nnz);   // sum of the ranks' element contributions (identical pattern on every rank)

@@ -738,6 +738,51 @@ __global__ void __launch_bounds__(256, 3) k_elem_plap(PlapParams P) {
   if (MODE == NODE_F01) grid_reduce<4>(red, op4, P.partials, P.ticket, P.red_out);
 }
 
+// Element-local slack (elem_schur.cuh), after the element kernel has written the node-local Schur complements into Hblk and
+// 1/a, q into hEEinv, hKE: adds Y'Y to the element blocks of the kept pairs and stores the factor R of W.  One thread per
+// element; the kept variables that own D rows are the distinct first members of the pairs (at most two).
+__global__ void __launch_bounds__(128) k_elem_local_schur(ElemParams E, PairList PL, ElemLocal EL, const double *__restrict__ hEEinv,
+                                                          const double *__restrict__ hKE, double *Hblk) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= E.N) return;
+  const int p = E.p, pp = p * p, nc = EL.nc;
+  int vars[2], nv = 0;
+  for (int pr = 0; pr < PL.npairs; ++pr)
+    if (nv == 0 || (PL.va[pr] != vars[0] && nv < 2)) vars[nv++] = PL.va[pr];
+  const int m = nv * p;
+  double X[kElemMaxP * kElemMaxCols], hinv[kElemMaxP], Pe[kElemMaxP * kElemMaxNc];
+  const int64_t node0 = e * p;
+  for (int i = 0; i < p; ++i) {
+    hinv[i] = hEEinv[node0 + i];
+    for (int k = 0; k < nc; ++k) Pe[i * nc + k] = EL.P[(node0 + i) * nc + k];
+    for (int c = 0; c < m; ++c) X[i * m + c] = 0.0;
+  }
+  for (int a = 0; a < E.nK; ++a) {   // X[i][(v, c)] = sum_{rows j of v} q_{j,i} D_j[i][c]
+    const int j = E.Krow[a], o = E.D_op[j];
+    const int col0 = (E.D_var[j] == vars[0]) ? 0 : p;
+    for (int i = 0; i < p; ++i) {
+      const double q = hKE[node0 + i + (int64_t)a * E.n];
+      if (q == 0.0) continue;
+      if (o < 0) X[i * m + col0 + i] += q;
+      else {
+        const double *blk = E.ops[o] + e * (int64_t)pp + i;
+        for (int c = 0; c < p; ++c) X[i * m + col0 + c] += q * blk[(int64_t)c * p];
+      }
+    }
+  }
+  elem_condense(p, nc, Pe, hinv, X, m, EL.R + e * elem_rsize(nc));
+  for (int pr = 0; pr < PL.npairs; ++pr) {
+    const int ca = (PL.va[pr] == vars[0]) ? 0 : p, cb = (PL.vb[pr] == vars[0]) ? 0 : p;
+    double *out = Hblk + ((int64_t)pr * E.N + e) * pp;
+    for (int r = 0; r < p; ++r)
+      for (int c = 0; c < p; ++c) {
+        double s = 0.0;
+        for (int i = 0; i < p; ++i) s += X[i * m + ca + r] * X[i * m + cb + c];
+        out[r * p + c] += s;
+      }
+  }
+}
+
 __global__ void __launch_bounds__(256) k_sell_gather(SellPlan P, const double *__restrict__ in, double *__restrict__ out) {
   const int64_t nz = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (nz >= P.nout) return;

@@ -409,9 +409,16 @@ SolveResult Engine::solve_compact(System &S, int ktop, const double *b, double *
   // (kappa -> sqrt(kappa) ~50 times per barrier step) before mgb_core gives up.  The reference's direct solve has no such
   // regime; refuse it up front unless the caller opts in (cfg.uncondensed_pcg).
   if (S.uncondensed_slack && !h->cfg.uncondensed_pcg && Lv.m > kDenseMaxUnknowns)
-    throw UnsupportedError("Newton system with a slack variable that cannot be eliminated node-locally (e.g. a slack in :broken_P1) and " +
+    throw UnsupportedError("Newton system with a slack variable that can be eliminated neither node-locally nor element-locally and " +
                            std::to_string((long long)Lv.m) + " unknowns: above the dense direct solver's size (8192) only the V-cycle PCG is available, "
                            "which is not reliable for these systems (set cfg.uncondensed_pcg = 1 to try anyway)");
+  // The same rule after an element-local elimination (e.g. a slack in :broken_P1): the condensed systems keep the late-ramp
+  // conditioning that stalls the V-cycle PCG (400 iterations without convergence from t max|f| ~ 3e5 on pure P2, CPU
+  // experiment tools/pure_p2_lab.py), so above the dense solver's size they are refused as well.
+  if (S.elem_local && !h->cfg.uncondensed_pcg && Lv.m > kDenseMaxUnknowns)
+    throw UnsupportedError("Newton system with an element-local slack variable (e.g. a slack in :broken_P1), eliminated exactly: the condensed "
+                           "system still has " + std::to_string((long long)Lv.m) + " unknowns, above the dense direct solver's size (8192); the V-cycle PCG "
+                           "is not reliable for these systems late in the t-ramp (set cfg.uncondensed_pcg = 1 to try anyway)");
   SolveResult r = pcg(S, ktop, b, x, tol);
   // PCG first, direct second: a solve that broke down or stayed inexact is redone by the dense Cholesky when the system is
   // small enough to hold as a dense matrix (the un-condensable families, the last steps of a parabolic ramp)
@@ -450,7 +457,8 @@ SolveResult Engine::solve(Amg &A, System &S, int J, const double *g, double *dir
     for (int e = 0; e < S.nE; ++e) C.Eoff[e] = A.voff[A.L - 1][S.elim[e]];
     C.hEEinv = A.hEEinv;
     C.hKE = A.hKE;
-    LAUNCH(KC_COND, k_condense_rhs<<<nblk(A.n), 256, 0, s>>>(C, g, A.G));
+    if (S.elem_local) LAUNCH(KC_COND, k_condense_rhs_elem<<<nblk(A.N), 256, 0, s>>>(C, S.el, A.N, A.p, g, A.G));
+    else LAUNCH(KC_COND, k_condense_rhs<<<nblk(A.n), 256, 0, s>>>(C, g, A.G));
     ElemParams E = elem_params(A);
     E.nK = S.nK;
     for (int j = 0; j < S.nK; ++j) E.Krow[j] = S.Krow[j];
@@ -472,7 +480,8 @@ SolveResult Engine::solve(Amg &A, System &S, int J, const double *g, double *dir
     spmv(A.RL, dir, nullptr, 1.0, A.gb);
     NodeParams NP = node_params(A, 0.0);
     NP.zf = A.gb;
-    LAUNCH(KC_COND, k_backsubst<<<nblk(A.n), 256, 0, s>>>(C, NP, g, dir));
+    if (S.elem_local) LAUNCH(KC_COND, k_backsubst_elem<<<nblk(A.N), 256, 0, s>>>(C, S.el, NP, A.N, g, dir));
+    else LAUNCH(KC_COND, k_backsubst<<<nblk(A.n), 256, 0, s>>>(C, NP, g, dir));
   }
   stage_end(STAGE_SOLVE, st);
   r.dg = dot2(A, J, dir, g);

@@ -189,6 +189,40 @@ SellPlan device_product_plan(Pool &pool, const DevCsr &Lm, const DevCsr &Rm, con
   tmp_free(rowof, s);
   return P;
 }
+// Is the prolongation block B (rows: the variable's n = N p broken nodes, cols: its fine-level coefficients) element-local?
+// Every column must be supported inside one element's node range, every element must own the same number nc <= kElemMaxNc
+// of consecutive columns.  Returns nc (0: not element-local) and fills c0 (first column per element) and P (N x p x nc).
+static int element_local_blocks(const HostCsr &B, int64_t N, int p, std::vector<int64_t> &c0, std::vector<double> &P) {
+  const HostCsr Bt = transpose(B);
+  std::vector<int64_t> elem_of(Bt.rows, -1);
+  for (int64_t c = 0; c < Bt.rows; ++c) {
+    if (Bt.ptr[c] == Bt.ptr[c + 1]) return 0;
+    const int64_t e = Bt.idx[Bt.ptr[c]] / p;
+    for (int64_t k = Bt.ptr[c]; k < Bt.ptr[c + 1]; ++k)
+      if (Bt.idx[k] / p != e) return 0;
+    elem_of[c] = e;
+  }
+  c0.assign(N, -1);
+  std::vector<int> cnt(N, 0);
+  for (int64_t c = 0; c < Bt.rows; ++c) {
+    const int64_t e = elem_of[c];
+    if (c0[e] < 0) c0[e] = c;
+    else if (c != c0[e] + cnt[e]) return 0;   // the element's columns must be consecutive
+    cnt[e]++;
+  }
+  const int nc = N > 0 ? cnt[0] : 0;
+  for (int64_t e = 0; e < N; ++e)
+    if (cnt[e] != nc) return 0;
+  if (nc < 1 || nc > kElemMaxNc) return 0;
+  P.assign((size_t)N * p * nc, 0.0);
+  for (int64_t i = 0; i < B.rows; ++i)
+    for (int64_t k = B.ptr[i]; k < B.ptr[i + 1]; ++k) {
+      const int64_t e = i / p;
+      P[(size_t)i * nc + (B.idx[k] - c0[e])] = B.val.empty() ? 1.0 : B.val[k];
+    }
+  return nc;
+}
+
 // -------------------------------------------------------------------------------------------------
 // host-side plan construction
 // -------------------------------------------------------------------------------------------------
@@ -239,6 +273,34 @@ std::unique_ptr<System> build_system(mgbx_handle *h, Amg &A, bool condensed, int
         }
     }
     if (ne == A.nu) is_elim[0] = 0;   // keep at least one variable in the reduced system
+    // otherwise, an element-local variable (single GPU): eliminated exactly element by element (elem_schur.cuh)
+    if (ne == 0 && A.nu > 1 && h->nranks == 1 && A.p <= kElemMaxP)
+      for (int v = 0; v < A.nu && !S->elem_local; ++v) {
+        bool idonly = true, any = false;
+        for (int j = 0; j < A.nD; ++j)
+          if (A.D_var[j] == v) {
+            any = true;
+            if (A.D_op[j] >= 0) idonly = false;
+          }
+        int coupled = 0;   // kept variables with D rows: Y has one p-column block per such variable
+        for (int u = 0; u < A.nu; ++u) {
+          bool rows = false;
+          for (int j = 0; j < A.nD; ++j) rows = rows || (u != v && A.D_var[j] == u);
+          coupled += rows ? 1 : 0;
+        }
+        if (!any || !idonly || coupled > 2) continue;
+        std::vector<int64_t> c0;
+        std::vector<double> Pe;
+        const int nc = element_local_blocks(submatrix(Rtop, (int64_t)v * A.n, (int64_t)(v + 1) * A.n, A.voff[L - 1][v], A.voff[L - 1][v + 1]),
+                                            A.N, A.p, c0, Pe);
+        if (nc == 0) continue;
+        is_elim[v] = 1;
+        S->elem_local = true;
+        S->el.nc = nc;
+        S->el.c0 = pool.upload<int64_t>(c0.data(), c0.size(), s);
+        S->el.P = pool.upload<double>(Pe.data(), Pe.size(), s);
+        S->el.R = pool.zeros<double>((size_t)A.N * elem_rsize(nc), s);
+      }
   }
   for (int v = 0; v < A.nu; ++v) (is_elim[v] ? S->elim : S->kept).push_back(v);
   S->nE = (int)S->elim.size();

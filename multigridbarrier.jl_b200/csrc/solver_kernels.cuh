@@ -67,6 +67,44 @@ __global__ void __launch_bounds__(256) k_backsubst(CondParams P, NodeParams NP, 
   }
 }
 
+// Element-local eliminated variable (elem_schur.cuh), one thread per element:
+// Gt[Krow[a]*n + i] = - q_{a,i} (P_e y)_i,  y = H_ss,e^-1 g_c,e  (so that rhs_u = g_u - R_u' H_us H_ss^-1 g_c after k_blockgrad)
+__global__ void __launch_bounds__(256) k_condense_rhs_elem(CondParams P, ElemLocal EL, int64_t N, int p, const double *__restrict__ g, double *Gt) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= N) return;
+  const int nc = EL.nc;
+  double y[kElemMaxNc];
+  const double *gc = g + P.Eoff[0] + EL.c0[e];
+  for (int k = 0; k < nc; ++k) y[k] = gc[k];
+  elem_hss_solve(nc, EL.R + e * elem_rsize(nc), y);
+  for (int r = 0; r < p; ++r) {
+    const int64_t i = e * p + r;
+    double v = 0.0;
+    for (int k = 0; k < nc; ++k) v += EL.P[i * nc + k] * y[k];
+    for (int a = 0; a < P.nK; ++a) Gt[i + (int64_t)P.Krow[a] * P.n] = -P.hKE[i + (int64_t)a * P.n] * v;
+  }
+}
+
+// dc_e = H_ss,e^-1 (g_c,e - P_e' sum_a q_a (D_a du)):  x[Eoff[0] + c0[e] + k]
+__global__ void __launch_bounds__(256) k_backsubst_elem(CondParams P, ElemLocal EL, NodeParams NP, int64_t N, const double *__restrict__ g, double *x) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= N) return;
+  const int nc = EL.nc, p = NP.p;
+  double rc[kElemMaxNc];
+  const int64_t col = P.Eoff[0] + EL.c0[e];
+  for (int k = 0; k < nc; ++k) rc[k] = g[col + k];
+  for (int r = 0; r < p; ++r) {
+    const int64_t i = e * p + r;
+    double y[MGBX_MAX_ND];
+    node_Dz(NP, i, y);   // NP.zf = broken image of the kept part of the direction
+    double s = 0.0;
+    for (int a = 0; a < P.nK; ++a) s += P.hKE[i + (int64_t)a * P.n] * y[P.Krow[a]];
+    for (int k = 0; k < nc; ++k) rc[k] -= EL.P[i * nc + k] * s;
+  }
+  elem_hss_solve(nc, EL.R + e * elem_rsize(nc), rc);
+  for (int k = 0; k < nc; ++k) x[col + k] = rc[k];
+}
+
 // start vector of the power iteration on D^-1 A (pcg2_lambda_power: a sharper lambda_max for the Chebyshev interval than the
 // Gershgorin bound): smooth + oscillatory parts, never orthogonal to the top eigenvector in practice
 __global__ void k_pw_init(int64_t m, double *v) {
